@@ -2,7 +2,7 @@
 """bench.py - headline benchmark of the B200 hot path (BASELINE.json: "poses/sec (fused MLP inference,
 bf16) at 1/2/4/8 B200; batch-1 p50 latency").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of LinearModel(1024, 2, residual, batch_norm, max_norm) inference over one
 batch of 2^20 synthetic poses per GPU (configs[1]).  N > 1 is launched by torch.distributed.run, one
@@ -17,6 +17,12 @@ poses per GPU, 8 x 2^21 = 16 M).
 --impl reference times the reference's own CPU implementation of the path.  TensorFlow is not
 installable here (no network, SURVEY 8c), so this is the NumPy restatement of linear_model.py's graph
 (oracle/mlp_ref.py, "port"), fp32, all host threads, on a bounded sample of the same workload.
+
+--dump-outputs DIR writes, after the timed steps, predictions y of the last timed step as DIR/y.npy (float32; with
+N > 1 one file per rank, DIR/y_rank<r>.npy): the same rows in every run, so that two builds run with the same arguments
+can be compared output for output (the inputs are seeded too).  Our arm writes a fixed, seeded sample of DUMP_ROWS of
+its 2^20 rows; the reference arm writes its first REF_DUMP_ROWS rows, which its sample always holds (the sample size
+follows the host's speed, its first rows do not).
 """
 from __future__ import annotations
 
@@ -43,6 +49,18 @@ L, NL, IN, OUT = 1024, 2, 32, 48
 FLOP_PER_POSE = 2 * (IN * L + 2 * NL * L * L + L * OUT)       # 8,552,448 (SURVEY 8d)
 B_PER_GPU = 1 << 20
 WORKLOAD = "LinearModel(linear_size=1024,num_layers=2,residual,batch_norm,max_norm) inference, batch 2^20 poses/GPU"
+DUMP_ROWS = 32768           # 6.3 MB of float32 predictions per rank: 8 ranks stay under 64 MB
+REF_DUMP_ROWS = 4096        # the reference arm's smallest sample
+
+
+def dump_rows(n):
+    """Row indices --dump-outputs writes out of n predictions: the same seeded sample in every run."""
+    return np.sort(np.random.RandomState(0).choice(n, min(n, DUMP_ROWS), replace=False))
+
+
+def write_dump(dirname, name, arr):
+    os.makedirs(dirname, exist_ok=True)
+    np.save(os.path.join(dirname, name + ".npy"), np.ascontiguousarray(arr, dtype=np.float32))
 
 
 def load_peaks():
@@ -163,7 +181,7 @@ def run_reference(args):
     # size the per-step sample so that the whole run stays within ~4 minutes: at the ~170 K poses/s of a 16-core host
     # that is the full 2^20-pose batch of our arm's config (same_config), fewer poses on a smaller host
     budget = float(os.environ.get("P3D_BENCH_REF_BUDGET_S", "240")) / max(1, args.steps + args.warmup)
-    sample = int(min(B_PER_GPU, max(4096, (rate0 * budget) // 4096 * 4096)))
+    sample = int(min(B_PER_GPU, max(REF_DUMP_ROWS, (rate0 * budget) // 4096 * 4096)))
     from oracle import mlp_ref as M
     from oracle import synth
     cfg = M.Config(L, NL, True, True, True)
@@ -173,8 +191,10 @@ def run_reference(args):
         cpu_forward(M, p, x, cfg, threads)
     t0 = time.perf_counter()
     for _ in range(args.steps):
-        cpu_forward(M, p, x, cfg, threads)
+        y = cpu_forward(M, p, x, cfg, threads)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        write_dump(args.dump_outputs, "y", y[:REF_DUMP_ROWS])
     value = sample * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
@@ -413,25 +433,10 @@ def secondary_measurements(torch, model, lib, _lib, peaks, dev, stream, sptr):
     return out
 
 
-def run_ours(args):
-    import torch
-    import torch.distributed as dist
-    if not torch.cuda.is_available():
-        print(json.dumps({"error": "no CUDA device: libp3d has no CPU fallback"}))
-        return 2
-    rank = int(os.environ.get("RANK", "0"))
-    local_rank = int(os.environ.get("LOCAL_RANK", "0"))
-    world = int(os.environ.get("WORLD_SIZE", "1"))
-    numa = bind_to_gpu_numa(local_rank) if world > 1 else {"bound": False, "note": "single rank: affinity left alone"}
-    torch.cuda.set_device(local_rank)
-    dev = torch.device("cuda", local_rank)
-    if world > 1:
-        dist.init_process_group("nccl", device_id=dev)
-    from p3d import LinearModel, _lib
-    lib = _lib.lib
-    peaks = load_peaks()
-
-    # random-init weights (the model's own kaiming init) + non-trivial BN statistics so that the folding is real
+def timed_model(local_rank):
+    """The model of the timed path: random-init weights (the model's own kaiming init) + non-trivial BN statistics so
+    that the folding is real."""
+    from p3d import LinearModel
     model = LinearModel(L, NL, True, True, True, 64, 1e-3, mode="bf16", device=local_rank, seed=1)
     rng = np.random.RandomState(2)
     for name, shape in model.variable_shapes().items():
@@ -446,10 +451,36 @@ def run_ours(args):
             model.set_variable(name, rng.normal(0, 0.5, shape))
         elif leaf == "moving_variance":
             model.set_variable(name, rng.uniform(0.5, 2.0, shape))
+    return model
 
-    B = B_PER_GPU
+
+def timed_inputs(torch, dev, rank):
+    """The B_PER_GPU input poses of the timed path on this rank."""
     g = torch.Generator(device=dev).manual_seed(1234 + rank)
-    x = torch.randn((B, IN), device=dev, generator=g)
+    return torch.randn((B_PER_GPU, IN), device=dev, generator=g)
+
+
+def run_ours(args):
+    import torch
+    import torch.distributed as dist
+    if not torch.cuda.is_available():
+        print(json.dumps({"error": "no CUDA device: libp3d has no CPU fallback"}))
+        return 2
+    rank = int(os.environ.get("RANK", "0"))
+    local_rank = int(os.environ.get("LOCAL_RANK", "0"))
+    world = int(os.environ.get("WORLD_SIZE", "1"))
+    numa = bind_to_gpu_numa(local_rank) if world > 1 else {"bound": False, "note": "single rank: affinity left alone"}
+    torch.cuda.set_device(local_rank)
+    dev = torch.device("cuda", local_rank)
+    if world > 1:
+        dist.init_process_group("nccl", device_id=dev)
+    from p3d import _lib
+    lib = _lib.lib
+    peaks = load_peaks()
+
+    model = timed_model(local_rank)
+    B = B_PER_GPU
+    x = timed_inputs(torch, dev, rank)
     t = torch.zeros((B, OUT), device=dev)
     y = torch.empty((B, OUT), device=dev)
     stream = torch.cuda.current_stream()
@@ -485,6 +516,7 @@ def run_ours(args):
     kms, kn = C.c_double(), C.c_int64()
     lib.p3d_profile_read(C.byref(kms), C.byref(kn))
     lib.p3d_profile_enable(0)
+    dumped = y[torch.from_numpy(dump_rows(B)).to(dev)].cpu().numpy() if args.dump_outputs else None
     clocks = sampler.summary() if sampler else None
     el = torch.tensor([elapsed_ms], device=dev, dtype=torch.float64)
     if world > 1:
@@ -630,6 +662,8 @@ def run_ours(args):
         if secondary:
             line["secondary"] = secondary
         print(json.dumps(line))
+    if dumped is not None:
+        write_dump(args.dump_outputs, "y" if world == 1 else f"y_rank{rank}", dumped)
     lib.p3d_host_free(yh_ptr)
     lib.p3d_host_free(xh_ptr)
     lib.p3d_host_free(th_ptr)
@@ -647,7 +681,10 @@ def main():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the batch sweep / training / preprocessing / evaluation lines")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write a fixed sample of the last timed step's predictions to DIR/y.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
     # The contract is ONE JSON line on stdout: libraries (NCCL's version banner, torchrun notices) also write to
     # fd 1, so fd 1 is pointed at stderr for the duration of the run and the line goes to the saved descriptor.
     sys.stdout.flush()

@@ -45,13 +45,14 @@ N = 64
 cams = synth.cameras(4, seed=3)
 world = synth.world_poses(N, seed=3)                          # [N,96] float64
 g = {"world": world}
+pts = world[:48].reshape(-1, 3)          # per-point camera arrays for the first 48 poses: keeps the file under 1 MB
 for ci, (R, T, f, c, k, p) in enumerate(cams):
     g[f"cam{ci}_R"], g[f"cam{ci}_T"], g[f"cam{ci}_f"] = R, T, f
     g[f"cam{ci}_c"], g[f"cam{ci}_k"], g[f"cam{ci}_p"] = c, k, p
-    proj, D, radial, tan, r2 = ref_cam.project_point_radial(world.reshape(-1, 3), R, T, f, c, k, p)
+    proj, D, radial, tan, r2 = ref_cam.project_point_radial(pts, R, T, f, c, k, p)
     g[f"cam{ci}_proj"], g[f"cam{ci}_D"], g[f"cam{ci}_radial"] = proj, D, radial
     g[f"cam{ci}_tan"], g[f"cam{ci}_r2"] = tan, r2
-    w2c = ref_cam.world_to_camera_frame(world.reshape(-1, 3), R, T)
+    w2c = ref_cam.world_to_camera_frame(pts, R, T)
     g[f"cam{ci}_w2c"] = w2c
     g[f"cam{ci}_c2w"] = ref_cam.camera_to_world_frame(w2c, R, T)
 

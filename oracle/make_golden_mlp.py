@@ -16,8 +16,8 @@ state) and run eagerly on the same shim with the same variables.
 
 Inputs and variables are seeded (oracle.synth / oracle.mlp_ref.init_params, rounded through float32 so that the CUDA
 library can hold the very same values); dropout noise is injected as the documented Philox4x32-10 stream
-(oracle.mlp_ref.dropout_mask_philox) that the CUDA kernels generate themselves.  Large tensors of the 1024-wide cases
-are recorded as strided samples plus norms to keep the fixture small.
+(oracle.mlp_ref.dropout_mask_philox) that the CUDA kernels generate themselves.  Tensors of more than 256
+entries are recorded as strided samples, norms and leading blocks, which keeps the fixture under 1 MB.
 Nothing at test/bench time reads /root/reference.
 """
 import os
@@ -73,18 +73,21 @@ def load_params(p):
     return byname
 
 
-def sample(a, big):
-    """What is stored of a tensor: everything, or (for matrices of the wide cases) a strided sample + norm."""
+def sample(a):
+    """What is stored of a tensor: everything (up to 256 entries), or a strided sample of 256 entries + the norm + the
+    leading block (16 entries of a vector, 4 rows of an output, 2 rows x 48 columns of a wider matrix); the tests read
+    it back with test_oracle_mlp_golden.strided_sample / head_of."""
     a = np.asarray(a, np.float64)
-    if not big or a.ndim < 2 or a.size <= 16384:
+    if a.size <= 256:
         return {"": a}
     flat = a.reshape(-1)
-    return {"@sample": flat[:: max(1, flat.size // 4093)][:4093].copy(), "@norm": np.array(np.linalg.norm(flat)),
-            "@head": a[:(64 if a.shape[1] <= 48 else 2)].copy()}
+    head = a[:16] if a.ndim == 1 else a[:(4 if a.shape[1] <= 48 else 2), :48]
+    return {"@sample": flat[:: 16 * max(1, flat.size // 4093)][:256].copy(), "@norm": np.array(np.linalg.norm(flat)),
+            "@head": head.copy()}
 
 
-def put(out, key, a, big=False):
-    for suf, v in sample(a, big).items():
+def put(out, key, a):
+    for suf, v in sample(a).items():
         out[key + suf] = v
 
 
@@ -110,7 +113,7 @@ def run_case(out, tag, L, nl, residual, bn, max_norm, B, lr=1e-3, predict_14=Fal
     tf.set_dropout_masks(None)
     r = model.step(sess, x, t, 1.0, isTraining=False)
     assert len(r) == 3
-    out[tag + "/eval_loss"] = np.array(r[0]); put(out, tag + "/eval_y", r[2], big)
+    out[tag + "/eval_loss"] = np.array(r[0]); put(out, tag + "/eval_y", r[2])
     assert list(r[1].keys()) == ["loss/loss"] and r[1]["loss/loss"] == r[0]
 
     # ---- gradients of the first training step (opt.compute_gradients, :143-144), no update
@@ -133,7 +136,7 @@ def run_case(out, tag, L, nl, residual, bn, max_norm, B, lr=1e-3, predict_14=Fal
     trainable = M.trainable_names(L, nl, batch_norm=bn)
     assert sorted(names) == sorted(trainable), (names, trainable)      # every W, b, gamma, beta; no moving statistics
     for nme, g in zip(names, gvals):
-        put(out, tag + "/grad0/" + nme, g, big)
+        put(out, tag + "/grad0/" + nme, g)
 
     # ---- training steps through LinearModel.step(isTraining=True): 4-tuple (:229-237)
     losses, lrs = [], []
@@ -142,19 +145,19 @@ def run_case(out, tag, L, nl, residual, bn, max_norm, B, lr=1e-3, predict_14=Fal
         r = model.step(sess, x, t, KEEP, isTraining=True)
         assert len(r) == 4
         losses.append(r[0]); lrs.append(r[2]["learning_rate/learning_rate"])
-        put(out, tag + "/train_y%d" % s, r[3], big)
+        put(out, tag + "/train_y%d" % s, r[3])
     out[tag + "/train_loss"] = np.array(losses)
     out[tag + "/train_lr"] = np.array(lrs)
     assert int(model.global_step.eval()) == steps
     for nme, v in byname.items():
         if nme in ("learning_rate", "global_step"):
             continue
-        put(out, tag + "/final/" + nme, v.eval(), big)
+        put(out, tag + "/final/" + nme, v.eval())
 
     # ---- inference after training (moving statistics now updated)
     tf.set_dropout_masks(None)
     r = model.step(sess, x, t, 1.0, isTraining=False)
-    out[tag + "/eval2_loss"] = np.array(r[0]); put(out, tag + "/eval2_y", r[2], big)
+    out[tag + "/eval2_loss"] = np.array(r[0]); put(out, tag + "/eval2_y", r[2])
     print("%-28s eval loss %.6f  train losses %s  lr %s" % (tag, out[tag + "/eval_loss"], np.round(losses, 6), lrs[-1]))
     return p, x
 

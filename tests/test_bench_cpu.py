@@ -7,6 +7,8 @@ import re
 import subprocess
 import sys
 
+import numpy as np
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -15,8 +17,9 @@ def run_bench(*flags, env=None):
     return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), *flags], capture_output=True, text=True, env=e, timeout=600)
 
 
-def test_reference_arm_prints_one_json_line_with_the_contract_keys():
-    r = run_bench("--impl", "reference", "--steps", "2", "--warmup", "1", env={"P3D_BENCH_REF_BUDGET_S": "6"})
+def test_reference_arm_prints_one_json_line_with_the_contract_keys(tmp_path):
+    r = run_bench("--impl", "reference", "--steps", "2", "--warmup", "1", "--dump-outputs", str(tmp_path),
+                  env={"P3D_BENCH_REF_BUDGET_S": "6"})
     assert r.returncode == 0, r.stderr[-2000:]
     lines = [ln for ln in r.stdout.splitlines() if ln.strip()]
     assert len(lines) == 1, r.stdout
@@ -28,6 +31,22 @@ def test_reference_arm_prints_one_json_line_with_the_contract_keys():
     assert cb["kind"] == "port" and cb["cores"] >= 1 and cb["value"] == d["value"] and "poses per step" in cb["sample"]
     assert d["e2e"] == {"value": d["value"], "unit": "poses/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert d["config"]["workload"].startswith("LinearModel(linear_size=1024,num_layers=2")
+    # --dump-outputs: the last step's predictions of the first 4096 poses, whatever the sample size, as the oracle
+    # computes them from the same weights and inputs
+    from oracle import mlp_ref as M
+    from oracle import synth
+    assert os.listdir(tmp_path) == ["y.npy"]
+    y = np.load(tmp_path / "y.npy")
+    assert y.dtype == np.float32 and y.shape == (4096, 48)
+    p = {k: v.astype(np.float32) for k, v in M.init_params(1024, 2, seed=1, bn="trained").items()}
+    x, _ = synth.mlp_inputs(4096, seed=0)
+    ref = M.forward(p, x, M.Config(1024, 2, True, True, True), training=False)
+    np.testing.assert_allclose(y, ref, rtol=1e-5, atol=1e-5)
+
+
+def test_steps_below_one_are_refused():
+    r = run_bench("--impl", "reference", "--steps", "0")
+    assert r.returncode == 2 and "--steps" in r.stderr
 
 
 def test_our_arm_has_no_cpu_fallback():

@@ -24,7 +24,7 @@ def cams_of(geo):
 
 def test_project_point_radial_golden(geo):
     from p3d import cameras
-    P = geo["world"].reshape(-1, 3)
+    P = geo["world"].reshape(-1, 3)[: len(geo["cam0_proj"])]      # the per-point arrays hold the first 48 poses
     for i, cam in enumerate(cams_of(geo)):
         proj, D, radial, tan, r2 = cameras.project_point_radial(P, *cam)
         assert proj.shape == (P.shape[0], 2) and proj.dtype == np.float64
@@ -39,7 +39,7 @@ def test_project_point_radial_golden(geo):
 
 def test_world_camera_roundtrip_golden(geo):
     from p3d import cameras
-    P = geo["world"].reshape(-1, 3)
+    P = geo["world"].reshape(-1, 3)[: len(geo["cam0_w2c"])]
     for i, cam in enumerate(cams_of(geo)):
         w2c = cameras.world_to_camera_frame(P, cam[0], cam[1])
         np.testing.assert_allclose(w2c, geo[f"cam{i}_w2c"], rtol=1e-12, atol=1e-8)

@@ -37,7 +37,27 @@ def case_setup(z, tag):
     return cfg, p, x.astype(np.float64), t.astype(np.float64), B, steps, bool(big), float(z[tag + "/lr0"])
 
 
-def check(z, key, a, rtol=1e-12):
+def strided_sample(a):
+    """The entries the fixture keeps under key@sample of a tensor of more than 256 entries: 256 entries of the flattened
+    tensor at a stride of 16 * (size // 4093), i.e. every 16th point of the 4093-point sample the reference run
+    recorded (thinned to keep the fixture under 1 MB)."""
+    flat = np.asarray(a, np.float64).reshape(-1)
+    return flat[:: 16 * max(1, flat.size // 4093)][:256]
+
+
+def head_of(a, head):
+    """The leading block of `a` that key@head holds (its first rows, and the first columns of a wide matrix)."""
+    return np.asarray(a, np.float64)[tuple(slice(0, n) for n in head.shape)]
+
+
+def stored(z, key):
+    """Every entry the fixture holds of a tensor, flattened: the whole tensor, or its sample and leading block."""
+    if key in z.files:
+        return z[key].reshape(-1)
+    return np.concatenate([z[key + "@sample"], z[key + "@head"].reshape(-1)])
+
+
+def check(z, key, a, rtol=1e-12, ntol=1e-10):
     """Compare `a` with what the fixture holds under `key` (whole tensor, or strided sample + norm + head)."""
     a = np.asarray(a, np.float64)
     if key in z.files:
@@ -46,14 +66,13 @@ def check(z, key, a, rtol=1e-12):
         scale = max(np.abs(ref).max(), 1e-30)
         assert np.abs(a - ref).max() <= rtol * max(scale, 1e-6), (key, np.abs(a - ref).max(), scale)
         return
-    flat = a.reshape(-1)
-    smp = flat[:: max(1, flat.size // 4093)][:4093]
+    smp = strided_sample(a)
     ref = z[key + "@sample"]
     scale = max(np.abs(ref).max(), 1e-30)
     assert np.abs(smp - ref).max() <= rtol * max(scale, 1e-6), (key, np.abs(smp - ref).max(), scale)
-    assert abs(np.linalg.norm(flat) - float(z[key + "@norm"])) <= 1e-10 * max(float(z[key + "@norm"]), 1e-6), key
+    assert abs(np.linalg.norm(a) - float(z[key + "@norm"])) <= ntol * max(float(z[key + "@norm"]), 1e-6), key
     head = z[key + "@head"]
-    assert np.abs(a[: head.shape[0]] - head).max() <= rtol * max(np.abs(head).max(), 1e-6), key
+    assert np.abs(head_of(a, head) - head).max() <= rtol * max(np.abs(head).max(), 1e-6), key
 
 
 def masks_for(step, n_hidden, B, L):
@@ -88,7 +107,7 @@ def test_oracle_matches_the_executed_reference_graph(gold, tag):
     for n in names:
         gref_key = tag + "/grad0/" + n
         a = g[n]
-        if gref_key in z.files and np.abs(z[gref_key]).max() < 1e-13:      # bias in front of BatchNorm: exactly zero
+        if np.abs(stored(z, gref_key)).max() < 1e-13:                      # bias in front of BatchNorm: exactly zero
             assert np.abs(a).max() < 1e-12, n
             continue
         check(z, gref_key, a, rtol=1e-9)
@@ -120,10 +139,10 @@ def test_posebase_twin_agrees_with_linear_model(gold):
     tag = "h_1024_b64"
     cfg, p, x, t, B, steps, big, lr0 = case_setup(z, tag)
     # PoseBase creates float32 variables (its kaiming() defaults to tf.float32), so this reading runs in float32
-    np.testing.assert_allclose(z[tag + "/posebase_eval_y"], z[tag + "/eval_y"], rtol=0, atol=2e-6)
-    check(z, tag + "/posebase_eval_y", M.forward(p, x, cfg, training=False), rtol=5e-6)
+    np.testing.assert_allclose(stored(z, tag + "/posebase_eval_y"), stored(z, tag + "/eval_y"), rtol=0, atol=2e-6)
+    check(z, tag + "/posebase_eval_y", M.forward(p, x, cfg, training=False), rtol=5e-6, ntol=5e-6)
     ytr, cache = M.forward(p, x, cfg, training=True, want_cache=True)
-    check(z, tag + "/posebase_train_y", ytr, rtol=5e-6)
+    check(z, tag + "/posebase_train_y", ytr, rtol=5e-6, ntol=5e-6)
     mm = "linear_model/batch_normalization/moving_mean"
     np.testing.assert_allclose(z[tag + "/posebase_mm/moving_mean"], p[mm] * 0.99 + cache[0]["mean"] * 0.01, atol=1e-6)
     mv = "linear_model/batch_normalization/moving_variance"
