@@ -116,9 +116,40 @@ static void drain() {
 }
 }  // namespace prof
 
+bool capturing(cudaStream_t st) {
+  cudaStreamCaptureStatus s = cudaStreamCaptureStatusNone;
+  if (cudaStreamIsCapturing(st, &s) != cudaSuccess) {     // e.g. the legacy stream while another stream captures
+    cudaGetLastError();
+    return true;
+  }
+  return s != cudaStreamCaptureStatusNone;
+}
+int refuse_in_capture(cudaStream_t st, const char* what) {
+  if (!capturing(st)) return P3D_OK;
+  set_error("%s cannot happen inside a CUDA graph capture: warm up first - run the same call (same batch size) once "
+            "outside the capture", what);
+  return P3D_ERR_STATE;
+}
+void retire(p3d_model* m, void* p) {
+  if (!p) return;
+  if (m->captured) m->retired.push_back(p);
+  else cudaFree(p);
+}
+
+int64_t grown_cap(const p3d_model* m, int64_t cap, int64_t need) {
+  return (m->captured && 2 * cap > need) ? 2 * cap : need;
+}
+
 int mark_model_work(p3d_model* m, cudaStream_t st) {
   if (!m->ev_done) P3D_CUDA(cudaEventCreateWithFlags(&m->ev_done, cudaEventDisableTiming));
-  P3D_CUDA(cudaEventRecord(m->ev_done, st));
+  if (capturing(st)) {
+    // an external event-record node: every replay of the graph records ev_done, and the event itself never becomes
+    // part of the capture (a plain record would leave it captured, and the next wait on it would be refused)
+    m->captured = true;
+    P3D_CUDA(cudaEventRecordWithFlags(m->ev_done, st, cudaEventRecordExternal));
+  } else {
+    P3D_CUDA(cudaEventRecord(m->ev_done, st));
+  }
   m->ev_done_recorded = true;
   return P3D_OK;
 }
@@ -229,7 +260,7 @@ int p3d_model_create(const p3d_cfg* cfg, p3d_model** out) {
   m->n_train = off;
   m->n_moving = mo;
   m->rows_total = row + 16;   // slack so the padded output rows exist (zero)
-  m->kpad = L < 64 ? 64 : L;
+  m->kpad = L < 64 ? 64 : (L + 7) / 8 * 8;   // rows start 16-byte aligned: the small-batch kernel loads 8 weights at a time
   auto fail = [&](int rc) { p3d_model_destroy(m); return rc; };
 #define P3D_ALLOC(ptr, bytes)                                                                  \
   do {                                                                                         \
@@ -247,6 +278,13 @@ int p3d_model_create(const p3d_cfg* cfg, p3d_model** out) {
   P3D_ALLOC(m->wfold, sizeof(float) * wf);
   P3D_ALLOC(m->norm2, sizeof(double) * nlay);
   P3D_ALLOC(m->pipe_loss, sizeof(double));
+  // fixed-size forward scratch exists from the start, so that no forward has to allocate it (a graph capture could not)
+  P3D_ALLOC(m->lat_counter, sizeof(unsigned long long) * 32);
+  P3D_ALLOC(m->xchg, sizeof(unsigned) * 64);
+  if (L == 1024 && cfg->mode == P3D_MODE_BF16) {       // the whole-chip kernels' exchange buffers (mlp_simt.cu, mlp_mid.cu)
+    P3D_ALLOC(m->lat_act, sizeof(uint2) * 1024 * 8 * 128);
+    P3D_ALLOC(m->mid_act, sizeof(unsigned long long) * 8 * 64 * 512);
+  }
 #undef P3D_ALLOC
   // TF default BN state: gamma 1, beta 0, moving_mean 0, moving_variance 1
   for (auto& ly : m->layers) {
@@ -288,6 +326,8 @@ void p3d_model_destroy(p3d_model* m) {
   cudaFree(m->theta); cudaFree(m->grad); cudaFree(m->adam_m); cudaFree(m->adam_v); cudaFree(m->moving);
   cudaFree(m->wt_bf16); cudaFree(m->bias_fold); cudaFree(m->wfold); cudaFree(m->norm2); cudaFree(m->pipe_loss);
   cudaFree(m->act_scratch); cudaFree(m->xb); cudaFree(m->f32_a); cudaFree(m->lat_counter); cudaFree(m->lay_act); cudaFree(m->lat_act); cudaFree(m->mid_act);
+  cudaFree(m->xchg);
+  for (void* p : m->retired) cudaFree(p);
   if (m->ev_done) cudaEventDestroy(m->ev_done);
   for (auto& e : m->pipe_ev) if (e) cudaEventDestroy(e);
   for (int i = 0; i < 3; ++i) {
@@ -356,15 +396,24 @@ int64_t p3d_model_global_step(p3d_model* m) { return m ? m->global_step : -1; }
 int p3d_model_prepare_inference(p3d_model* m, void* stream) {
   P3D_REQUIRE(m, "prepare_inference: null model");
   P3D_CUDA(cudaSetDevice(m->cfg.device));
-  return prep::prepare(m, static_cast<cudaStream_t>(stream));
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  // the fold rewrites the packed weights in place (graphs captured earlier read the new ones); captured itself, it
+  // would leave pack_valid set before any replay had computed it
+  if (capturing(st)) {
+    set_error("prepare_inference cannot be captured into a CUDA graph: call it outside the capture");
+    return P3D_ERR_STATE;
+  }
+  P3D_TRY(prep::prepare(m, st));
+  return mark_model_work(m, st);
 }
 
 // packed input buffer [cap][64] bf16 of the tensor-core paths
-static int ensure_xb(p3d_model* m, int64_t B) {
+static int ensure_xb(p3d_model* m, int64_t B, cudaStream_t st) {
   if (m->xb_cap < B) {
-    if (m->xb) cudaFree(m->xb);
+    P3D_TRY(refuse_in_capture(st, "forward: growing the packed-input buffer"));
+    const int64_t cap = grown_cap(m, m->xb_cap, B < 1024 ? 1024 : B);
+    retire(m, m->xb);
     m->xb = nullptr; m->xb_cap = 0;
-    const int64_t cap = B < 1024 ? 1024 : B;
     P3D_CUDA(cudaMalloc(&m->xb, sizeof(__nv_bfloat16) * 64ull * cap));
     m->xb_cap = cap;
   }
@@ -382,7 +431,14 @@ static int forward_packed(p3d_model* m, float* y, int64_t B, cudaStream_t st) {
 }
 
 static int forward_on(p3d_model* m, const float* x, float* y, int64_t B, cudaStream_t st) {
-  if (!m->pack_valid) P3D_TRY(prep::prepare(m, st));
+  if (!m->pack_valid) {
+    if (capturing(st)) {
+      set_error("forward: the variables changed since the last weight fold, and the fold cannot be captured into a "
+                "CUDA graph: call prepare_inference outside the capture first");
+      return P3D_ERR_STATE;
+    }
+    P3D_TRY(prep::prepare(m, st));
+  }
   if (m->cfg.mode == P3D_MODE_FP32) return simt::forward_fp32(m, x, y, B, st);
   const int L = m->L;
   if (B == 1 && L == 1024) {                            // single pose: whole-chip kernel (or the 16-CTA cluster kernel), one launch
@@ -401,7 +457,7 @@ static int forward_on(p3d_model* m, const float* x, float* y, int64_t B, cudaStr
     if (B <= kSmallBatchMax) return simt::forward_small(m, x, y, B, st);
     return simt::forward_fp32(m, x, y, B, st);
   }
-  P3D_TRY(ensure_xb(m, B));
+  P3D_TRY(ensure_xb(m, B, st));
   P3D_TRY(prep::pack_input(x, m->xb, B, st));
   return forward_packed(m, y, B, st);
 }
@@ -424,7 +480,7 @@ int p3d_model_mse(p3d_model* m, const float* y, const float* t, int64_t B, float
   P3D_TRY(sqerr_accumulate(y, t, static_cast<size_t>(B) * m->out_size, m->pipe_loss, st));
   finish_mse_kernel<<<1, 1, 0, st>>>(m->pipe_loss, static_cast<double>(B) * m->out_size, loss);
   P3D_LAUNCH_CHECK();
-  return P3D_OK;
+  return mark_model_work(m, st);     // pipe_loss is the host-buffer step's accumulator too
 }
 
 int p3d_model_step_eval_host(p3d_model* m, const float* x_host, const float* t_host, float* y_host, float* loss_host, int64_t B) {

@@ -272,8 +272,39 @@ bool fused_fits(int M, int N, int K, int num_sms);   // can the fused training e
 int sqerr_accumulate(const float* y, const float* t, size_t n, double* acc, cudaStream_t st);
 int l2persist_acquire(int dev, size_t bytes);                // mlp_tc.cu: persisting-L2 set-aside for the fused inference kernel
 int l2persist_release(int dev);                              // ... handed back (training steps want the whole L2)
+bool l2persist_held(int dev, size_t bytes);                  // ... currently set aside, at least `bytes`
 int mark_model_work(p3d_model* m, cudaStream_t st);          // record ev_done on st
 int order_after_model_work(p3d_model* m, cudaStream_t st);   // st waits for the last recorded ev_done
+// CUDA-graph capture (include/p3d.h, "CUDA graphs"): a call on a capturing stream may not allocate, free or
+// synchronise.  capturing(st): st is capturing now.  refuse_in_capture(st, what): P3D_OK when st is not capturing,
+// otherwise P3D_ERR_STATE with a message that names `what` and the warm-up rule.
+bool capturing(cudaStream_t st);
+int refuse_in_capture(cudaStream_t st, const char* what);
+// a growable scratch buffer is being replaced by a larger one: freed at once while no graph can hold its address,
+// kept until p3d_model_destroy once the model has been captured
+void retire(p3d_model* m, void* p);
+// new capacity (rows) of a growable scratch buffer that holds `cap` rows and must hold `need`: exactly `need` while
+// superseded buffers are freed at once; once they are kept, at least twice the old capacity, so that what is kept
+// stays below the live buffer's size
+int64_t grown_cap(const p3d_model* m, int64_t cap, int64_t need);
+
+// Exchange tags of the whole-chip inference kernels (p3d_model::xchg: [0] epoch, [32] arrival counter).  Every thread
+// loads the epoch at kernel entry (xchg_tag: tag = epoch + 1, never 0).  Once every thread of a CTA has used its tag
+// (compared it in the first gather), one thread arrives (xchg_arrive); the CTA that arrives last resets the counter and advances the epoch
+// (xchg_advance).  All CTAs have read the epoch by then, and the next launch on the stream sees the new value, so no
+// two launches - eager calls or graph replays, in any order - share a tag.
+__device__ __forceinline__ unsigned xchg_tag(const unsigned* xchg) {
+  unsigned e;
+  asm volatile("ld.relaxed.gpu.global.u32 %0, [%1];" : "=r"(e) : "l"(xchg) : "memory");
+  return e + 1u;
+}
+// The compiler aggregates the arrival per warp and waits for its result at once: one contended L2 round trip for the
+// arriving warp, so the kernels arrive just before a gather, where the warp waits for other CTAs' outputs anyway.
+__device__ __forceinline__ unsigned xchg_arrive(unsigned* xchg) { return atomicAdd(xchg + 32, 1u); }
+__device__ __forceinline__ void xchg_advance(unsigned* xchg, unsigned tag) {
+  asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(xchg + 32), "r"(0u) : "memory");
+  asm volatile("st.relaxed.gpu.global.u32 [%0], %1;" ::"l"(xchg), "r"(tag == 0xFFFFFFFFu ? 0u : tag) : "memory");
+}
 
 }  // namespace p3d
 
@@ -294,7 +325,7 @@ struct p3d_model {
   // inference pack
   bool pack_valid = false;
   int rows_total = 0;      // sum of N over layers
-  int kpad = 0;            // row pitch (elements) of wt_bf16 = max(L,64)
+  int kpad = 0;            // row pitch (elements) of wt_bf16 = max(L rounded up to 8, 64)
   __nv_bfloat16* wt_bf16 = nullptr;  // [rows_total][kpad], K-major, BN+clip folded
   float* bias_fold = nullptr;        // [rows_total]
   float* wfold = nullptr;            // fp32 folded [K,N] per layer, concatenated
@@ -312,13 +343,19 @@ struct p3d_model {
   const void* lay_x = nullptr;
   __nv_bfloat16* lay_act = nullptr;      // [2][lay_cap][L] bf16
   int64_t lay_cap = 0;
-  unsigned long long* lat_counter = nullptr;   // grid-barrier counter of the latency kernel (monotonic)
+  unsigned long long* lat_counter = nullptr;   // grid-barrier counter of the latency kernel (monotonic), [8..] stamps
   unsigned long long lat_base = 0;
-  void* lat_act = nullptr;               // batch-1 whole-chip kernel: activation exchange words {value, tag} [16][1024]
-  unsigned lat_tag = 0;                  // ... and its call counter
+  void* lat_act = nullptr;               // 1 .. 8 poses whole-chip kernel (mlp_simt.cu): exchange words {value, tag}, 8 MB
   void* mid_act = nullptr;               // 9 .. 64 poses whole-chip kernel (mlp_mid.cu): exchange words {bf16 pair, tag} [8][64][512]
-  float* f32_a = nullptr;                // fp32-path activations [3][cap][L]
+  // Exchange tags of both whole-chip kernels, in device memory: [0] epoch, [32] arrival counter.  Every CTA of a launch
+  // reads the epoch at entry (tag = epoch + 1, never 0); the last CTA to finish resets the counter and advances the
+  // epoch, so every launch - eager or a graph replay - uses a tag no earlier launch used.
+  unsigned* xchg = nullptr;
+  float* f32_a = nullptr;                // fp32-path activations [2][cap][L]
   int64_t f32_cap = 0;
+  // growable scratch that a captured graph may still address (retire()): freed by p3d_model_destroy
+  bool captured = false;                 // a call of this model has run on a capturing stream
+  std::vector<void*> retired;
   // host-step pipeline
   cudaStream_t pipe_streams[3] = {nullptr, nullptr, nullptr};
   float* pipe_x[3] = {nullptr, nullptr, nullptr};

@@ -7,7 +7,9 @@
 // Why: a single 128-pose tile walks the six layers of the persistent kernel in ~100 us - one SM (pair) has
 // to stream all 8.6 MB of weights by itself.  Splitting every layer over N (L/64 CTAs) spreads the weight
 // stream over 16+ SMs; the layers are separate launches whose plans (tensor maps + parameters) are cached
-// per batch size, so a call costs 1 + nlayers back-to-back launches and no host-side encoding.
+// per batch size, so a call costs 1 + nlayers back-to-back launches and no host-side encoding.  The plans are kernel
+// parameters (tensor maps by value), so a captured graph keeps its own copy; the buffers they address are never freed
+// while a graph may hold them (retire()).
 #include "common.cuh"
 
 namespace p3d {
@@ -47,9 +49,10 @@ int forward(p3d_model* m, const __nv_bfloat16* xb, float* y, int64_t B, cudaStre
   P3D_REQUIRE(B <= 0x7fffffff, "layered path: batch too large");
   bool rebuild = (m->lay_B != B) || (m->lay_x != xb) || m->lay_plans.empty();
   if (m->lay_cap < B) {
-    if (m->lay_act) cudaFree(m->lay_act);
+    P3D_TRY(refuse_in_capture(st, "forward: growing the layered path's activation buffers"));
+    const int64_t cap = grown_cap(m, m->lay_cap, B < 1024 ? 1024 : B);
+    retire(m, m->lay_act);
     m->lay_act = nullptr; m->lay_cap = 0;
-    const int64_t cap = B < 1024 ? 1024 : B;
     P3D_CUDA(cudaMalloc(&m->lay_act, sizeof(__nv_bfloat16) * 2ull * cap * L));
     m->lay_cap = cap;
     rebuild = true;

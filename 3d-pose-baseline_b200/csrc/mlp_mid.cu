@@ -14,9 +14,11 @@
 //   math     mma.sync.m16n8k16 bf16 -> fp32 (legacy tensor-core path: a 32 x 16 x 1024 problem per CTA and layer is far
 //            below what tcgen05 needs to pay for its TMEM round trip); the 8 warps split K, partial sums meet in
 //            shared memory
-//   exchange act[layer][pose][512] words {2 x bf16, call tag}: a producer stores each word with ONE 8-byte store, the
-//            consumers poll the words they need until they carry this call's tag (no flag, no fence: an 8-byte
-//            aligned access is single-copy atomic); the tag is the model's call counter, so nothing is ever cleared
+//   exchange act[layer][pose][512] words {2 x bf16, launch tag}: a producer stores each word with ONE 8-byte store, the
+//            consumers poll the words they need until they carry this launch's tag (no flag, no fence: an 8-byte
+//            aligned access is single-copy atomic); the tag comes from the model's epoch word in device memory, which
+//            every launch advances on its way out (xchg_tag in common.cuh), so nothing is ever cleared and a launch
+//            captured into a CUDA graph gets a fresh tag on every replay
 //   rounding the same points as the tcgen05 paths (x, every ReLU output and every residual sum rounded to bf16, fp32
 //            accumulation): tests/helpers.py:emulate_bf16_forward
 #include "common.cuh"
@@ -34,7 +36,7 @@ constexpr int NOUT = 8;                   // output-layer features per CTA (one 
 struct Args {
   const float* x; float* y; const __nv_bfloat16* wt; const float* bias;
   unsigned long long* act;                // [nlayers - 1][64 poses][512] {bf16 pair, tag}
-  unsigned tag;
+  unsigned* xchg;                         // epoch + arrival counter (p3d_model::xchg)
   int nlayers, out, kpad, residual, rows;
   int sentinel;                           // poll one pose until it arrives before requesting the batch (diagnostics switch)
   unsigned long long* stamps;             // optional [16] %globaltimer stamps of CTA 0 (P3D_LAT_STAMPS=1, tools/bench_latency.py)
@@ -101,6 +103,8 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
   const int out_rows = has_out ? min(NOUT, a.out - fg * NOUT) : 0;
 
   MID_STAMP(0);
+  const unsigned tag = xchg_tag(a.xchg);                       // in flight with the weight copies; first used by layer 0's stores
+  unsigned arrived = 0;                                        // thread 0: CTAs that arrived before this one
   if (tid == 0) {
     for (int l = 0; l <= nhid; ++l) mbar_init(&wbar[l], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -155,7 +159,7 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
     }
     const float v0 = bf16r(fmaxf(acc0 + __ldg(a.bias + n), 0.f)), v1 = bf16r(fmaxf(acc1 + __ldg(a.bias + n + 1), 0.f));
     sres[er * NF + 2 * ej] = v0; sres[er * NF + 2 * ej + 1] = v1;             // block input of the first residual block
-    if (er < live) st_word(words(0, row0 + er) + fg * (NF / 2) + ej, pack_bf16(v0, v1), a.tag);
+    if (er < live) st_word(words(0, row0 + er) + fg * (NF / 2) + ej, pack_bf16(v0, v1), tag);
   }
   MID_STAMP(1);
 
@@ -175,7 +179,7 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
       unsigned long long s0, s1;
       for (;;) {
         ld_words(src, s0, s1);
-        if (static_cast<uint32_t>(s0 >> 32) == a.tag && static_cast<uint32_t>(s1 >> 32) == a.tag) break;
+        if (static_cast<uint32_t>(s0 >> 32) == tag && static_cast<uint32_t>(s1 >> 32) == tag) break;
         if (++spins > (1u << 24)) { printf("p3d: mid-batch kernel: layer %d never arrived (block %d)\n", lp, (int)blockIdx.x); __trap(); }
       }
     }
@@ -190,7 +194,7 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
           if (b * 16 + r < live) ld_words(src + static_cast<size_t>(b * 16 + r) * 512, w0[r], w1[r]);
 #pragma unroll
         for (int r = 0; r < 16; ++r)
-          if (b * 16 + r < live) ok = ok && static_cast<uint32_t>(w0[r] >> 32) == a.tag && static_cast<uint32_t>(w1[r] >> 32) == a.tag;
+          if (b * 16 + r < live) ok = ok && static_cast<uint32_t>(w0[r] >> 32) == tag && static_cast<uint32_t>(w1[r] >> 32) == tag;
         if (ok) break;
         if (++spins > (1u << 24)) { printf("p3d: mid-batch kernel: layer %d never arrived (block %d)\n", lp, (int)blockIdx.x); __trap(); }
       }
@@ -241,6 +245,8 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
   // ---- hidden layers 1 .. nhid.  The residual of an even layer is the block input (output of layer l - 2), whose 16
   // features of this row group the CTA produced itself: sres.
   for (int l = 1; l <= nhid; ++l) {
+    // every thread of the CTA has compared its tag in the first gather: arrive, while the outputs of layer 1 are on their way
+    if (l == 2 && tid == 0) arrived = xchg_arrive(a.xchg);
     gather(l - 1);
     __syncthreads();
     mbar_wait(&wbar[l - 1], 0);
@@ -268,12 +274,13 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
         if (a.residual) { v0 = bf16r(v0 + sres[er * NF + 2 * ej]); v1 = bf16r(v1 + sres[er * NF + 2 * ej + 1]); }
         sres[er * NF + 2 * ej] = v0; sres[er * NF + 2 * ej + 1] = v1;
       }
-      if (er < live) st_word(words(l, row0 + er) + fg * (NF / 2) + ej, pack_bf16(v0, v1), a.tag);
+      if (er < live) st_word(words(l, row0 + er) + fg * (NF / 2) + ej, pack_bf16(v0, v1), tag);
     }
     __syncthreads();                                           // the next gather overwrites the scratch
     MID_STAMP(1 + l);
   }
   // ---- output layer: feature group fg < ceil(out / 8) computes 8 features for its row group
+  if (nhid < 2 && tid == 0) arrived = xchg_arrive(a.xchg);
   if (has_out) {
     gather(nhid);
     __syncthreads();
@@ -298,6 +305,7 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
       if (r < live && n < a.out) a.y[static_cast<size_t>(row0 + r) * a.out + n] = s + __ldg(a.bias + (a.nlayers - 1) * 1024 + n);
     }
   }
+  if (tid == 0 && arrived == gridDim.x - 1) xchg_advance(a.xchg, tag);
   MID_STAMP(a.nlayers);
 }
 
@@ -311,31 +319,21 @@ int forward(p3d_model* m, const float* x, float* y, int rows, cudaStream_t st) {
   const int mt = rows > 32 ? 2 : 1;
   const int groups = (rows + 16 * mt - 1) / (16 * mt);
   if (m->num_sms < NFG * groups) return 1;
+  if (!m->mid_act) return 1;                            // allocated (2 MB, zero) by p3d_model_create for width 1024 / bf16
   static PerDeviceOnce attr;
   if (attr.needed()) {
+    P3D_TRY(refuse_in_capture(st, "forward: first use of the 9-64 pose whole-chip kernel on this device"));
     P3D_CUDA(cudaFuncSetAttribute(mid_grid_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(1)));
     P3D_CUDA(cudaFuncSetAttribute(mid_grid_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(2)));
     attr.mark();
   }
-  if (!m->mid_act) {
-    const size_t bytes = sizeof(unsigned long long) * 8 * 64 * 512;       // up to 8 layers of outputs
-    P3D_CUDA(cudaMalloc(&m->mid_act, bytes));
-    P3D_CUDA(cudaMemsetAsync(m->mid_act, 0, bytes, st));
-  }
-  if (++m->lat_tag == 0) ++m->lat_tag;                  // 0 is what a fresh buffer holds
   Args a;
-  a.x = x; a.y = y; a.wt = m->wt_bf16; a.bias = m->bias_fold; a.act = static_cast<unsigned long long*>(m->mid_act); a.tag = m->lat_tag;
+  a.x = x; a.y = y; a.wt = m->wt_bf16; a.bias = m->bias_fold; a.act = static_cast<unsigned long long*>(m->mid_act); a.xchg = m->xchg;
   a.nlayers = nlayers; a.out = m->out_size; a.kpad = m->kpad; a.residual = m->cfg.residual; a.rows = rows;
   static const int sentinel = [] { const char* e = getenv("P3D_MID_SENTINEL"); return e ? atoi(e) : 1; }();
   a.sentinel = sentinel;
   a.stamps = nullptr;
-  if (getenv("P3D_LAT_STAMPS")) {
-    if (!m->lat_counter) {
-      P3D_CUDA(cudaMalloc(&m->lat_counter, sizeof(unsigned long long) * 32));
-      P3D_CUDA(cudaMemset(m->lat_counter, 0, sizeof(unsigned long long) * 32));
-    }
-    a.stamps = m->lat_counter + 8;
-  }
+  if (getenv("P3D_LAT_STAMPS")) a.stamps = m->lat_counter + 8;
   cudaLaunchConfig_t cfg{};
   cfg.gridDim = dim3(NFG * groups); cfg.blockDim = dim3(MGT); cfg.dynamicSmemBytes = smem_bytes(mt); cfg.stream = st;
   cudaLaunchAttribute at[1];

@@ -118,15 +118,22 @@ int sgemm(bool ta, bool tb, int64_t M, int N, int K, const float* A, int lda, co
   return P3D_OK;
 }
 
-// fp32-mode inference through the folded fp32 weights; activations in three [cap,L] fp32 buffers
+// fp32 activations P | Q of at least `rows` rows each (m->f32_a, [2][f32_cap][L])
+static int ensure_f32(p3d_model* m, int64_t rows, cudaStream_t st) {
+  if (m->f32_cap >= rows) return P3D_OK;
+  P3D_TRY(refuse_in_capture(st, "forward: growing the fp32 activation buffers"));
+  const int64_t cap = grown_cap(m, m->f32_cap, rows);
+  retire(m, m->f32_a);
+  m->f32_a = nullptr; m->f32_cap = 0;
+  P3D_CUDA(cudaMalloc(&m->f32_a, sizeof(float) * 2ull * cap * m->L));
+  m->f32_cap = cap;
+  return P3D_OK;
+}
+
+// fp32-mode inference through the folded fp32 weights; activations in two [cap,L] fp32 buffers
 int forward_fp32(p3d_model* m, const float* x, float* y, int64_t B, cudaStream_t st) {
   const int L = m->L;
-  if (m->f32_cap < B) {
-    if (m->f32_a) cudaFree(m->f32_a);
-    m->f32_a = nullptr; m->f32_cap = 0;
-    P3D_CUDA(cudaMalloc(&m->f32_a, sizeof(float) * 2ull * B * L));
-    m->f32_cap = B;
-  }
+  P3D_TRY(ensure_f32(m, B, st));
   float* P = m->f32_a;
   float* Q = m->f32_a + static_cast<size_t>(m->f32_cap) * L;
   const int nl = static_cast<int>(m->layers.size());
@@ -171,6 +178,13 @@ __global__ void __launch_bounds__(256) small_batch_layer_kernel(const float* __r
 #pragma unroll
   for (int r = 0; r < ROWS; ++r) acc[r] = 0.f;
   for (int k = lane * 8; k < K; k += 256) {
+    if (k + 8 > K) {       // the ragged tail of a width that is not a multiple of 8 (kpad is): element by element
+#pragma unroll
+      for (int r = 0; r < ROWS; ++r)
+        if (r < rows)
+          for (int i = 0; i < K - k; ++i) acc[r] = fmaf(hin[static_cast<size_t>(r) * ldin + k + i], __bfloat162float(wrow[k + i]), acc[r]);
+      continue;
+    }
     const uint4 wv = __ldg(reinterpret_cast<const uint4*>(wrow + k));
     const __nv_bfloat162* w2 = reinterpret_cast<const __nv_bfloat162*>(&wv);
     float w[8];
@@ -331,16 +345,7 @@ static int launch_latency(p3d_model* m, LatArgs& a, cudaStream_t st) {
 
 int forward_latency(p3d_model* m, const float* x, float* y, int64_t B, cudaStream_t st) {
   const int L = m->L;
-  if (m->f32_cap < SB_ROWS) {
-    if (m->f32_a) cudaFree(m->f32_a);
-    m->f32_a = nullptr; m->f32_cap = 0;
-    P3D_CUDA(cudaMalloc(&m->f32_a, sizeof(float) * 2ull * SB_ROWS * L));
-    m->f32_cap = SB_ROWS;
-  }
-  if (!m->lat_counter) {
-    P3D_CUDA(cudaMalloc(&m->lat_counter, sizeof(unsigned long long) * 32));
-    P3D_CUDA(cudaMemset(m->lat_counter, 0, sizeof(unsigned long long) * 32));
-  }
+  P3D_TRY(ensure_f32(m, SB_ROWS, st));
   for (int64_t r0 = 0; r0 < B; r0 += SB_ROWS) {
     LatArgs a;
     a.rows = static_cast<int>(B - r0 < SB_ROWS ? B - r0 : SB_ROWS);
@@ -570,6 +575,7 @@ static int launch_latency_cluster(p3d_model* m, const float* x, float* y, const 
   int& okd = ok_dev[m->cfg.device & 63];
   int ok = okd == 1 ? 1 : (okd == 2 ? 0 : -1);
   if (ok < 0) {
+    P3D_TRY(refuse_in_capture(st, "forward: probing the 16-CTA cluster kernel"));
     ok = 0;
     if (cudaFuncSetAttribute(latency_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess &&
         cudaFuncSetAttribute(latency_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LAT_SMEM) == cudaSuccess) {
@@ -587,10 +593,6 @@ static int launch_latency_cluster(p3d_model* m, const float* x, float* y, const 
   }
   if (!ok || m->layers.size() < 3) return 1;       // caller falls back to the per-layer kernels
   LatArgs a;
-  if (!m->lat_counter) {
-    P3D_CUDA(cudaMalloc(&m->lat_counter, sizeof(unsigned long long) * 32));
-    P3D_CUDA(cudaMemset(m->lat_counter, 0, sizeof(unsigned long long) * 32));
-  }
   if (f) a.rt = *f;
   a.rows = 1; a.x = x; a.y = y; a.wt = m->wt_bf16; a.bias = m->bias_fold; a.hP = a.hQ = nullptr; a.counter = nullptr; a.base = 0;
   a.stamps = getenv("P3D_LAT_STAMPS") ? m->lat_counter + 8 : nullptr;
@@ -612,16 +614,18 @@ static int launch_latency_cluster(p3d_model* m, const float* x, float* y, const 
 // launch: all resident) own 8 output features of every layer each: a CTA's whole share of the weights is 64 KB and is
 // requested in the first instructions (the chip pulls the 8.56 MB in parallel, ~2 us), so what remains is the layer
 // chain itself.  Activations travel between the layers through a global buffer of self-validating words {fp32 value,
-// call tag}: a producer stores its feature with one 8-byte store, every consumer polls the words it needs until they
-// carry this call's tag - no counter, no fence, no barrier: one L2 write + read per layer (~1 us) instead of the
-// ~3 us round trips of a grid-wide barrier.  The tag is a per-model call counter, so the buffer is never cleared.
+// launch tag}: a producer stores its feature with one 8-byte store, every consumer polls the words it needs until they
+// carry this launch's tag - no counter, no fence, no barrier: one L2 write + read per layer (~1 us) instead of the
+// ~3 us round trips of a grid-wide barrier.  The tag comes from the model's epoch word in device memory (xchg_tag in
+// common.cuh), which every launch advances on its way out, so the buffer is never cleared and a launch captured into a
+// CUDA graph gets a fresh tag on every replay.
 constexpr int GLC = 128;          // CTAs
 constexpr int GLT = 256;          // threads: 8 warps, one output feature per warp and layer
 constexpr int GLF = GLT / 32;     // features per CTA and layer
 struct GridLatArgs {
   const float* x; float* y; const __nv_bfloat16* wt; const float* bias;
   uint2* act;                     // [nlayers - 1][8 poses][1024] {value bits, tag}
-  unsigned tag;
+  unsigned* xchg;                 // epoch + arrival counter (p3d_model::xchg)
   int nlayers, out, kpad, residual, rows, backoff_ns;
   unsigned long long* stamps;
 };
@@ -647,6 +651,8 @@ __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs 
   float* sQ = sP + ROWS * L;
   uint64_t* wbar = reinterpret_cast<uint64_t*>(sQ + ROWS * L);     // [nhid + 1]
   GLAT_STAMP(0);
+  const unsigned tag = xchg_tag(a.xchg);                            // in flight with the weight copies; first used by layer 0's publish
+  unsigned arrived = 0;                                             // thread 0: CTAs that arrived before this one
   if (threadIdx.x == 0) {
     for (int l = 0; l <= nhid; ++l) lat_mbar_init(&wbar[l], 1);
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
@@ -669,8 +675,8 @@ __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs 
       const int r = threadIdx.x >> 2, q = threadIdx.x & 3;
       if (r < a.rows) {
         uint2* dst = word(l, r) + c * GLF + 2 * q;
-        asm volatile("st.volatile.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "r"(__float_as_uint(spub[r][2 * q])), "r"(a.tag),
-                     "r"(__float_as_uint(spub[r][2 * q + 1])), "r"(a.tag) : "memory");
+        asm volatile("st.volatile.global.v4.u32 [%0], {%1, %2, %3, %4};" ::"l"(dst), "r"(__float_as_uint(spub[r][2 * q])), "r"(tag),
+                     "r"(__float_as_uint(spub[r][2 * q + 1])), "r"(tag) : "memory");
       }
     }
   };
@@ -708,7 +714,7 @@ __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs 
         u[r] = ld_ll2(src); v[r] = ld_ll2(src + 2);
       }
 #pragma unroll
-      for (int r = 0; r < ROWS; ++r) ok = ok && u[r].y == a.tag && u[r].w == a.tag && v[r].y == a.tag && v[r].w == a.tag;
+      for (int r = 0; r < ROWS; ++r) ok = ok && u[r].y == tag && u[r].w == tag && v[r].y == tag && v[r].w == tag;
       if (ok) break;
       if (++spins > (1u << 24)) { printf("p3d: batch-1 kernel: layer %d never arrived (block %d)\n", lp, (int)blockIdx.x); __trap(); }
       // back off between polls: 32 K threads re-reading the same 8 KB as fast as they can keep the L2 slices that hold it
@@ -726,6 +732,8 @@ __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs 
     float* src = (l & 1) ? sP : sQ;
     const bool add_res = a.residual && l >= 2 && !(l & 1);
     const float bias = __ldg(a.bias + l * L + n);
+    // every thread of the CTA has compared its tag in the first gather: arrive, while the outputs of layer 1 are on their way
+    if (l == 2 && threadIdx.x == 0) arrived = xchg_arrive(a.xchg);
     gather(l - 1, src);
     __syncthreads();
     lat_mbar_wait(&wbar[l - 1], 0);
@@ -760,6 +768,7 @@ __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs 
     GLAT_STAMP(1 + l);
   }
   // ---- output layer: CTA c < out computes feature c from its row in shared memory
+  if (nhid < 2 && threadIdx.x == 0) arrived = xchg_arrive(a.xchg);
   if (c < a.out) {
     const int l = a.nlayers - 1;
     float* src = (l & 1) ? sP : sQ;
@@ -781,6 +790,7 @@ __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs 
       if (lane == 0) a.y[warp * a.out + c] = acc + __ldg(a.bias + l * L + c);
     }
   }
+  if (threadIdx.x == 0 && arrived == gridDim.x - 1) xchg_advance(a.xchg, tag);
   GLAT_STAMP(a.nlayers);
 }
 
@@ -795,25 +805,17 @@ static int launch_latency_grid(p3d_model* m, const float* x, float* y, int rows,
   const int smem = 128 + nhid * (GLF * 2048) + 2048 + 2 * R * 1024 * 4 + 8 * (nhid + 1) + 64;
   using K = void (*)(const GridLatArgs);
   const K fn = R == 1 ? latency_grid_kernel<1> : (R == 2 ? latency_grid_kernel<2> : (R == 4 ? latency_grid_kernel<4> : latency_grid_kernel<8>));
+  if (!m->lat_act) return 1;                           // allocated (8 MB, zero) by p3d_model_create for width 1024 / bf16
   static PerDeviceOnce attr;
   if (attr.needed()) {
+    P3D_TRY(refuse_in_capture(st, "forward: first use of the whole-chip kernel on this device"));
     const int cap = 128 + 6 * (GLF * 2048) + 2048 + 2 * 8 * 1024 * 4 + 256;
     for (K k : {static_cast<K>(latency_grid_kernel<1>), static_cast<K>(latency_grid_kernel<2>), static_cast<K>(latency_grid_kernel<4>), static_cast<K>(latency_grid_kernel<8>)})
       P3D_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
     attr.mark();
   }
-  if (!m->lat_act) {
-    // one pose: [128 consumer CTAs][layers <= 8][1024] (8 MB); more poses: [layers <= 8][poses 8][1024] in the same buffer
-    P3D_CUDA(cudaMalloc(&m->lat_act, sizeof(uint2) * 1024 * 8 * GLC));
-    P3D_CUDA(cudaMemset(m->lat_act, 0, sizeof(uint2) * 1024 * 8 * GLC));
-  }
-  if (!m->lat_counter) {
-    P3D_CUDA(cudaMalloc(&m->lat_counter, sizeof(unsigned long long) * 32));
-    P3D_CUDA(cudaMemset(m->lat_counter, 0, sizeof(unsigned long long) * 32));
-  }
-  if (++m->lat_tag == 0) ++m->lat_tag;                 // 0 is what a fresh buffer holds
   GridLatArgs a;
-  a.x = x; a.y = y; a.wt = m->wt_bf16; a.bias = m->bias_fold; a.act = static_cast<uint2*>(m->lat_act); a.tag = m->lat_tag;
+  a.x = x; a.y = y; a.wt = m->wt_bf16; a.bias = m->bias_fold; a.act = static_cast<uint2*>(m->lat_act); a.xchg = m->xchg;
   a.nlayers = nlayers; a.out = m->out_size; a.kpad = m->kpad; a.residual = m->cfg.residual; a.rows = rows;
   static const int backoff = [] { const char* e = getenv("P3D_LAT_BACKOFF_NS"); return e ? atoi(e) : 0; }();
   a.backoff_ns = backoff;
@@ -845,12 +847,7 @@ int forward_latency_cluster_rt(p3d_model* m, const rt::Fused& f, float* y, cudaS
 
 int forward_small(p3d_model* m, const float* x, float* y, int64_t B, cudaStream_t st) {
   const int L = m->L;
-  if (m->f32_cap < SB_ROWS) {
-    if (m->f32_a) cudaFree(m->f32_a);
-    m->f32_a = nullptr; m->f32_cap = 0;
-    P3D_CUDA(cudaMalloc(&m->f32_a, sizeof(float) * 2ull * SB_ROWS * L));
-    m->f32_cap = SB_ROWS;
-  }
+  P3D_TRY(ensure_f32(m, SB_ROWS, st));
   float* P = m->f32_a;
   float* Q = m->f32_a + static_cast<size_t>(m->f32_cap) * L;
   const int nl = static_cast<int>(m->layers.size());

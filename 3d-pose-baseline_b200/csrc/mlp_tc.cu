@@ -40,6 +40,9 @@ int l2persist_acquire(int dev, size_t bytes) {
   g_l2_set_aside[dev].store(bytes, std::memory_order_release);
   return P3D_OK;
 }
+bool l2persist_held(int dev, size_t bytes) {
+  return dev >= 0 && dev < 64 && g_l2_set_aside[dev].load(std::memory_order_acquire) >= bytes;
+}
 int l2persist_release(int dev) {
   if (dev < 0 || dev >= 64 || g_l2_set_aside[dev].load(std::memory_order_acquire) == 0) return P3D_OK;
   cudaCtxResetPersistingL2Cache();
@@ -472,7 +475,10 @@ static int launch_forward(p3d_model* m, const __nv_bfloat16* xb, float* y, int64
   // traffic per 2^20-pose launch against 0.34 GB of compulsory x / y bytes.  An access-policy window on the scratch with
   // a persisting-L2 set-aside keeps those lines resident: 2.42 GB, and 156.6 -> 159.7 M poses/s on the same box
   // (round 2, profiles/r2_l2persist.md).  P3D_L2_PERSIST=0 switches it off.
+  // Under graph capture nothing host-side may change: the window goes into the graph only while the set-aside is held.
+  // A replay after a training step has handed the set-aside back is slower (the scratch competes for the L2), not wrong.
   static const bool l2_persist = [] { const char* e = getenv("P3D_L2_PERSIST"); return !(e && e[0] == '0'); }();
+  const bool cap = capturing(st);
   if (l2_persist) {
     int dev = 0, max_persist = 0, max_window = 0;
     P3D_CUDA(cudaGetDevice(&dev));
@@ -481,8 +487,9 @@ static int launch_forward(p3d_model* m, const __nv_bfloat16* xb, float* y, int64
     const size_t scratch = sizeof(__nv_bfloat16) * 2ull * grid * BM * L;
     // only when the whole scratch fits the set-aside (width 1024: 77.6 MB); a partial window over the 310 MB of the
     // width-4096 model bought nothing and cost the weights their L2 share (0.73 -> 0.65 of peak)
-    if (scratch <= static_cast<size_t>(max_persist) && scratch <= static_cast<size_t>(max_window)) {
-      P3D_TRY(l2persist_acquire(dev, scratch));
+    if (scratch <= static_cast<size_t>(max_persist) && scratch <= static_cast<size_t>(max_window) &&
+        (!cap || l2persist_held(dev, scratch))) {
+      if (!cap) P3D_TRY(l2persist_acquire(dev, scratch));
       attr[1].id = cudaLaunchAttributeAccessPolicyWindow;
       attr[1].val.accessPolicyWindow.base_ptr = m->act_scratch;
       attr[1].val.accessPolicyWindow.num_bytes = scratch;
@@ -493,7 +500,7 @@ static int launch_forward(p3d_model* m, const __nv_bfloat16* xb, float* y, int64
     }
   }
   cudaEvent_t e0 = nullptr, e1 = nullptr;
-  if (prof::enabled()) prof::begin(st, &e0, &e1);
+  if (prof::enabled() && !cap) prof::begin(st, &e0, &e1);     // timing events are read on the host: eager launches only
   P3D_CUDA(cudaLaunchKernelEx(&cfg, mlp_forward_tc_kernel<CG>, tm_x, tm_act, tm_w, tm_wout, p));
   P3D_LAUNCH_CHECK();
   if (e0) prof::end(st, e0, e1);
@@ -505,6 +512,7 @@ int forward_bf16(p3d_model* m, const __nv_bfloat16* xb, float* y, int64_t B, cud
   P3D_REQUIRE(L % BN == 0 && L / 64 <= MAX_SLABS, "bf16 tensor-core path needs linear_size %% 256 == 0 and <= 4096 (got %d)", L);
   // per-CTA activation scratch, sized for a full grid once
   if (m->act_grid < m->num_sms) {
+    P3D_TRY(refuse_in_capture(st, "forward: allocating the fused kernel's activation scratch"));
     if (m->act_scratch) cudaFree(m->act_scratch);
     P3D_CUDA(cudaMalloc(&m->act_scratch, sizeof(__nv_bfloat16) * 2ull * m->num_sms * BM * L));
     m->act_grid = m->num_sms;

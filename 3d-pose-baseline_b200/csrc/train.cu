@@ -1073,6 +1073,10 @@ int p3d_model_train_step(p3d_model* m, const float* x, const float* t, int64_t B
   if (global_B <= 0) global_B = B;
   P3D_REQUIRE(m->world > 1 || global_B == B, "train_step: global_B != B without a communicator");
   P3D_CUDA(cudaSetDevice(m->cfg.device));
+  if (capturing(static_cast<cudaStream_t>(stream))) {      // the step captures and replays CUDA graphs of its own
+    set_error("train_step cannot be captured into a CUDA graph (only inference calls can)");
+    return P3D_ERR_STATE;
+  }
   return train::train_step(m, x, t, B, keep_prob, seed, mask_or_null, global_B, row0, loss, lr_used, y, static_cast<cudaStream_t>(stream));
 }
 
@@ -1082,6 +1086,10 @@ int p3d_model_train_epoch(p3d_model* m, const float* X, const float* T, int64_t 
   P3D_REQUIRE(batch_size >= 1 && n >= 0, "train_epoch: bad sizes");
   P3D_REQUIRE(keep_prob > 0.f && keep_prob <= 1.f, "train_epoch: dropout_keep_prob must be in (0,1]");
   P3D_CUDA(cudaSetDevice(m->cfg.device));
+  if (capturing(static_cast<cudaStream_t>(stream))) {
+    set_error("train_epoch cannot be captured into a CUDA graph (only inference calls can)");
+    return P3D_ERR_STATE;
+  }
   return train::train_epoch(m, X, T, n, reinterpret_cast<const long long*>(perm_or_null), batch_size, keep_prob, seed, losses,
                             lr_last_or_null, static_cast<cudaStream_t>(stream));
 }

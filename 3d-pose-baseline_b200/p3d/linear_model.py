@@ -234,6 +234,15 @@ class LinearModel(object):
         for n, v in values.items():
             self.set_variable(n, v)
 
+    def prepare_inference(self):
+        """Fold clip_by_norm and the BatchNorm statistics into the packed inference weights now, on the current torch
+        stream (p3d_model_prepare_inference).  Inference does this by itself after set_variable, restore or a training
+        step, but not inside a CUDA graph capture; the fold rewrites the packed weights in place, so graphs captured
+        earlier see the new weights on their next replay.  Call it outside any capture."""
+        torch = _lib.require_cuda()
+        with torch.cuda.device(self.device):
+            check(lib.p3d_model_prepare_inference(self._handle, _lib.current_stream()))
+
     # tf.train.Saver stand-in (linear_model.py:151; predict_3dpose.py:158-186,328): one .npz keyed by TF names
     def save(self, path):
         path = path if path.endswith(".npz") else path + ".npz"      # np.savez would append it silently

@@ -14,6 +14,25 @@
  *     asynchronous on that stream unless they take/return host data.
  *   - handles are not thread-safe; distinct handles may be used from distinct threads.
  *   - there is NO CPU fallback: without a CUDA device every compute call fails with P3D_ERR_CUDA.
+ *
+ * CUDA graphs
+ *   - capturable on a stream in capture (cudaStreamBeginCapture, torch.cuda.graph): p3d_model_forward,
+ *     p3d_model_mse and p3d_realtime_step, at any batch size, width and mode.  Every other call that takes a
+ *     model returns P3D_ERR_STATE on a capturing stream (training steps and epochs, prepare_inference) or is
+ *     synchronous and must not be called during a capture (host-buffer steps, the realtime host frame).
+ *   - warm-up: a call may allocate or grow scratch, or set up a kernel, the first time it meets a batch size.  On
+ *     a capturing stream it cannot, and returns P3D_ERR_STATE instead; run the same call once outside the capture
+ *     first (PyTorch's warm-up convention).
+ *   - weights: a graph reads the packed inference weights in place.  After set_param_host, a checkpoint restore
+ *     or a training step, call p3d_model_prepare_inference outside the capture before the next replay (a capture
+ *     while the fold is stale returns P3D_ERR_STATE rather than capturing the fold).
+ *   - the caller's buffers (x, y, t, loss, the realtime inputs and outputs) must outlive the graph; the library's
+ *     scratch does (buffers a graph may address are freed by p3d_model_destroy only; once a model has been
+ *     captured, growing scratch at least doubles, so what is kept stays below the size of the live buffer).
+ *   - a replay is ordered before later host-buffer steps and realtime host frames of the model, as eager calls
+ *     are.  Replays of graphs of ONE model must not run concurrently (they share the model's scratch): replay
+ *     them on one stream, or order them.  A replay after a training step has handed the fused kernel's
+ *     persisting-L2 set-aside back is slower, not different.
  */
 #ifndef P3D_H_
 #define P3D_H_
