@@ -283,9 +283,10 @@ mlp_forward_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_con
           const uint32_t acc = q & 1, aphase = (q >> 1) & 1;
           const int wrow0 = last ? (nlayers - 1) * L : l * L + c * BN;
           // bias of this chunk -> smem.  Double buffered: a fast warp may stage chunk q+1 while a slow one still
-          // reads chunk q; the named barrier below keeps everybody within one chunk of each other.
+          // reads chunk q; the named barrier below keeps everybody within one chunk of each other.  The output layer
+          // has only out_n packed rows (bias_fold ends 16 floats after them): its other rows stay unstaged, unread.
           float* sBias = sBiasAll + (q & 1) * BN;
-          sBias[row] = __ldg(p.bias + wrow0 + row);
+          if (!last || row < p.out_n) sBias[row] = __ldg(p.bias + wrow0 + row);
           if (!last) sBias[row + 128] = __ldg(p.bias + wrow0 + row + 128);
           named_bar_sync(1, 128);
           mbar_wait(&tfull[acc], aphase, 4);

@@ -291,6 +291,7 @@ __device__ __forceinline__ void totals_wait(const Params& p, int n0, int et, dou
 template <int OUT, bool RES, int CS>
 __global__ void __launch_bounds__((OUT >= 3) ? FUSED_NTHREADS : NTHREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
+  static_assert(CS == 0 || OUT < 2, "column sums are taken of the fp32 stores only");
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int STAGES = p.stages;
@@ -839,10 +840,6 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
           const int m = mrow0 + 4 * i;
           const bool live = m < p.M;
           float o[4] = {alpha * t4[i].x + b4.x, alpha * t4[i].y + b4.y, alpha * t4[i].z + b4.z, alpha * t4[i].w + b4.w};
-          if (CS == 1) {
-#pragma unroll
-            for (int j = 0; j < 4; ++j) { const float q = live ? o[j] : 0.f; cs1[j] += q; cs2[j] += q * q; }
-          }
           if (OUT == 2) {
             // bf16 activations of the layered inference path: same rounding points as the fused persistent kernel
             // (relu(.) rounded to bf16, then the residual added and rounded again)
@@ -859,6 +856,10 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
             if (live) *reinterpret_cast<uint2*>(p.out_b + static_cast<size_t>(m) * p.ldob + n) = q;
           } else {
             if (use_res) { o[0] += r4[i].x; o[1] += r4[i].y; o[2] += r4[i].z; o[3] += r4[i].w; }
+            if (CS == 1) {            // sums of the stored values: residual included
+#pragma unroll
+              for (int j = 0; j < 4; ++j) { const float q = live ? o[j] : 0.f; cs1[j] += q; cs2[j] += q * q; }
+            }
             float* crow = p.C + static_cast<size_t>(m) * p.ldc + n;
             if (live) {
               if (OUT == 1) asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(crow), "f"(o[0]), "f"(o[1]), "f"(o[2]), "f"(o[3]) : "memory");
@@ -881,13 +882,13 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
           for (int j = 0; j < 4; ++j) {
             if (n + j >= p.N) continue;
             float o = alpha * tv[j] + bias[j];
-            if (CS == 1) { cs1[j] += o; cs2[j] += o * o; }
             if (OUT == 2) {
               __nv_bfloat16 ob = __float2bfloat16_rn(p.relu ? fmaxf(o, 0.f) : o);
               if (use_res) ob = __float2bfloat16_rn(__bfloat162float(ob) + __bfloat162float(p.res_b[static_cast<size_t>(m) * p.ldrb + n + j]));
               p.out_b[static_cast<size_t>(m) * p.ldob + n + j] = ob;
             } else {
               if (use_res) o += __ldg(p.res + static_cast<size_t>(m) * p.ldres + n + j);
+              if (CS == 1) { cs1[j] += o; cs2[j] += o * o; }
               float* c = p.C + static_cast<size_t>(m) * p.ldc + n + j;
               if (OUT == 1) atomicAdd(c, o); else *c = o;
             }
