@@ -31,7 +31,8 @@ namespace simt { int forward_fp32(p3d_model*, const float*, float*, int64_t, cud
                  int forward_latency_cluster(p3d_model*, const float*, float*, cudaStream_t); }
 namespace mid { int forward(p3d_model*, const float*, float*, int, cudaStream_t); }
 namespace tcg { int mma_rate(int, int, long long*, cudaStream_t); }
-namespace layered { int forward(p3d_model*, const __nv_bfloat16*, float*, int64_t, cudaStream_t); }
+namespace layered { int forward(p3d_model*, const __nv_bfloat16*, float*, int64_t, cudaStream_t);
+                    int forward_split(p3d_model*, const float*, float*, int64_t, cudaStream_t); }
 namespace train { void free_workspace(p3d_model*); }
 
 constexpr int kSmallBatchMax = 16;   // rows served by the latency (GEMV) path
@@ -201,7 +202,7 @@ int p3d_model_create(const p3d_cfg* cfg, p3d_model** out) {
   P3D_REQUIRE(cfg && out, "model_create: null argument");
   P3D_REQUIRE(cfg->linear_size >= 16 && cfg->linear_size % 4 == 0, "linear_size must be a positive multiple of 4");
   P3D_REQUIRE(cfg->num_layers >= 0 && cfg->num_layers <= 64, "num_layers out of range");
-  P3D_REQUIRE(cfg->mode == P3D_MODE_BF16 || cfg->mode == P3D_MODE_FP32, "unknown mode %d", cfg->mode);
+  P3D_REQUIRE(cfg->mode == P3D_MODE_BF16 || cfg->mode == P3D_MODE_FP32 || cfg->mode == P3D_MODE_BF16X3, "unknown mode %d", cfg->mode);
   int ndev = 0;
   P3D_CUDA(cudaGetDeviceCount(&ndev));
   P3D_REQUIRE(cfg->device >= 0 && cfg->device < ndev, "device %d not present (%d devices)", cfg->device, ndev);
@@ -285,6 +286,10 @@ int p3d_model_create(const p3d_cfg* cfg, p3d_model** out) {
     P3D_ALLOC(m->lat_act, sizeof(uint2) * 1024 * 8 * 128);
     P3D_ALLOC(m->mid_act, sizeof(unsigned long long) * 8 * 64 * 512);
   }
+  if (cfg->mode == P3D_MODE_BF16X3 && L % 8 == 0) {    // the split weight pair of the bf16x3 GEMMs (zeroed: padding)
+    m->x3_seg = (L + 63) / 64 * 64;
+    P3D_ALLOC(m->wt_x3, sizeof(__nv_bfloat16) * static_cast<size_t>(m->rows_total) * 2 * m->x3_seg);
+  }
 #undef P3D_ALLOC
   // TF default BN state: gamma 1, beta 0, moving_mean 0, moving_variance 1
   for (auto& ly : m->layers) {
@@ -327,6 +332,7 @@ void p3d_model_destroy(p3d_model* m) {
   cudaFree(m->wt_bf16); cudaFree(m->bias_fold); cudaFree(m->wfold); cudaFree(m->norm2); cudaFree(m->pipe_loss);
   cudaFree(m->act_scratch); cudaFree(m->xb); cudaFree(m->f32_a); cudaFree(m->lat_counter); cudaFree(m->lay_act); cudaFree(m->lat_act); cudaFree(m->mid_act);
   cudaFree(m->xchg);
+  cudaFree(m->wt_x3); cudaFree(m->x3_in); cudaFree(m->x3_act); cudaFree(m->x3_res);
   for (void* p : m->retired) cudaFree(p);
   if (m->ev_done) cudaEventDestroy(m->ev_done);
   for (auto& e : m->pipe_ev) if (e) cudaEventDestroy(e);
@@ -440,6 +446,11 @@ static int forward_on(p3d_model* m, const float* x, float* y, int64_t B, cudaStr
     P3D_TRY(prep::prepare(m, st));
   }
   if (m->cfg.mode == P3D_MODE_FP32) return simt::forward_fp32(m, x, y, B, st);
+  if (m->cfg.mode == P3D_MODE_BF16X3) {
+    // widths no tensor-core tiling covers: the FFMA chain, which keeps the same precision contract
+    if ((m->L % 8) != 0) return simt::forward_fp32(m, x, y, B, st);
+    return layered::forward_split(m, x, y, B, st);
+  }
   const int L = m->L;
   if (B == 1 && L == 1024) {                            // single pose: whole-chip kernel (or the 16-CTA cluster kernel), one launch
     const int rc = simt::forward_latency_cluster(m, x, y, st);

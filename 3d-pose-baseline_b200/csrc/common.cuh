@@ -260,6 +260,13 @@ struct GemmArgs {
   void* dbg = nullptr;                // diagnostics: [ctas][8] globaltimer stamps
   int fused_mode = 0;                 // 0, or 3 / 4: fused training epilogue (unsplit K; every tile resident at once)
   FusedTrain fused;
+  // Segment schedule (bf16x3 inference; 0 = off): A and B are K-major split pairs, each row the hi segment (columns
+  // 0 .. K) then the lo segment from column seg_a / seg_b (a multiple of 64, >= K rounded up to 64; the columns
+  // between K and the lo segment must be zero).  The K loop makes three passes: A.hi B.hi + A.lo B.hi + A.hi B.lo.
+  int seg_a = 0, seg_b = 0;
+  // split-pair result (with the segment schedule): r = relu?(acc + bias) (+ res, fp32) -> C when C is set (may equal
+  // res: in place), and bf16(r) | bf16(r - bf16(r)) -> out_bf16 columns n | out_lo + n
+  int out_lo = 0;
 };
 // A planned GEMM: tensor maps + kernel parameters, built once (host cost of two cuTensorMapEncodeTiled calls)
 // and launched many times while the operand pointers/shapes stay the same.
@@ -353,6 +360,16 @@ struct p3d_model {
   unsigned* xchg = nullptr;
   float* f32_a = nullptr;                // fp32-path activations [2][cap][L]
   int64_t f32_cap = 0;
+  // bf16x3 mode (mlp_layered.cu forward_split): split pairs, every row [hi segment | lo segment], segment x3_seg =
+  // L rounded up to 64 columns, padding zero
+  int x3_seg = 0;
+  __nv_bfloat16* wt_x3 = nullptr;        // folded W'^T split [rows_total][2 x3_seg], allocated at model creation
+  __nv_bfloat16* x3_in = nullptr;        // input split [x3_cap][128]: hi columns 0..31, lo 64..95
+  __nv_bfloat16* x3_act = nullptr;       // hidden activations split, [2][x3_cap][2 x3_seg]
+  float* x3_res = nullptr;               // fp32 block input of the residual stream [x3_cap][L] (residual models)
+  int64_t x3_cap = 0;
+  struct X3Plans { int64_t rows = -1; const void* y = nullptr; std::vector<p3d::tcg::GemmPlan> pl; };
+  X3Plans x3_plans[2];                   // full row chunks, the last (partial) chunk
   // growable scratch that a captured graph may still address (retire()): freed by p3d_model_destroy
   bool captured = false;                 // a call of this model has run on a capturing stream
   std::vector<void*> retired;

@@ -5,7 +5,10 @@
 //   tf.layers.batch_normalization(training=False)   :112,181,193 (moving statistics, eps 1e-3)
 // into  W' = W * clip_scale * s,  b' = (b - moving_mean) * s + beta,  s = gamma / sqrt(moving_var + eps)
 // and writes them (a) fp32 [K,N] for the FFMA path and (b) bf16 transposed [N,Kpad] (K contiguous) for
-// the tcgen05 path, all layers stacked along rows.
+// the tcgen05 path, all layers stacked along rows; bf16x3 models also get (c) the split pair of (b), bf16(W') and
+// bf16(W' - bf16(W')), side by side in each row.
+#include <cstring>
+
 #include "common.cuh"
 
 namespace p3d {
@@ -40,8 +43,9 @@ struct FoldArgs {
   const double* norm2; // ||W||_F^2 (device) or null when max_norm is off
   float* wfold;        // [K,N]
   __nv_bfloat16* wt;   // [N rows starting at row_off][kpad]
+  __nv_bfloat16* wt3;  // bf16x3 models: [N rows starting at row_off][2 seg3], hi = bf16(W'), lo = bf16(W' - hi); else null
   float* bias_fold;    // [N] starting at row_off
-  int K, N, kpad;
+  int K, N, kpad, seg3;
 };
 
 __global__ void fold_pack_kernel(const FoldArgs a) {
@@ -68,7 +72,16 @@ __global__ void fold_pack_kernel(const FoldArgs a) {
   // write [n][k] coalesced along k
   for (int nn = threadIdx.y; nn < 32; nn += blockDim.y) {
     const int n = n0 + nn, k = k0 + threadIdx.x;
-    if (n < a.N && k < a.K) a.wt[static_cast<size_t>(n) * a.kpad + k] = __float2bfloat16_rn(tile[threadIdx.x][nn]);
+    if (n < a.N && k < a.K) {
+      const float v = tile[threadIdx.x][nn];
+      const __nv_bfloat16 hi = __float2bfloat16_rn(v);
+      a.wt[static_cast<size_t>(n) * a.kpad + k] = hi;
+      if (a.wt3) {
+        __nv_bfloat16* row = a.wt3 + static_cast<size_t>(n) * 2 * a.seg3;
+        row[k] = hi;
+        row[a.seg3 + k] = __float2bfloat16_rn(v - __bfloat162float(hi));
+      }
+    }
   }
   if (blockIdx.y == 0 && threadIdx.y == 0) {
     const int n = n0 + threadIdx.x;
@@ -101,6 +114,29 @@ __global__ void pack_input_kernel(const float* __restrict__ x, __nv_bfloat16* __
   reinterpret_cast<uint4*>(xb)[idx] = o;
 }
 
+// bf16x3: x fp32 [B,32] -> split pair [B,128]: hi = bf16(x) in columns 0..31, lo = bf16(x - hi) in 64..95, zeros
+// elsewhere (each half is one K=64 segment of the layer-0 GEMM)
+__global__ void pack_input_split_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ xs, long long B) {
+  const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;   // one 8-element group
+  if (idx >= B * 16) return;
+  const long long row = idx >> 4;
+  const int g = static_cast<int>(idx & 15);
+  uint4 o = make_uint4(0, 0, 0, 0);
+  if ((g & 7) < 4) {
+    const float4* xp = reinterpret_cast<const float4*>(x + row * kIn + (g & 7) * 8);
+    const float4 a = __ldg(xp), b = __ldg(xp + 1);
+    float v[8] = {a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w};
+    __nv_bfloat16 h[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      h[j] = __float2bfloat16_rn(v[j]);
+      if (g >= 8) h[j] = __float2bfloat16_rn(v[j] - __bfloat162float(h[j]));
+    }
+    memcpy(&o, h, 16);
+  }
+  reinterpret_cast<uint4*>(xs)[idx] = o;
+}
+
 int prepare(p3d_model* m, cudaStream_t st) {
   const int nl = static_cast<int>(m->layers.size());
   P3D_CUDA(cudaMemsetAsync(m->wt_bf16, 0, sizeof(__nv_bfloat16) * static_cast<size_t>(m->rows_total) * m->kpad, st));
@@ -128,8 +164,10 @@ int prepare(p3d_model* m, cudaStream_t st) {
     a.norm2 = m->cfg.max_norm ? m->norm2 + l : nullptr;
     a.wfold = m->wfold + ly.off_wfold;
     a.wt = m->wt_bf16 + static_cast<size_t>(ly.row_off) * m->kpad;
+    // the split pair is rewritten in place like wt_bf16; its padding columns were zeroed at model creation
+    a.wt3 = m->wt_x3 ? m->wt_x3 + static_cast<size_t>(ly.row_off) * 2 * m->x3_seg : nullptr;
     a.bias_fold = m->bias_fold + ly.row_off;
-    a.K = ly.K; a.N = ly.N; a.kpad = m->kpad;
+    a.K = ly.K; a.N = ly.N; a.kpad = m->kpad; a.seg3 = m->x3_seg;
     dim3 grid((ly.N + 31) / 32, (ly.K + 31) / 32), block(32, 8);
     fold_pack_kernel<<<grid, block, 0, st>>>(a);
     P3D_LAUNCH_CHECK();
@@ -141,6 +179,13 @@ int prepare(p3d_model* m, cudaStream_t st) {
 int pack_input(const float* x, __nv_bfloat16* xb, int64_t B, cudaStream_t st) {
   const long long groups = B * 8;
   pack_input_kernel<<<static_cast<unsigned>((groups + 255) / 256), 256, 0, st>>>(x, xb, B);
+  P3D_LAUNCH_CHECK();
+  return P3D_OK;
+}
+
+int pack_input_split(const float* x, __nv_bfloat16* xs, int64_t B, cudaStream_t st) {
+  const long long groups = B * 16;
+  pack_input_split_kernel<<<static_cast<unsigned>((groups + 255) / 256), 256, 0, st>>>(x, xs, B);
   P3D_LAUNCH_CHECK();
   return P3D_OK;
 }

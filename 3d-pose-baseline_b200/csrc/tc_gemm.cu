@@ -81,6 +81,8 @@ struct Params {
   unsigned long long* dbg;  // optional [ctas][32] globaltimer stamps (diagnostics)
   FusedTrain ft;            // OUT = 3 / 4 only
   long long wait_limit_ns;  // > 0: a wait for peers / the grid longer than this traps (diagnostics; 0 = wait like NCCL does)
+  int seg_a, seg_b;         // SEG: column of the lo segment of A / B (see GemmArgs::seg_a)
+  int ob_lo;                // OUT = 5: column of the lo halves in out_b
 };
 __device__ __forceinline__ unsigned long long gtime() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
 #define P3D_STAMP(i) do { if (p.dbg && lane == 0) p.dbg[(static_cast<size_t>(blockIdx.z * gridDim.y + blockIdx.y) * gridDim.x + blockIdx.x) * 32 + (i)] = gtime(); } while (0)
@@ -286,10 +288,13 @@ __device__ __forceinline__ void totals_wait(const Params& p, int n0, int et, dou
 }
 
 // OUT: 0 = fp32 store, 1 = fp32 reduction (split-K / accumulate), 2 = bf16 (relu, residual in bf16), 3 / 4 = fused
-// training epilogues (forward / backward).  RES: a residual operand is added.  CS: column sums of the result and its
-// square are accumulated (BatchNorm statistics of a forward layer on the unfused path).
-template <int OUT, bool RES, int CS>
-__global__ void __launch_bounds__((OUT >= 3) ? FUSED_NTHREADS : NTHREADS, 1)
+// training epilogues (forward / backward), 5 = split pair (relu, fp32 residual; the fp32 value to C when given, its
+// bf16 hi / lo halves to out_b).  RES: a residual operand is added.  CS: column sums of the result and its
+// square are accumulated (BatchNorm statistics of a forward layer on the unfused path).  SEG: segment schedule of the
+// split-precision (bf16x3) forward - the K loop runs three passes, reading the (A, B) segments (hi, hi), (lo, hi),
+// (hi, lo) into one accumulator.
+template <int OUT, bool RES, int CS, bool SEG = false>
+__global__ void __launch_bounds__((OUT == 3 || OUT == 4) ? FUSED_NTHREADS : NTHREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
   static_assert(CS == 0 || OUT < 2, "column sums are taken of the fp32 stores only");
   extern __shared__ uint8_t smem_raw[];
@@ -315,7 +320,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
   const int n0 = blockIdx.x * p.bn, m0 = blockIdx.y * BM;
   const int kbeg = blockIdx.z * p.k_per_split;
   const int kend = (kbeg + p.k_per_split < p.K) ? kbeg + p.k_per_split : p.K;
-  const int nk = (kend - kbeg + BK - 1) / BK;
+  const int nkp = (kend - kbeg + BK - 1) / BK;   // k-blocks of one pass
+  const int nk = SEG ? 3 * nkp : nkp;
 
   if (threadIdx.x == 0) {
     tma_prefetch_desc(&tm_a); tma_prefetch_desc(&tm_b);
@@ -354,13 +360,23 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
     auto load = [&](int stg, int k0) {
       tma_load_2d_s(dst0 + static_cast<uint32_t>(stg) * slot, my_map, full_s + static_cast<uint32_t>(stg) * 8u, my_mn ? fix : k0, my_mn ? k0 : fix);
     };
+    // K coordinate of k-block kb for this lane's operand.  SEG: pass 1 reads A's lo segment, pass 2 B's.
+    auto kcoord = [&](int kb) {
+      if constexpr (!SEG) {
+        return kbeg + kb * BK;
+      } else {
+        const int pass = kb / nkp;
+        const int lo = is_a ? (pass == 1 ? p.seg_a : 0) : (pass == 2 ? p.seg_b : 0);
+        return (kb - pass * nkp) * BK + lo;
+      }
+    };
     // Programmatic dependent launch: when B is marked independent of the preceding kernels (weights), its tiles for
     // the first ring pass are requested BEFORE griddepcontrol.wait, i.e. while the previous layer is still running.
     const int npre = p.b_independent ? (nk < STAGES ? nk : STAGES) : 0;
     for (int kb = 0; kb < npre; ++kb) {            // ring slots are free on the first pass
       if (lane == 0) mbar_arrive_expect_tx(&full[kb], bytes);
       __syncwarp();
-      if (is_b) load(kb, kbeg + kb * BK);
+      if (is_b) load(kb, kcoord(kb));
     }
     __syncwarp();
     grid_dependency_wait();
@@ -369,7 +385,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
       mbar_wait(&empty[stage], phase ^ 1, 1);
       if (kb >= npre && lane == 0) mbar_arrive_expect_tx(&full[stage], bytes);
       __syncwarp();
-      if (is_a || (is_b && kb >= npre)) load(stage, kbeg + kb * BK);
+      if (is_a || (is_b && kb >= npre)) load(stage, kcoord(kb));
       if (p.dbg) { if (kb == 3) P3D_STAMP(8); if (kb == 7) P3D_STAMP(9); if (kb == 11) P3D_STAMP(10); }
       if (++stage == STAGES) { stage = 0; phase ^= 1; }
     }
@@ -798,6 +814,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
     bool fast = (n0 + p.bn <= p.N);
     if (OUT == 2) fast = fast && ((p.ldob & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.out_b) & 7) == 0) &&
                          (!RES || (((p.ldrb & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.res_b) & 7) == 0)));
+    else if (OUT == 5) fast = fast && ((p.ldob & 3) == 0) && ((p.ob_lo & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.out_b) & 7) == 0) &&
+                              (!p.C || (((p.ldc & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0))) &&
+                              (!RES || (((p.ldres & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.res) & 15) == 0)));
     else fast = fast && ((p.ldc & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.C) & 15) == 0) &&
                         (!RES || (((p.ldres & 3) == 0) && ((reinterpret_cast<uintptr_t>(p.res) & 15) == 0)));
     mbar_wait(accf, 0, 3);
@@ -831,6 +850,8 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
             r4[i] = make_float4(0.f, 0.f, 0.f, 0.f); rb[i] = make_uint2(0u, 0u);
             if (m < p.M) {
               if (OUT == 2) rb[i] = *reinterpret_cast<const uint2*>(p.res_b + static_cast<size_t>(m) * p.ldrb + n);
+              // in place (res == C): a plain load, not the read-only path, for memory this kernel writes
+              else if (OUT == 5) r4[i] = *reinterpret_cast<const float4*>(p.res + static_cast<size_t>(m) * p.ldres + n);
               else r4[i] = __ldg(reinterpret_cast<const float4*>(p.res + static_cast<size_t>(m) * p.ldres + n));
             }
           }
@@ -854,6 +875,25 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
             }
             uint2 q; memcpy(&q, ob, 8);
             if (live) *reinterpret_cast<uint2*>(p.out_b + static_cast<size_t>(m) * p.ldob + n) = q;
+          } else if (OUT == 5) {
+            // split pair: r = relu(.) (+ fp32 residual) stays fp32; hi = bf16(r), lo = bf16(r - hi) (r - hi is exact)
+            __nv_bfloat16 hb[4], lb[4];
+            float r[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) r[j] = p.relu ? fmaxf(o[j], 0.f) : o[j];
+            if (use_res) { r[0] += r4[i].x; r[1] += r4[i].y; r[2] += r4[i].z; r[3] += r4[i].w; }
+#pragma unroll
+            for (int j = 0; j < 4; ++j) {
+              hb[j] = __float2bfloat16_rn(r[j]);
+              lb[j] = __float2bfloat16_rn(r[j] - __bfloat162float(hb[j]));
+            }
+            if (live) {
+              if (p.C) *reinterpret_cast<float4*>(p.C + static_cast<size_t>(m) * p.ldc + n) = make_float4(r[0], r[1], r[2], r[3]);
+              uint2 qh, ql; memcpy(&qh, hb, 8); memcpy(&ql, lb, 8);
+              __nv_bfloat16* ob = p.out_b + static_cast<size_t>(m) * p.ldob + n;
+              *reinterpret_cast<uint2*>(ob) = qh;
+              *reinterpret_cast<uint2*>(ob + p.ob_lo) = ql;
+            }
           } else {
             if (use_res) { o[0] += r4[i].x; o[1] += r4[i].y; o[2] += r4[i].z; o[3] += r4[i].w; }
             if (CS == 1) {            // sums of the stored values: residual included
@@ -886,6 +926,13 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
               __nv_bfloat16 ob = __float2bfloat16_rn(p.relu ? fmaxf(o, 0.f) : o);
               if (use_res) ob = __float2bfloat16_rn(__bfloat162float(ob) + __bfloat162float(p.res_b[static_cast<size_t>(m) * p.ldrb + n + j]));
               p.out_b[static_cast<size_t>(m) * p.ldob + n + j] = ob;
+            } else if (OUT == 5) {
+              float r = p.relu ? fmaxf(o, 0.f) : o;
+              if (use_res) r += p.res[static_cast<size_t>(m) * p.ldres + n + j];
+              if (p.C) p.C[static_cast<size_t>(m) * p.ldc + n + j] = r;
+              const __nv_bfloat16 hb = __float2bfloat16_rn(r);
+              p.out_b[static_cast<size_t>(m) * p.ldob + n + j] = hb;
+              p.out_b[static_cast<size_t>(m) * p.ldob + p.ob_lo + n + j] = __float2bfloat16_rn(r - __bfloat162float(hb));
             } else {
               if (use_res) o += __ldg(p.res + static_cast<size_t>(m) * p.ldres + n + j);
               if (CS == 1) { cs1[j] += o; cs2[j] += o * o; }
@@ -1053,9 +1100,20 @@ int plan(const GemmArgs& g, GemmPlan* out) {
   // K-major A of a short problem: fetch only the rows that exist (the MMA still reads 128 smem rows; what it makes
   // of the stale ones lands in accumulator rows >= M, which are never stored)
   const int a_rows = (!g.a_mn && g.M < BM) ? ((g.M + 7) / 8 * 8) : BM;
-  if (!g.a_mn) P3D_TRY(make_map(&d->ta, g.A, g.K, g.M, g.lda, a_rows));
+  const bool seg = g.seg_a != 0 || g.seg_b != 0;
+  if (seg) {
+    P3D_REQUIRE(!g.a_mn && !g.b_mn && !g.split_k && !g.accumulate && !g.colsum && !g.fused_mode && !g.res_bf16,
+                "tc_gemm: the segment schedule takes K-major operands, an unsplit K and the plain or split-pair epilogues");
+    P3D_REQUIRE(g.seg_a % BK == 0 && g.seg_b % BK == 0 && g.seg_a >= kblocks * BK && g.seg_b >= kblocks * BK,
+                "tc_gemm: lo segments must start at a multiple of %d columns past the hi segment (K %d, seg %d / %d)",
+                BK, g.K, g.seg_a, g.seg_b);
+    P3D_REQUIRE(!g.out_bf16 || g.out_lo > 0, "tc_gemm: the segment schedule writes fp32 or split-pair output");
+  }
+  P3D_REQUIRE(!g.out_lo || (seg && g.out_bf16), "tc_gemm: split-pair output needs the segment schedule and out_bf16");
+  // SEG: a map covers both segments; reads past the lo segment's K are zero-filled, the hi segment's tail is padding
+  if (!g.a_mn) P3D_TRY(make_map(&d->ta, g.A, g.seg_a + g.K, g.M, g.lda, a_rows));
   else P3D_TRY(make_map(&d->ta, g.A, g.M, g.K, g.lda, BK));
-  if (!g.b_mn) P3D_TRY(make_map(&d->tb, g.B, g.K, g.N, g.ldb, bn));
+  if (!g.b_mn) P3D_TRY(make_map(&d->tb, g.B, g.seg_b + g.K, g.N, g.ldb, bn));
   else P3D_TRY(make_map(&d->tb, g.B, g.N, g.K, g.ldb, BK));
   Params& p = d->p;
   p.M = g.M; p.N = g.N; p.K = g.K; p.bn = bn; p.k_per_split = kps; p.a_mn = g.a_mn; p.b_mn = g.b_mn;
@@ -1080,6 +1138,7 @@ int plan(const GemmArgs& g, GemmPlan* out) {
   // the fused epilogues wait for their peers like an NCCL collective does (ranks must stay in lockstep)
   static const long long wait_ns = [] { const char* e = getenv("P3D_SYNC_TIMEOUT_S"); return e ? static_cast<long long>(atof(e) * 1e9) : 0LL; }();
   p.wait_limit_ns = wait_ns;
+  p.seg_a = g.seg_a; p.seg_b = g.seg_b; p.ob_lo = g.out_lo;
   d->pdl = g.pdl;
   p.ft = g.fused;
   d->fused_mode = g.fused_mode;
@@ -1111,15 +1170,19 @@ int launch(const GemmPlan& pl, cudaStream_t st) {
   const PlanData* d = reinterpret_cast<const PlanData*>(pl.blob);
   using KernelFn = void (*)(const CUtensorMap, const CUtensorMap, const Params);
   const Params& q = d->p;
-  const int out = q.out_b ? 2 : (q.atomic ? 1 : 0);
-  const bool res = q.out_b ? (q.res_b != nullptr) : (q.res != nullptr);
+  const int out = q.ob_lo ? 5 : (q.out_b ? 2 : (q.atomic ? 1 : 0));
+  const bool res = (out == 2) ? (q.res_b != nullptr) : (q.res != nullptr);
   const int cs = q.colsum ? 1 : 0;
+  const bool seg = q.seg_a != 0;
   KernelFn fn = nullptr;
-#define P3D_TCG_PICK(O, R, S) if (out == O && res == R && cs == S) fn = tc_gemm_kernel<O, R, S>;
+#define P3D_TCG_PICK(O, R, S) if (!seg && out == O && res == R && cs == S) fn = tc_gemm_kernel<O, R, S>;
   P3D_TCG_PICK(0, false, 0) P3D_TCG_PICK(0, false, 1) P3D_TCG_PICK(0, true, 0) P3D_TCG_PICK(0, true, 1)
   P3D_TCG_PICK(1, false, 0) P3D_TCG_PICK(1, true, 0)
   P3D_TCG_PICK(2, false, 0) P3D_TCG_PICK(2, true, 0)
 #undef P3D_TCG_PICK
+#define P3D_TCG_PICK_SEG(O, R) if (seg && out == O && res == R && cs == 0) fn = tc_gemm_kernel<O, R, 0, true>;
+  P3D_TCG_PICK_SEG(0, false) P3D_TCG_PICK_SEG(5, false) P3D_TCG_PICK_SEG(5, true)
+#undef P3D_TCG_PICK_SEG
   if (d->fused_mode == 3) fn = tc_gemm_kernel<3, false, 0>;
   if (d->fused_mode == 4) fn = tc_gemm_kernel<4, false, 0>;
   P3D_REQUIRE(fn != nullptr, "tc_gemm: unsupported epilogue combination (out %d res %d colsum %d)", out, (int)res, (int)cs);
@@ -1128,7 +1191,8 @@ int launch(const GemmPlan& pl, cudaStream_t st) {
     KernelFn all[] = {tc_gemm_kernel<0, false, 0>, tc_gemm_kernel<0, false, 1>, tc_gemm_kernel<0, true, 0>,
                       tc_gemm_kernel<0, true, 1>, tc_gemm_kernel<1, false, 0>, tc_gemm_kernel<1, true, 0>,
                       tc_gemm_kernel<2, false, 0>, tc_gemm_kernel<2, true, 0>,
-                      tc_gemm_kernel<3, false, 0>, tc_gemm_kernel<4, false, 0>};
+                      tc_gemm_kernel<3, false, 0>, tc_gemm_kernel<4, false, 0>,
+                      tc_gemm_kernel<0, false, 0, true>, tc_gemm_kernel<5, false, 0, true>, tc_gemm_kernel<5, true, 0, true>};
     for (KernelFn f : all) P3D_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     attr.mark();
   }

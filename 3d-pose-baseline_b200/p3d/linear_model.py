@@ -5,7 +5,8 @@ are replaced by libp3d.so (hand-written sm_100a CUDA).  There is no TensorFlow, 
 
 Differences that are visible to a caller, all additive:
   * `session` is accepted and ignored (there is no tf.Session).
-  * keyword-only extras: `mode` ('bf16' tensor-core path, or 'fp32'), `device`, `seed`, `dist`.
+  * keyword-only extras: `mode` ('bf16' tensor-core path, 'fp32', or 'bf16x3': fp32 accuracy on the tensor cores
+    for inference, trained like 'fp32'), `device`, `seed`, `dist`.
   * `step()` also accepts torch CUDA tensors (fp32) and then returns torch tensors without any host copy.
   * summaries are `Summary(tag, value)` tuples that serialize to the TF `Summary` protobuf on demand; with a
     `summaries_dir` the train/test writers append real TensorBoard event files (p3d/summary.py), without one they
@@ -144,8 +145,9 @@ class LinearModel(object):
         self._lr0 = float(learning_rate)
         self._seed = int(seed) if seed is not None else int.from_bytes(os.urandom(4), "little")
         self._handle = None
-        if mode not in ("bf16", "fp32"):
-            raise ValueError("mode must be 'bf16' or 'fp32'")
+        modes = {"bf16": _lib.MODE_BF16, "fp32": _lib.MODE_FP32, "bf16x3": _lib.MODE_BF16X3}
+        if mode not in modes:
+            raise ValueError("mode must be 'bf16', 'fp32' or 'bf16x3'")
         # Summary writers for train and test runs (linear_model.py:80-82)
         if summaries_dir:
             self.train_writer = FileWriter(os.path.join(summaries_dir, "train"))
@@ -155,7 +157,7 @@ class LinearModel(object):
 
         cfg = _lib.Cfg(self.linear_size, self.num_layers, int(self.residual), int(self.batch_norm),
                        int(self.max_norm), int(self.predict_14),
-                       _lib.MODE_BF16 if mode == "bf16" else _lib.MODE_FP32, self.device, self._lr0)
+                       modes[mode], self.device, self._lr0)
         h = C.c_void_p()
         check(lib.p3d_model_create(C.byref(cfg), C.byref(h)))
         self._handle = h

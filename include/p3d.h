@@ -52,6 +52,11 @@ extern "C" {
 
 #define P3D_MODE_BF16 0 /* tcgen05 bf16 x bf16 -> fp32 accumulate (headline path) */
 #define P3D_MODE_FP32 1 /* fp32 FFMA path, <=1e-4 relative to the fp64 oracle */
+/* fp32-class (<=1e-4 relative to the fp64 oracle): inference on tcgen05 as three split-bf16 products per MatMul
+ * (hi*hi + lo*hi + hi*lo, fp32 accumulation, fp32 activations); linear_size % 8 != 0 runs the FFMA path.  Training
+ * steps and epochs are those of P3D_MODE_FP32; the whole-chip bf16 kernels and the one-launch realtime frame are not
+ * used (frames take the staged route). */
+#define P3D_MODE_BF16X3 2
 
 const char* p3d_last_error(void);
 int p3d_version(void);
