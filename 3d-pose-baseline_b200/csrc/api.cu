@@ -635,6 +635,15 @@ int p3d_debug_tc_gemm(const void* A, int lda, int a_mn, const void* B, int ldb, 
   return tcg::gemm(g, static_cast<cudaStream_t>(stream));
 }
 
+int p3d_debug_tc_gemm_seg(const void* A, int lda, int a_mn, int seg_a, const void* B, int ldb, int b_mn, int seg_b, float* C, int ldc,
+                          int M, int N, int K, const float* res, float alpha, int split_k, void* stream) {
+  P3D_REQUIRE(seg_a > 0 && seg_b > 0, "debug_tc_gemm_seg: both operands are split pairs (seg_a, seg_b > 0)");
+  tcg::GemmArgs g;
+  g.M = M; g.N = N; g.K = K; g.A = A; g.lda = lda; g.a_mn = a_mn; g.seg_a = seg_a; g.B = B; g.ldb = ldb; g.b_mn = b_mn; g.seg_b = seg_b;
+  g.C = C; g.ldc = ldc; g.res = res; g.ldres = ldc; g.alpha = alpha; g.split_k = split_k;
+  return tcg::gemm(g, static_cast<cudaStream_t>(stream));
+}
+
 int p3d_debug_mma_rate(int N, int iters, int64_t* out_dev, void* stream) {
   P3D_REQUIRE(out_dev, "debug_mma_rate: null argument");
   return tcg::mma_rate(N, iters, reinterpret_cast<long long*>(out_dev), static_cast<cudaStream_t>(stream));

@@ -109,6 +109,15 @@ struct TrainWorkspace {
   __nv_bfloat16* dzb = nullptr;   // [B][L]
   __nv_bfloat16* dyb = nullptr;   // [B][48] (pad columns zero)
   __nv_bfloat16* wb = nullptr;    // weights [K][N] per layer at theta's offsets; W4 rows padded to 48
+  // split-pair operands of the bf16x3 training route (P3D_TRAIN_MATMUL_BF16X3): every row [hi segment | lo segment],
+  // segment = width rounded up to 64 columns (x, dy, W4: 64), padding zero.  Allocated zeroed.
+  int64_t x3_B = 0;                // rows xs / hs / dzs / dys hold
+  __nv_bfloat16* xs = nullptr;     // [B][128]
+  __nv_bfloat16* hs = nullptr;     // [nhidden][B][2 seg]
+  __nv_bfloat16* dzs = nullptr;    // [B][2 seg]
+  __nv_bfloat16* dys = nullptr;    // [B][128]
+  __nv_bfloat16* ws = nullptr;     // weights [K][2 seg_N] per layer at ws_off (unclipped; the clip scale is the GEMM's alpha)
+  std::vector<size_t> ws_off;      // per layer, elements into ws
   void* tab = nullptr;            // device LayerTabEntry[nlayers]
   void* sc = nullptr;             // device StepScalars (per-step values: Adam step size, lr, dropout seed/step)
   // CUDA-graph replay of the step: fixed-address staging of x / t / y / (loss, lr) and one graph per (B, dropout)
@@ -260,9 +269,10 @@ struct GemmArgs {
   void* dbg = nullptr;                // diagnostics: [ctas][8] globaltimer stamps
   int fused_mode = 0;                 // 0, or 3 / 4: fused training epilogue (unsplit K; every tile resident at once)
   FusedTrain fused;
-  // Segment schedule (bf16x3 inference; 0 = off): A and B are K-major split pairs, each row the hi segment (columns
-  // 0 .. K) then the lo segment from column seg_a / seg_b (a multiple of 64, >= K rounded up to 64; the columns
-  // between K and the lo segment must be zero).  The K loop makes three passes: A.hi B.hi + A.lo B.hi + A.hi B.lo.
+  // Segment schedule (bf16x3; 0 = off): A and B are split pairs, each row the hi segment then the lo segment from
+  // column seg_a / seg_b (a multiple of 64) of the operand's contiguous dimension.  K-major: seg >= K rounded up to 64,
+  // the columns between K and the lo segment must be zero.  MN-major: seg >= M (A) or N (B).  The K loop makes three
+  // passes: A.hi B.hi + A.lo B.hi + A.hi B.lo; split K and the fp32 reduction epilogue are allowed.
   int seg_a = 0, seg_b = 0;
   // split-pair result (with the segment schedule): r = relu?(acc + bias) (+ res, fp32) -> C when C is set (may equal
   // res: in place), and bf16(r) | bf16(r - bf16(r)) -> out_bf16 columns n | out_lo + n
@@ -388,6 +398,7 @@ struct p3d_model {
   cudaEvent_t ev_done = nullptr;
   bool ev_done_recorded = false;
   // training
+  int train_matmul = P3D_TRAIN_MATMUL_DEFAULT;   // p3d_model_set_train_matmul
   p3d::TrainWorkspace tw;
   void* nccl_comm = nullptr;
   int rank = 0, world = 1;

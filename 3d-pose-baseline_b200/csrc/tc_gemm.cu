@@ -291,8 +291,8 @@ __device__ __forceinline__ void totals_wait(const Params& p, int n0, int et, dou
 // training epilogues (forward / backward), 5 = split pair (relu, fp32 residual; the fp32 value to C when given, its
 // bf16 hi / lo halves to out_b).  RES: a residual operand is added.  CS: column sums of the result and its
 // square are accumulated (BatchNorm statistics of a forward layer on the unfused path).  SEG: segment schedule of the
-// split-precision (bf16x3) forward - the K loop runs three passes, reading the (A, B) segments (hi, hi), (lo, hi),
-// (hi, lo) into one accumulator.
+// split-precision (bf16x3) GEMMs, inference and training - the K loop runs three passes, reading the (A, B) segments
+// (hi, hi), (lo, hi), (hi, lo) into one accumulator; either operand K-major or MN-major, K split or not.
 template <int OUT, bool RES, int CS, bool SEG = false>
 __global__ void __launch_bounds__((OUT == 3 || OUT == 4) ? FUSED_NTHREADS : NTHREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
@@ -360,15 +360,21 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
     auto load = [&](int stg, int k0) {
       tma_load_2d_s(dst0 + static_cast<uint32_t>(stg) * slot, my_map, full_s + static_cast<uint32_t>(stg) * 8u, my_mn ? fix : k0, my_mn ? k0 : fix);
     };
-    // K coordinate of k-block kb for this lane's operand.  SEG: pass 1 reads A's lo segment, pass 2 B's.
-    auto kcoord = [&](int kb) {
-      if constexpr (!SEG) {
-        return kbeg + kb * BK;
-      } else {
-        const int pass = kb / nkp;
-        const int lo = is_a ? (pass == 1 ? p.seg_a : 0) : (pass == 2 ? p.seg_b : 0);
-        return (kb - pass * nkp) * BK + lo;
-      }
+    // K coordinate of k-block kb for this lane's operand.
+    auto kcoord = [&](int kb) { return kbeg + kb * BK; };
+    // SEG: pass 1 reads A's lo segment, pass 2 B's.  The lo segment lies `seg` columns along the operand's CONTIGUOUS
+    // dimension: the K coordinate of a K-major operand, the MN coordinate (fix) of an MN-major one.  Each pass walks
+    // this split's own K range [kbeg, kend).
+    auto load_seg = [&](int stg, int kb) {
+      const int pass = kb / nkp;
+      const int lo = is_a ? (pass == 1 ? p.seg_a : 0) : (pass == 2 ? p.seg_b : 0);
+      const int k0 = kbeg + (kb - pass * nkp) * BK;
+      tma_load_2d_s(dst0 + static_cast<uint32_t>(stg) * slot, my_map, full_s + static_cast<uint32_t>(stg) * 8u,
+                    my_mn ? fix + lo : k0 + lo, my_mn ? k0 : fix);
+    };
+    auto fetch = [&](int stg, int kb) {
+      if constexpr (SEG) load_seg(stg, kb);
+      else load(stg, kcoord(kb));
     };
     // Programmatic dependent launch: when B is marked independent of the preceding kernels (weights), its tiles for
     // the first ring pass are requested BEFORE griddepcontrol.wait, i.e. while the previous layer is still running.
@@ -376,7 +382,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
     for (int kb = 0; kb < npre; ++kb) {            // ring slots are free on the first pass
       if (lane == 0) mbar_arrive_expect_tx(&full[kb], bytes);
       __syncwarp();
-      if (is_b) load(kb, kcoord(kb));
+      if (is_b) fetch(kb, kb);
     }
     __syncwarp();
     grid_dependency_wait();
@@ -385,7 +391,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
       mbar_wait(&empty[stage], phase ^ 1, 1);
       if (kb >= npre && lane == 0) mbar_arrive_expect_tx(&full[stage], bytes);
       __syncwarp();
-      if (is_a || (is_b && kb >= npre)) load(stage, kcoord(kb));
+      if (is_a || (is_b && kb >= npre)) fetch(stage, kb);
       if (p.dbg) { if (kb == 3) P3D_STAMP(8); if (kb == 7) P3D_STAMP(9); if (kb == 11) P3D_STAMP(10); }
       if (++stage == STAGES) { stage = 0; phase ^= 1; }
     }
@@ -1102,19 +1108,26 @@ int plan(const GemmArgs& g, GemmPlan* out) {
   const int a_rows = (!g.a_mn && g.M < BM) ? ((g.M + 7) / 8 * 8) : BM;
   const bool seg = g.seg_a != 0 || g.seg_b != 0;
   if (seg) {
-    P3D_REQUIRE(!g.a_mn && !g.b_mn && !g.split_k && !g.accumulate && !g.colsum && !g.fused_mode && !g.res_bf16,
-                "tc_gemm: the segment schedule takes K-major operands, an unsplit K and the plain or split-pair epilogues");
-    P3D_REQUIRE(g.seg_a % BK == 0 && g.seg_b % BK == 0 && g.seg_a >= kblocks * BK && g.seg_b >= kblocks * BK,
-                "tc_gemm: lo segments must start at a multiple of %d columns past the hi segment (K %d, seg %d / %d)",
-                BK, g.K, g.seg_a, g.seg_b);
+    P3D_REQUIRE(g.seg_a > 0 && g.seg_b > 0 && !g.accumulate && !g.colsum && !g.fused_mode && !g.res_bf16,
+                "tc_gemm: the segment schedule takes split pairs on both sides and the plain, reduction or split-pair epilogues");
+    // the lo segment starts past the hi segment's contiguous extent: K (rounded up to a k-block) for a K-major
+    // operand, M or N for an MN-major one
+    const int need_a = g.a_mn ? g.M : kblocks * BK, need_b = g.b_mn ? g.N : kblocks * BK;
+    P3D_REQUIRE(g.seg_a % BK == 0 && g.seg_b % BK == 0 && g.seg_a >= need_a && g.seg_b >= need_b,
+                "tc_gemm: lo segments must start at a multiple of %d columns past the hi segment (M %d, N %d, K %d, seg %d / %d)",
+                BK, g.M, g.N, g.K, g.seg_a, g.seg_b);
     P3D_REQUIRE(!g.out_bf16 || g.out_lo > 0, "tc_gemm: the segment schedule writes fp32 or split-pair output");
   }
   P3D_REQUIRE(!g.out_lo || (seg && g.out_bf16), "tc_gemm: split-pair output needs the segment schedule and out_bf16");
-  // SEG: a map covers both segments; reads past the lo segment's K are zero-filled, the hi segment's tail is padding
+  // SEG: a map covers both segments of the contiguous dimension; its outer extent is the operand's own, so the K tail
+  // of an MN-major operand (batch rows of a weight gradient) is zero-filled by TMA.
+  //   K-major: reads past the lo segment's K are zero-filled, the hi segment's K tail is zero padding (must be).
+  //   MN-major: a 64-column box past M (N) reads padding, the other segment or zero fill into accumulator rows
+  //             (columns) >= M (N), which are never stored - harmless.
   if (!g.a_mn) P3D_TRY(make_map(&d->ta, g.A, g.seg_a + g.K, g.M, g.lda, a_rows));
-  else P3D_TRY(make_map(&d->ta, g.A, g.M, g.K, g.lda, BK));
+  else P3D_TRY(make_map(&d->ta, g.A, g.seg_a + g.M, g.K, g.lda, BK));
   if (!g.b_mn) P3D_TRY(make_map(&d->tb, g.B, g.seg_b + g.K, g.N, g.ldb, bn));
-  else P3D_TRY(make_map(&d->tb, g.B, g.N, g.K, g.ldb, BK));
+  else P3D_TRY(make_map(&d->tb, g.B, g.seg_b + g.N, g.K, g.ldb, BK));
   Params& p = d->p;
   p.M = g.M; p.N = g.N; p.K = g.K; p.bn = bn; p.k_per_split = kps; p.a_mn = g.a_mn; p.b_mn = g.b_mn;
   p.C = g.C; p.ldc = g.ldc; p.bias = g.bias; p.res = g.res; p.ldres = g.ldres; p.alpha_dev = g.alpha_dev; p.alpha = g.alpha;
@@ -1182,6 +1195,7 @@ int launch(const GemmPlan& pl, cudaStream_t st) {
 #undef P3D_TCG_PICK
 #define P3D_TCG_PICK_SEG(O, R) if (seg && out == O && res == R && cs == 0) fn = tc_gemm_kernel<O, R, 0, true>;
   P3D_TCG_PICK_SEG(0, false) P3D_TCG_PICK_SEG(5, false) P3D_TCG_PICK_SEG(5, true)
+  P3D_TCG_PICK_SEG(0, true) P3D_TCG_PICK_SEG(1, false)       // bf16x3 training: data gradient + residual, split-K weight gradient
 #undef P3D_TCG_PICK_SEG
   if (d->fused_mode == 3) fn = tc_gemm_kernel<3, false, 0>;
   if (d->fused_mode == 4) fn = tc_gemm_kernel<4, false, 0>;
@@ -1192,7 +1206,8 @@ int launch(const GemmPlan& pl, cudaStream_t st) {
                       tc_gemm_kernel<0, true, 1>, tc_gemm_kernel<1, false, 0>, tc_gemm_kernel<1, true, 0>,
                       tc_gemm_kernel<2, false, 0>, tc_gemm_kernel<2, true, 0>,
                       tc_gemm_kernel<3, false, 0>, tc_gemm_kernel<4, false, 0>,
-                      tc_gemm_kernel<0, false, 0, true>, tc_gemm_kernel<5, false, 0, true>, tc_gemm_kernel<5, true, 0, true>};
+                      tc_gemm_kernel<0, false, 0, true>, tc_gemm_kernel<5, false, 0, true>, tc_gemm_kernel<5, true, 0, true>,
+                      tc_gemm_kernel<0, true, 0, true>, tc_gemm_kernel<1, false, 0, true>};
     for (KernelFn f : all) P3D_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     attr.mark();
   }

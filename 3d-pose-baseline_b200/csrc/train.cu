@@ -7,6 +7,8 @@
 // tcgen05 tensor cores (tc_gemm.cu) with bf16 operands, fp32 accumulation and fp32 master weights; H, dZ and W
 // are consumed in their natural row-major layouts (MN-major UMMA descriptors where the reduction dimension is
 // the row index), the forward GEMM's epilogue also produces the BatchNorm column sums.  P3D_MODE_FP32: FFMA GEMMs.
+// P3D_TRAIN_MATMUL_BF16X3 (fp32 / bf16x3 models, opt-in): the FFMA route's kernels, with every GEMM replaced by three
+// split-bf16 tcgen05 products (tc_gemm.cu segment schedule) on split-pair copies of x, h, dz, dy and W.
 // Data parallel (one process per GPU): rows are sharded, BN statistics and their backward sums are
 // all-reduced (SyncBN - required for parity with the single-device reference), and the flat gradient
 // buffer is all-reduced once with NCCL before the (replicated) Adam update.
@@ -20,6 +22,7 @@
 #include "train_common.cuh"
 
 namespace p3d {
+namespace prep { int pack_input_split(const float*, __nv_bfloat16*, int64_t, cudaStream_t); }
 
 namespace train {
 
@@ -80,11 +83,23 @@ constexpr int RCH4 = 64;   // rows per block of the float4 column-reduction kern
 __global__ void set_scalars_kernel(StepScalars* dst, const StepScalars v) { *dst = v; }
 
 // per-layer table for the kernels that sweep all weight matrices in one launch (gridDim.y = layer)
-struct LayerTabEntry { long long off_w, off_wb; int K, N, ldwb, pad; };
+struct LayerTabEntry { long long off_w, off_wb, off_ws; int K, N, ldwb, seg; };
 
-// W -> bf16 operand copy (row pitch ldwb >= N) and ||W||_F^2, every layer in ONE launch
+// bf16x3 split pair of 4 consecutive values: hi = bf16(v) at p[0..3], lo = bf16(v - hi) at p[lo..lo+3] (v - hi is exact)
+__device__ __forceinline__ void store_split4(__nv_bfloat16* p, int lo, const float (&v)[4]) {
+  __nv_bfloat16 h[4], l[4];
+#pragma unroll
+  for (int j = 0; j < 4; ++j) { h[j] = __float2bfloat16_rn(v[j]); l[j] = __float2bfloat16_rn(v[j] - __bfloat162float(h[j])); }
+  uint2 qh, ql;
+  memcpy(&qh, h, 8); memcpy(&ql, l, 8);
+  *reinterpret_cast<uint2*>(p) = qh;
+  *reinterpret_cast<uint2*>(p + lo) = ql;
+}
+
+// W -> bf16 operand copy (row pitch ldwb >= N) and ||W||_F^2, every layer in ONE launch; ws: the split pair of W instead
+// (bf16x3 training route, rows [hi | lo] of pitch 2 seg at off_ws).  The norm is summed in the same order either way.
 __global__ void wprep_kernel(const float* __restrict__ theta, const LayerTabEntry* __restrict__ tab, __nv_bfloat16* __restrict__ wb,
-                             double* __restrict__ norm2) {
+                             double* __restrict__ norm2, __nv_bfloat16* __restrict__ ws) {
   const LayerTabEntry e = tab[blockIdx.y];
   const long long n = static_cast<long long>(e.K) * e.N;
   const float* w = theta + e.off_w;
@@ -99,12 +114,23 @@ __global__ void wprep_kernel(const float* __restrict__ theta, const LayerTabEntr
         uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
         *reinterpret_cast<uint2*>(wb + e.off_wb + i) = pk;
       }
+      if (ws) {      // N % 4 == 0 here (hidden widths, and the output layer only when N == its 48-column pitch)
+        const long long r = i / e.N;
+        const float vv[4] = {v.x, v.y, v.z, v.w};
+        store_split4(ws + e.off_ws + r * 2 * e.seg + (i - r * e.N), e.seg, vv);
+      }
     }
   } else {
     for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n; i += static_cast<long long>(gridDim.x) * blockDim.x) {
       const float v = w[i];
       acc += static_cast<double>(v) * v;
       if (wb) { const long long r = i / e.N; wb[e.off_wb + r * e.ldwb + (i - r * e.N)] = __float2bfloat16_rn(v); }
+      if (ws) {
+        const long long r = i / e.N;
+        __nv_bfloat16* row = ws + e.off_ws + r * 2 * e.seg + (i - r * e.N);
+        const __nv_bfloat16 h = __float2bfloat16_rn(v);
+        row[0] = h; row[e.seg] = __float2bfloat16_rn(v - __bfloat162float(h));
+      }
     }
   }
   if (norm2) {
@@ -188,6 +214,7 @@ struct ActArgs {
   const float* z; const float* mean; const float* rstd; const float* gamma; const float* beta;
   const float* res; float* h; __nv_bfloat16* hb; uint8_t* mask; const uint8_t* mask_in;
   const StepScalars* sc; unsigned layer; long long row0, B; int L; int has_bn; int dropout;
+  __nv_bfloat16* hs; int seg;     // bf16x3 training route: split pair of h, rows [hi | lo] of pitch 2 seg (else null)
 };
 
 // h = dropout(relu(bn(z))) (+res); one thread per 4 columns; also materialises the keep-mask
@@ -232,6 +259,7 @@ __global__ void fwd_act_kernel(const ActArgs a) {
       uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
       *reinterpret_cast<uint2*>(a.hb + r * a.L + c) = pk;
     }
+    if (a.hs) store_split4(a.hs + r * 2 * a.seg + c, a.seg, v);     // operand of the next layer's bf16x3 GEMMs
   }
 }
 
@@ -247,13 +275,21 @@ __global__ void to_bf16_kernel(const float* __restrict__ src, __nv_bfloat16* __r
 }
 
 // dy = 2 (y - t) / (Bg*out), loss accumulator += sum (y-t)^2
+// dyb: bf16 operand copy of dy with row pitch ld_b; lo_b > 0: the split pair instead, lo half at column lo_b + c
 __global__ void loss_dy_kernel(const float* __restrict__ y, const float* __restrict__ t, size_t n, float scale,
-                               float* __restrict__ dy, double* __restrict__ acc, __nv_bfloat16* __restrict__ dyb, int out, int ld_b) {
+                               float* __restrict__ dy, double* __restrict__ acc, __nv_bfloat16* __restrict__ dyb, int out, int ld_b,
+                               int lo_b) {
   double s = 0;
   for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < n; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
     const float d = y[i] - t[i];
     dy[i] = scale * d;
-    if (dyb) { const size_t r = i / out; dyb[r * ld_b + (i - r * out)] = __float2bfloat16_rn(scale * d); }
+    if (dyb) {
+      const size_t r = i / out;
+      const float v = scale * d;
+      const __nv_bfloat16 h = __float2bfloat16_rn(v);
+      dyb[r * ld_b + (i - r * out)] = h;
+      if (lo_b) dyb[r * ld_b + lo_b + (i - r * out)] = __float2bfloat16_rn(v - __bfloat162float(h));
+    }
     s += static_cast<double>(d) * d;
   }
   for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(0xffffffffu, s, o);
@@ -274,6 +310,7 @@ __global__ void finish_step_scalars_kernel(const double* acc, double denom, cons
 struct BwdArgs {
   const float* dh; const float* z; const float* mean; const float* rstd; const float* gamma; const float* beta;
   const uint8_t* mask; float* dz; __nv_bfloat16* dzb; double* sums; const StepScalars* sc; long long B; int L; int has_bn; int dropout;
+  __nv_bfloat16* dzs; int seg;    // bf16x3 training route, layers without BN: split pair of dz (else null)
 };
 
 // pass A: da = dh * dropout * relu'(a); column sums of da and da*xhat (for BN backward / dgamma, dbeta).
@@ -318,6 +355,7 @@ __global__ void __launch_bounds__(256) bwd_act_kernel(const BwdArgs a) {
         uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
         *reinterpret_cast<uint2*>(a.dzb + o) = pk;
       }
+      if (a.dzs) store_split4(a.dzs + static_cast<size_t>(r) * 2 * a.seg + c, a.seg, da);
     }
   }
 #pragma unroll
@@ -341,7 +379,8 @@ __global__ void bwd_bn_kernel(float* __restrict__ dz, const float* __restrict__ 
                               const double* __restrict__ sums, float invB, long long B, int L, __nv_bfloat16* __restrict__ dzb,
                               int write_f32, double pg_scale, float* __restrict__ ggamma, float* __restrict__ gbeta,
                               const float* __restrict__ dh, const uint8_t* __restrict__ mask, const float* __restrict__ beta,
-                              const StepScalars* __restrict__ sc) {
+                              const StepScalars* __restrict__ sc, __nv_bfloat16* __restrict__ dzs, int seg) {
+  // dzs: the split pair of dz (bf16x3 training route), rows [hi | lo] of pitch 2 seg
   // dh != null: da is recomputed from (dh, z, mask) instead of being read back - pass A then never stores it
   const int L4 = L / 4;
   const long long total = B * L4;
@@ -386,6 +425,7 @@ __global__ void bwd_bn_kernel(float* __restrict__ dz, const float* __restrict__ 
       uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
       *reinterpret_cast<uint2*>(dzb + o) = pk;
     }
+    if (dzs) store_split4(dzs + static_cast<size_t>(r) * 2 * seg + c, seg, v);
     if (r == 0) {
 #pragma unroll
       for (int j = 0; j < 4; ++j) { gbeta[c + j] = static_cast<float>(sums[c + j] * pg_scale); ggamma[c + j] = static_cast<float>(sums[L + c + j] * pg_scale); }
@@ -469,6 +509,7 @@ void free_workspace(p3d_model* m) {
   cudaFree(w.z); cudaFree(w.h); cudaFree(w.dh); cudaFree(w.dz); cudaFree(w.dres); cudaFree(w.dy);
   cudaFree(w.stats); cudaFree(w.mean); cudaFree(w.rstd); cudaFree(w.scal); cudaFree(w.maskbuf);
   cudaFree(w.xb); cudaFree(w.hb); cudaFree(w.dzb); cudaFree(w.dyb); cudaFree(w.wb);
+  cudaFree(w.xs); cudaFree(w.hs); cudaFree(w.dzs); cudaFree(w.dys); cudaFree(w.ws);
   cudaFree(w.tab); cudaFree(w.sc); cudaFree(w.gx); cudaFree(w.gt); cudaFree(w.gy); cudaFree(w.gscal);
   for (auto& ge : w.graphs) if (ge.exec) cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(ge.exec));
   if (w.cap_stream) cudaStreamDestroy(w.cap_stream);
@@ -482,13 +523,51 @@ void free_workspace(p3d_model* m) {
 constexpr int kOutPad = 48;   // bf16 pitch of dy / W4 rows: 96 B keeps TMA's 16-byte pitch rule for out = 42 too
 // bf16 mode runs the step's GEMMs on the tensor cores (tc_gemm.cu); fp32 mode keeps the FFMA GEMMs
 static inline bool use_tc(const p3d_model* m) { return m->cfg.mode == P3D_MODE_BF16 && (m->L % 8) == 0; }
+// P3D_TRAIN_MATMUL_BF16X3 (fp32 / bf16x3 models): the step's GEMMs as three split-bf16 products on the tensor cores;
+// widths the tcgen05 GEMM does not tile keep FFMA
+static inline bool use_x3(const p3d_model* m) {
+  return m->train_matmul == P3D_TRAIN_MATMUL_BF16X3 && m->cfg.mode != P3D_MODE_BF16 && (m->L % 8) == 0;
+}
+static inline int seg_of(int n) { return (n + 63) / 64 * 64; }   // lo-segment column of a split pair of width n
+
+static void drop_graphs(TrainWorkspace& w) {
+  for (auto& ge : w.graphs) if (ge.exec) cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(ge.exec));   // they hold the old pointers
+  w.graphs.clear();
+}
+
+// the split-pair buffers of the bf16x3 route for cap_B rows, zeroed once (their padding columns are never written)
+static int ensure_split_buffers(p3d_model* m) {
+  TrainWorkspace& w = m->tw;
+  const int nh = static_cast<int>(m->layers.size()) - 1, ld = 2 * seg_of(m->L);
+  if (w.x3_B >= w.cap_B) return P3D_OK;
+  drop_graphs(w);
+  cudaFree(w.xs); cudaFree(w.hs); cudaFree(w.dzs); cudaFree(w.dys);
+  w.xs = w.hs = w.dzs = w.dys = nullptr; w.x3_B = 0;
+  const size_t B = static_cast<size_t>(w.cap_B);
+  const size_t nx = B * 128, nhs = B * ld * nh, ndz = B * ld, ndy = B * 128;
+  P3D_CUDA(cudaMalloc(&w.xs, sizeof(__nv_bfloat16) * nx));
+  P3D_CUDA(cudaMalloc(&w.hs, sizeof(__nv_bfloat16) * nhs));
+  P3D_CUDA(cudaMalloc(&w.dzs, sizeof(__nv_bfloat16) * ndz));
+  P3D_CUDA(cudaMalloc(&w.dys, sizeof(__nv_bfloat16) * ndy));
+  P3D_CUDA(cudaMemset(w.hs, 0, sizeof(__nv_bfloat16) * nhs));
+  P3D_CUDA(cudaMemset(w.dzs, 0, sizeof(__nv_bfloat16) * ndz));
+  P3D_CUDA(cudaMemset(w.dys, 0, sizeof(__nv_bfloat16) * ndy));      // (pack_input_split writes every column of xs)
+  if (!w.ws) {
+    const size_t n = w.ws_off.back() + static_cast<size_t>(m->layers.back().K) * 2 * seg_of(m->out_size);
+    P3D_CUDA(cudaMalloc(&w.ws, sizeof(__nv_bfloat16) * n));
+    P3D_CUDA(cudaMemset(w.ws, 0, sizeof(__nv_bfloat16) * n));
+  }
+  w.x3_B = w.cap_B;
+  return P3D_OK;
+}
 
 static int ensure_workspace(p3d_model* m, int64_t B) {
   TrainWorkspace& w = m->tw;
   const int L = m->L, nh = static_cast<int>(m->layers.size()) - 1, nl = nh + 1;
-  if (w.cap_B >= B) return P3D_OK;
-  for (auto& ge : w.graphs) if (ge.exec) cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(ge.exec));   // they hold the old pointers
-  w.graphs.clear();
+  if (w.cap_B >= B) return use_x3(m) ? ensure_split_buffers(m) : P3D_OK;
+  drop_graphs(w);
+  cudaFree(w.xs); cudaFree(w.hs); cudaFree(w.dzs); cudaFree(w.dys);
+  w.xs = w.hs = w.dzs = w.dys = nullptr; w.x3_B = 0;
   cudaFree(w.gx); cudaFree(w.gt); cudaFree(w.gy);
   w.gx = w.gt = w.gy = nullptr;
   cudaFree(w.z); cudaFree(w.h); cudaFree(w.dh); cudaFree(w.dz); cudaFree(w.dres); cudaFree(w.dy); cudaFree(w.maskbuf);
@@ -535,16 +614,21 @@ static int ensure_workspace(p3d_model* m, int64_t B) {
     for (auto& e : w.ev) P3D_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
     P3D_CUDA(cudaMalloc(&w.sc, sizeof(StepScalars)));
     std::vector<LayerTabEntry> tab(nl);
+    w.ws_off.assign(nl, 0);
+    size_t off_ws = 0;
     for (int l = 0; l < nl; ++l) {
       const Layer& ly = m->layers[l];
       tab[l].off_w = static_cast<long long>(ly.off_w); tab[l].off_wb = static_cast<long long>(ly.off_w);
-      tab[l].K = ly.K; tab[l].N = ly.N; tab[l].ldwb = (l == nl - 1) ? kOutPad : ly.N; tab[l].pad = 0;
+      tab[l].K = ly.K; tab[l].N = ly.N; tab[l].ldwb = (l == nl - 1) ? kOutPad : ly.N;
+      tab[l].seg = seg_of(ly.N); tab[l].off_ws = static_cast<long long>(off_ws);
+      w.ws_off[l] = off_ws;
+      off_ws += static_cast<size_t>(ly.K) * 2 * tab[l].seg;
     }
     P3D_CUDA(cudaMalloc(&w.tab, sizeof(LayerTabEntry) * nl));
     P3D_CUDA(cudaMemcpy(w.tab, tab.data(), sizeof(LayerTabEntry) * nl, cudaMemcpyHostToDevice));
   }
   w.cap_B = B;
-  return P3D_OK;
+  return use_x3(m) ? ensure_split_buffers(m) : P3D_OK;
 }
 
 // P3D_TRAIN_FUSED=0 forces the unfused path (GEMM + statistics + finalize + activation kernels) at every batch size; read
@@ -613,7 +697,7 @@ static int fwd_bwd_fused(p3d_model* m, const float* t, int64_t B, bool dropout, 
     P3D_TRY(tcg::gemm(g, st));
   }
   const size_t ny = static_cast<size_t>(B) * out;
-  loss_dy_kernel<<<egrid(static_cast<long long>(ny)), 256, 0, st>>>(y, t, ny, 2.0f * invB / out, w.dy, lossacc, w.dyb, out, kOutPad);
+  loss_dy_kernel<<<egrid(static_cast<long long>(ny)), 256, 0, st>>>(y, t, ny, 2.0f * invB / out, w.dy, lossacc, w.dyb, out, kOutPad, 0);
   P3D_LAUNCH_CHECK();
   // ---------------------------------------------------------------- backward
   // (data parallel: the loss sum rides on the first backward exchange, see fused_dgrad)
@@ -717,6 +801,10 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
   const bool clip = m->cfg.max_norm != 0;
   const bool residual = m->cfg.residual != 0;
   const bool tc = use_tc(m);
+  const bool x3 = use_x3(m);        // bf16x3 split products on tcgen05 (unfused route, FFMA's elementwise kernels)
+  const bool lowp = tc || x3;       // the GEMMs read the bf16 operand buffers, not the fp32 activations
+  const int seg = seg_of(L), ld = 2 * seg;
+  const size_t bls = static_cast<size_t>(B) * ld;   // one layer of split activations
   using tcg::GemmArgs;
   double* dots = w.red + 2ull * nh * L;
   double* lossacc = dots + nlay;
@@ -728,10 +816,10 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
   P3D_CUDA(cudaMemsetAsync(w.stats, 0, sizeof(double) * (4ull * nh * L + nlay + 1 + 2ull * nh), st));
   P3D_CUDA(cudaMemsetAsync(m->grad, 0, sizeof(float) * m->n_train, st));
   if (clip) P3D_CUDA(cudaMemsetAsync(m->norm2, 0, sizeof(double) * nlay, st));
-  if (clip || tc) {
-    // one launch over all layers: ||W||_F^2 (clip_by_norm) and, on the tensor-core path, this step's bf16 copy of
-    // W in its natural [K][N] layout (W4 rows padded to kOutPad)
-    wprep_kernel<<<dim3(148, nlay), 256, 0, st>>>(m->theta, tab, tc ? w.wb : nullptr, clip ? m->norm2 : nullptr);
+  if (clip || lowp) {
+    // one launch over all layers: ||W||_F^2 (clip_by_norm) and, on the tensor-core paths, this step's bf16 copy (or
+    // split pair) of the UNCLIPPED W in its natural [K][N] layout (W4 rows padded); the clip scale is the GEMMs' alpha
+    wprep_kernel<<<dim3(148, nlay), 256, 0, st>>>(m->theta, tab, tc ? w.wb : nullptr, clip ? m->norm2 : nullptr, x3 ? w.ws : nullptr);
     P3D_LAUNCH_CHECK();
   }
   if (clip) {
@@ -742,6 +830,7 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
     to_bf16_kernel<<<egrid(static_cast<long long>(B) * kIn / 4 + 1), 256, 0, st>>>(x, w.xb, B, kIn, kIn);
     P3D_LAUNCH_CHECK();
   }
+  if (x3) P3D_TRY(prep::pack_input_split(x, w.xs, B, st));      // [B][128]: hi columns 0..31, lo 64..95
   // fused epilogues: every tile of a hidden layer must be resident at once; data parallel they need the peer-memory
   // exchange (otherwise the unfused path reduces through NCCL).  Every rank decides alike: B is the same everywhere up
   // to one row and the host layer attaches peer memory on all ranks or on none.
@@ -764,6 +853,13 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       g.B = w.wb + ly.off_w; g.ldb = L; g.b_mn = 1;
       g.C = z; g.ldc = L; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + li : nullptr;
       g.colsum = ly.has_bn ? stats : nullptr;
+      P3D_TRY(tcg::gemm(g, st));
+    } else if (x3) {
+      GemmArgs g;   // z = (x|h) W * clip + b: A K-major, W MN-major, both split pairs
+      g.M = static_cast<int>(B); g.N = L; g.K = ly.K;
+      g.A = li == 0 ? w.xs : w.hs + (li - 1) * bls; g.lda = li == 0 ? 128 : ld; g.seg_a = li == 0 ? 64 : seg;
+      g.B = w.ws + w.ws_off[li]; g.ldb = ld; g.b_mn = 1; g.seg_b = seg;
+      g.C = z; g.ldc = L; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + li : nullptr;
       P3D_TRY(tcg::gemm(g, st));
     } else {
       Epilogue e; e.bias = m->theta + ly.off_b; e.alpha_dev = clip ? scale + li : nullptr;
@@ -791,9 +887,10 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
     a.z = z; a.mean = mean; a.rstd = rstd;
     a.gamma = ly.has_bn ? m->theta + ly.off_gamma : nullptr; a.beta = ly.has_bn ? m->theta + ly.off_beta : nullptr;
     a.res = (residual && li >= 2 && (li % 2) == 0) ? w.h + (li - 2) * bl : nullptr;
-    // on the tensor-core path the fp32 copy of h is only read back as a residual (by layer li + 2)
-    const bool h_needed = !tc || (residual && (li % 2) == 0 && li + 2 < nh);
+    // on the tensor-core paths the fp32 copy of h is only read back as a residual (by layer li + 2)
+    const bool h_needed = !lowp || (residual && (li % 2) == 0 && li + 2 < nh);
     a.h = h_needed ? w.h + li * bl : nullptr; a.hb = tc ? w.hb + li * bl : nullptr; a.mask = maskbuf + li * bl; a.mask_in = mask_in ? mask_in + li * bl : nullptr;
+    a.hs = x3 ? w.hs + li * bls : nullptr; a.seg = seg;
     a.sc = sc; a.layer = li;
     a.row0 = row0; a.B = B; a.L = L; a.has_bn = ly.has_bn; a.dropout = dropout;
     fwd_act_kernel<<<egrid(static_cast<long long>(bl / 4)), 256, 0, st>>>(a);
@@ -808,6 +905,13 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       g.B = w.wb + ly.off_w; g.ldb = kOutPad; g.b_mn = 1;
       g.C = y; g.ldc = out; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + nh : nullptr;
       P3D_TRY(tcg::gemm(g, st));
+    } else if (x3) {
+      GemmArgs g;   // y = h W4 * clip + b4 (W4 split pair: [L][128], segment 64)
+      g.M = static_cast<int>(B); g.N = out; g.K = L;
+      g.A = w.hs + (nh - 1) * bls; g.lda = ld; g.seg_a = seg;
+      g.B = w.ws + w.ws_off[nh]; g.ldb = 128; g.b_mn = 1; g.seg_b = 64;
+      g.C = y; g.ldc = out; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + nh : nullptr;
+      P3D_TRY(tcg::gemm(g, st));
     } else {
       Epilogue e; e.bias = m->theta + ly.off_b; e.alpha_dev = clip ? scale + nh : nullptr;
       P3D_TRY(sgemm(false, false, B, out, L, w.h + (nh - 1) * bl, L, m->theta + ly.off_w, out, y, out, e, st));
@@ -815,7 +919,8 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
   }
   const size_t ny = static_cast<size_t>(B) * out;
   loss_dy_kernel<<<egrid(static_cast<long long>(ny)), 256, 0, st>>>(y, t, ny, static_cast<float>(2.0 * invBg / out), w.dy, lossacc,
-                                                                          tc ? w.dyb : nullptr, out, kOutPad);
+                                                                          tc ? w.dyb : (x3 ? w.dys : nullptr), out, tc ? kOutPad : 128,
+                                                                          x3 ? 64 : 0);
   P3D_LAUNCH_CHECK();
   P3D_TRY(allreduce(m, lossacc, 1, ncclDouble, st));
   // ---------------------------------------------------------------- backward
@@ -828,6 +933,13 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       gw.M = L; gw.N = out; gw.K = static_cast<int>(B);
       gw.A = w.hb + (nh - 1) * bl; gw.lda = L; gw.a_mn = 1;
       gw.B = w.dyb; gw.ldb = kOutPad; gw.b_mn = 1;
+      gw.C = m->grad + ly.off_w; gw.ldc = out; gw.split_k = 1;
+      P3D_TRY(tcg::gemm(gw, st));
+    } else if (x3) {
+      GemmArgs gw;   // dW4 = h^T dy: both split pairs MN-major, K = batch rows, split-K
+      gw.M = L; gw.N = out; gw.K = static_cast<int>(B);
+      gw.A = w.hs + (nh - 1) * bls; gw.lda = ld; gw.a_mn = 1; gw.seg_a = seg;
+      gw.B = w.dys; gw.ldb = 128; gw.b_mn = 1; gw.seg_b = 64;
       gw.C = m->grad + ly.off_w; gw.ldc = out; gw.split_k = 1;
       P3D_TRY(tcg::gemm(gw, st));
     } else {
@@ -843,6 +955,13 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       gd.B = w.wb + ly.off_w; gd.ldb = kOutPad;
       gd.C = G[cur]; gd.ldc = L; gd.alpha_dev = clip ? scale + nh : nullptr;
       P3D_TRY(tcg::gemm(gd, st));
+    } else if (x3) {
+      GemmArgs gd;   // dh = dy W4^T * clip: both K-major (W4 rows are the output rows), K = out
+      gd.M = static_cast<int>(B); gd.N = L; gd.K = out;
+      gd.A = w.dys; gd.lda = 128; gd.seg_a = 64;
+      gd.B = w.ws + w.ws_off[nh]; gd.ldb = 128; gd.seg_b = 64;
+      gd.C = G[cur]; gd.ldc = L; gd.alpha_dev = clip ? scale + nh : nullptr;
+      P3D_TRY(tcg::gemm(gd, st));
     } else {
       Epilogue e1; e1.alpha_dev = clip ? scale + nh : nullptr;
       P3D_TRY(sgemm(false, true, B, L, out, w.dy, out, m->theta + ly.off_w, out, G[cur], L, e1, st));
@@ -854,8 +973,9 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
     BwdArgs a;
     a.dh = G[cur]; a.z = w.z + li * bl; a.mean = w.mean + static_cast<size_t>(li) * L; a.rstd = w.rstd + static_cast<size_t>(li) * L;
     a.gamma = ly.has_bn ? m->theta + ly.off_gamma : nullptr; a.beta = ly.has_bn ? m->theta + ly.off_beta : nullptr;
-    a.mask = maskbuf + li * bl; a.dz = (tc && ly.has_bn) ? nullptr : w.dz;   // tensor-core + BN: pass B recomputes da
+    a.mask = maskbuf + li * bl; a.dz = (lowp && ly.has_bn) ? nullptr : w.dz;   // tensor-core + BN: pass B recomputes da
     a.dzb = (tc && !ly.has_bn) ? w.dzb : nullptr; a.sums = w.red + 2ull * li * L; a.sc = sc;
+    a.dzs = (x3 && !ly.has_bn) ? w.dzs : nullptr; a.seg = seg;
     a.B = B; a.L = L; a.has_bn = ly.has_bn; a.dropout = dropout;
     bwd_act_kernel<<<dim3((L / 4 + 31) / 32, static_cast<unsigned>((B + RCH4 - 1) / RCH4)), dim3(32, 8), 0, st>>>(a);
     P3D_LAUNCH_CHECK();
@@ -865,9 +985,10 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       // so every rank holds the full dgamma/dbeta: pre-divide by world so that the flat gradient all-reduce (a sum)
       // restores them exactly once.
       bwd_bn_kernel<<<egrid(static_cast<long long>(bl / 4)), 256, 0, st>>>(w.dz, a.z, a.mean, a.rstd, a.gamma, a.sums, static_cast<float>(invBg), B, L,
-                                                                           tc ? w.dzb : nullptr, tc ? 0 : 1, 1.0 / m->world,
+                                                                           tc ? w.dzb : nullptr, lowp ? 0 : 1, 1.0 / m->world,
                                                                            m->grad + ly.off_gamma, m->grad + ly.off_beta,
-                                                                           tc ? a.dh : nullptr, dropout ? a.mask : nullptr, a.beta, sc);
+                                                                           lowp ? a.dh : nullptr, dropout ? a.mask : nullptr, a.beta, sc,
+                                                                           x3 ? w.dzs : nullptr, seg);
       P3D_LAUNCH_CHECK();
       // the bias feeding a BN layer has an exactly-zero gradient (it is removed by the mean subtraction)
     } else {
@@ -883,6 +1004,13 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       gw.B = w.dzb; gw.ldb = L; gw.b_mn = 1;
       gw.C = m->grad + ly.off_w; gw.ldc = L; gw.split_k = 1;
       P3D_TRY(tcg::gemm(gw, st));
+    } else if (x3) {
+      GemmArgs gw;   // dW = in^T dz: both split pairs MN-major, K = batch rows, split-K
+      gw.M = ly.K; gw.N = L; gw.K = static_cast<int>(B);
+      gw.A = li == 0 ? w.xs : w.hs + (li - 1) * bls; gw.lda = li == 0 ? 128 : ld; gw.a_mn = 1; gw.seg_a = li == 0 ? 64 : seg;
+      gw.B = w.dzs; gw.ldb = ld; gw.b_mn = 1; gw.seg_b = seg;
+      gw.C = m->grad + ly.off_w; gw.ldc = L; gw.split_k = 1;
+      P3D_TRY(tcg::gemm(gw, st));
     } else {
       Epilogue e0;
       P3D_TRY(sgemm(true, false, ly.K, L, static_cast<int>(B), in, lda, w.dz, L, m->grad + ly.off_w, L, e0, st));
@@ -896,6 +1024,14 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
         gd.M = static_cast<int>(B); gd.N = L; gd.K = L;
         gd.A = w.dzb; gd.lda = L;
         gd.B = w.wb + ly.off_w; gd.ldb = L;
+        gd.C = G[nxt]; gd.ldc = L; gd.alpha_dev = clip ? scale + li : nullptr;
+        if (add) { gd.res = G[keepi]; gd.ldres = L; }
+        P3D_TRY(tcg::gemm(gd, st));
+      } else if (x3) {
+        GemmArgs gd;   // dh_prev = dz W^T * clip (+ the gradient that bypassed the block): both K-major split pairs
+        gd.M = static_cast<int>(B); gd.N = L; gd.K = L;
+        gd.A = w.dzs; gd.lda = ld; gd.seg_a = seg;
+        gd.B = w.ws + w.ws_off[li]; gd.ldb = ld; gd.seg_b = seg;
         gd.C = G[nxt]; gd.ldc = L; gd.alpha_dev = clip ? scale + li : nullptr;
         if (add) { gd.res = G[keepi]; gd.ldres = L; }
         P3D_TRY(tcg::gemm(gd, st));
@@ -1092,6 +1228,17 @@ int p3d_model_train_epoch(p3d_model* m, const float* X, const float* T, int64_t 
   }
   return train::train_epoch(m, X, T, n, reinterpret_cast<const long long*>(perm_or_null), batch_size, keep_prob, seed, losses,
                             lr_last_or_null, static_cast<cudaStream_t>(stream));
+}
+
+int p3d_model_set_train_matmul(p3d_model* m, int kind) {
+  P3D_REQUIRE(m, "set_train_matmul: null model");
+  P3D_REQUIRE(kind == P3D_TRAIN_MATMUL_DEFAULT || kind == P3D_TRAIN_MATMUL_BF16X3, "set_train_matmul: unknown kind %d", kind);
+  P3D_REQUIRE(m->cfg.mode != P3D_MODE_BF16, "set_train_matmul: bf16-mode models train on their own tcgen05 bf16 route");
+  if (kind == m->train_matmul) return P3D_OK;
+  P3D_CUDA(cudaSetDevice(m->cfg.device));
+  train::drop_graphs(m->tw);        // captured with the other route's launches; the next step captures again
+  m->train_matmul = kind;
+  return P3D_OK;
 }
 
 int p3d_model_gathered_outputs(p3d_model* m, float* y_global, int64_t global_B, void* stream) {

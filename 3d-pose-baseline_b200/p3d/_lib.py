@@ -40,6 +40,7 @@ class Camera(C.Structure):
 
 
 MODE_BF16, MODE_FP32, MODE_BF16X3 = 0, 1, 2
+TRAIN_MATMUL_DEFAULT, TRAIN_MATMUL_BF16X3 = 0, 1
 
 # name -> (restype, argtypes): every symbol include/p3d.h declares
 PROTOTYPES = {
@@ -95,10 +96,13 @@ PROTOTYPES = {
     "p3d_model_p2p_detach": (c_int, [c_void_p]),
     "p3d_debug_dp_part": (c_int, [c_void_p, c_int, c_void_p]),
     "p3d_model_gathered_outputs": (c_int, [c_void_p, c_void_p, c_int64, c_void_p]),
+    "p3d_model_set_train_matmul": (c_int, [c_void_p, c_int]),
     "p3d_model_train_epoch": (c_int, [c_void_p, c_void_p, c_void_p, c_int64, c_void_p, c_int64, c_float, C.c_uint64,
                                       c_void_p, c_void_p, c_void_p]),
     "p3d_debug_tc_gemm": (c_int, [c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_void_p, c_int, c_int, c_int, c_int,
                                   c_void_p, c_void_p, c_float, c_int, c_void_p, c_void_p]),
+    "p3d_debug_tc_gemm_seg": (c_int, [c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int, c_int, c_void_p, c_int, c_int,
+                                      c_int, c_int, c_void_p, c_float, c_int, c_void_p]),
     "p3d_debug_mma_rate": (c_int, [c_int, c_int, c_void_p, c_void_p]),
     "p3d_debug_umma_gemm": (c_int, [c_void_p, c_void_p, c_void_p, c_int, c_int, c_void_p]),
 }

@@ -6,7 +6,8 @@ are replaced by libp3d.so (hand-written sm_100a CUDA).  There is no TensorFlow, 
 Differences that are visible to a caller, all additive:
   * `session` is accepted and ignored (there is no tf.Session).
   * keyword-only extras: `mode` ('bf16' tensor-core path, 'fp32', or 'bf16x3': fp32 accuracy on the tensor cores
-    for inference, trained like 'fp32'), `device`, `seed`, `dist`.
+    for inference, trained like 'fp32'), `train_matmul` (None: the mode's own training route; 'bf16x3' with mode
+    'fp32' or 'bf16x3': the training step's MatMuls as three split-bf16 tensor-core products), `device`, `seed`, `dist`.
   * `step()` also accepts torch CUDA tensors (fp32) and then returns torch tensors without any host copy.
   * summaries are `Summary(tag, value)` tuples that serialize to the TF `Summary` protobuf on demand; with a
     `summaries_dir` the train/test writers append real TensorBoard event files (p3d/summary.py), without one they
@@ -130,7 +131,7 @@ class LinearModel(object):
 
     def __init__(self, linear_size, num_layers, residual, batch_norm, max_norm, batch_size, learning_rate,
                  summaries_dir=None, predict_14=False, dtype=np.float32, *, mode="bf16", device=0, seed=None,
-                 dist=None):
+                 dist=None, train_matmul=None):
         self.HUMAN_2D_SIZE = 16 * 2                                  # linear_model.py:60
         self.HUMAN_3D_SIZE = 14 * 3 if predict_14 else 16 * 3         # :69
         self.input_size = self.HUMAN_2D_SIZE
@@ -148,6 +149,13 @@ class LinearModel(object):
         modes = {"bf16": _lib.MODE_BF16, "fp32": _lib.MODE_FP32, "bf16x3": _lib.MODE_BF16X3}
         if mode not in modes:
             raise ValueError("mode must be 'bf16', 'fp32' or 'bf16x3'")
+        # the arithmetic of the training step's MatMuls (p3d_model_set_train_matmul); with `dist`, every rank passes the
+        # same value
+        if train_matmul not in (None, "bf16x3"):
+            raise ValueError("train_matmul must be None or 'bf16x3'")
+        if train_matmul is not None and mode == "bf16":
+            raise ValueError("train_matmul='bf16x3' needs mode 'fp32' or 'bf16x3' (bf16 models train on bf16 tensor cores)")
+        self.train_matmul = train_matmul
         # Summary writers for train and test runs (linear_model.py:80-82)
         if summaries_dir:
             self.train_writer = FileWriter(os.path.join(summaries_dir, "train"))
@@ -161,6 +169,8 @@ class LinearModel(object):
         h = C.c_void_p()
         check(lib.p3d_model_create(C.byref(cfg), C.byref(h)))
         self._handle = h
+        if train_matmul == "bf16x3":
+            check(lib.p3d_model_set_train_matmul(self._handle, _lib.TRAIN_MATMUL_BF16X3))
         self.global_step = _Evaluable(lambda: int(lib.p3d_model_global_step(self._handle)))
         self.learning_rate = _Evaluable(self._decayed_lr)
         self._names = self._query_names()

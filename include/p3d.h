@@ -54,8 +54,9 @@ extern "C" {
 #define P3D_MODE_FP32 1 /* fp32 FFMA path, <=1e-4 relative to the fp64 oracle */
 /* fp32-class (<=1e-4 relative to the fp64 oracle): inference on tcgen05 as three split-bf16 products per MatMul
  * (hi*hi + lo*hi + hi*lo, fp32 accumulation, fp32 activations); linear_size % 8 != 0 runs the FFMA path.  Training
- * steps and epochs are those of P3D_MODE_FP32; the whole-chip bf16 kernels and the one-launch realtime frame are not
- * used (frames take the staged route). */
+ * steps and epochs are those of P3D_MODE_FP32 unless p3d_model_set_train_matmul(P3D_TRAIN_MATMUL_BF16X3) puts their
+ * MatMuls on the tensor cores too; the whole-chip bf16 kernels and the one-launch realtime frame are not used (frames
+ * take the staged route). */
 #define P3D_MODE_BF16X3 2
 
 const char* p3d_last_error(void);
@@ -135,6 +136,22 @@ int p3d_model_train_step(p3d_model* m, const float* x, const float* t, int64_t B
  * learning rate.  Single GPU (data-parallel models call p3d_model_train_step per batch). */
 int p3d_model_train_epoch(p3d_model* m, const float* X, const float* T, int64_t n, const int64_t* perm_or_null, int64_t batch_size,
                           float keep_prob, uint64_t seed, float* losses, float* lr_last_or_null, void* stream);
+
+/* Which arithmetic runs the MatMuls of a training step (steps and epochs), chosen per model:
+ *   P3D_TRAIN_MATMUL_DEFAULT: the mode's own route - tcgen05 bf16 (P3D_MODE_BF16), FFMA (P3D_MODE_FP32, P3D_MODE_BF16X3).
+ *   P3D_TRAIN_MATMUL_BF16X3 : every MatMul of the step (forward, data and weight gradients) on tcgen05 as three split-bf16
+ *                             products hi*hi + lo*hi + hi*lo with fp32 accumulation; activations, BatchNorm, dropout,
+ *                             the loss and Adam stay fp32 as on the FFMA route.  fp32-class, not bit-equal to FFMA: at
+ *                             batch 64 gradients are within 2e-5 of each tensor's max of the fp64 graph; at batch 4096
+ *                             the split operands move pre-activations by ~1e-5 relative, which flips the ReLU of a few
+ *                             dozen units near zero (gradients within ~3e-3 relative L2) - hence opt-in.  Widths with
+ *                             linear_size % 8 != 0 keep the FFMA route.
+ * Valid on P3D_MODE_FP32 and P3D_MODE_BF16X3 models; a P3D_MODE_BF16 model returns P3D_ERR_ARG.  A host call without a
+ * stream: it must not be made while a training step of the model is in flight.  Switching drops the model's captured
+ * training-step graphs (the next step captures again).  Data-parallel ranks must all set the same kind. */
+#define P3D_TRAIN_MATMUL_DEFAULT 0
+#define P3D_TRAIN_MATMUL_BF16X3 1
+int p3d_model_set_train_matmul(p3d_model* m, int kind);
 /* Data parallel: a NCCL communicator owned by the library (SyncBN statistics + one gradient
  * all-reduce per step).  id_host = 128-byte ncclUniqueId made by rank 0 and broadcast by the caller. */
 int p3d_nccl_unique_id(uint8_t* id_host /*[128]*/);
@@ -272,6 +289,12 @@ int p3d_debug_latency_stamps(p3d_model* m, uint64_t* out_host, int n);
  * zeroed); colsum (optional, [2][N] doubles, +=) receives the column sums of C and C^2. */
 int p3d_debug_tc_gemm(const void* A, int lda, int a_mn, const void* B, int ldb, int b_mn, float* C, int ldc, int M, int N, int K,
                       const float* bias, const float* res, float alpha, int split_k, double* colsum, void* stream);
+/* Diagnostics: the same GEMM under the segment schedule of the bf16x3 GEMMs.  A and B are split pairs: along the
+ * operand's contiguous dimension (K of a K-major operand, M / N of an MN-major one) every row holds the hi halves from
+ * column 0 and the lo halves from column seg_a / seg_b (multiples of 64); C = alpha * (A.hi B.hi + A.lo B.hi + A.hi B.lo)
+ * (+res[m][n]); split_k != 0 splits K over the grid with fp32 atomics (C must be zeroed). */
+int p3d_debug_tc_gemm_seg(const void* A, int lda, int a_mn, int seg_a, const void* B, int ldb, int b_mn, int seg_b, float* C, int ldc,
+                          int M, int N, int K, const float* res, float alpha, int split_k, void* stream);
 /* Diagnostics: cycles of `iters` back-to-back tcgen05.mma 128 x N x 16 on resident shared-memory operands (one CTA).
  * out_dev[0] = cycles to issue, out_dev[1] = cycles until the commit completes. */
 int p3d_debug_mma_rate(int N, int iters, int64_t* out_dev, void* stream);
