@@ -21,7 +21,7 @@ void set_error(const char* fmt, ...) {
 void count_launch(int n) { launch_counter()->fetch_add(n); }
 long long launch_count_now() { return launch_counter()->load(); }
 
-namespace prep { int prepare(p3d_model*, cudaStream_t); int pack_input(const float*, __nv_bfloat16*, int64_t, cudaStream_t); }
+namespace prep { int prepare(p3d_model*, cudaStream_t); int pack_input(const float*, __nv_bfloat16*, int64_t, bool, cudaStream_t); }
 namespace tc { int forward_bf16(p3d_model*, const __nv_bfloat16*, float*, int64_t, cudaStream_t);
                int debug_umma_gemm(const void*, const void*, float*, int, int, cudaStream_t); }
 namespace simt { int forward_fp32(p3d_model*, const float*, float*, int64_t, cudaStream_t);
@@ -202,7 +202,8 @@ int p3d_model_create(const p3d_cfg* cfg, p3d_model** out) {
   P3D_REQUIRE(cfg && out, "model_create: null argument");
   P3D_REQUIRE(cfg->linear_size >= 16 && cfg->linear_size % 4 == 0, "linear_size must be a positive multiple of 4");
   P3D_REQUIRE(cfg->num_layers >= 0 && cfg->num_layers <= 64, "num_layers out of range");
-  P3D_REQUIRE(cfg->mode == P3D_MODE_BF16 || cfg->mode == P3D_MODE_FP32 || cfg->mode == P3D_MODE_BF16X3, "unknown mode %d", cfg->mode);
+  P3D_REQUIRE(cfg->mode == P3D_MODE_BF16 || cfg->mode == P3D_MODE_FP32 || cfg->mode == P3D_MODE_BF16X3 || cfg->mode == P3D_MODE_FP16,
+              "unknown mode %d", cfg->mode);
   int ndev = 0;
   P3D_CUDA(cudaGetDeviceCount(&ndev));
   P3D_REQUIRE(cfg->device >= 0 && cfg->device < ndev, "device %d not present (%d devices)", cfg->device, ndev);
@@ -282,7 +283,7 @@ int p3d_model_create(const p3d_cfg* cfg, p3d_model** out) {
   // fixed-size forward scratch exists from the start, so that no forward has to allocate it (a graph capture could not)
   P3D_ALLOC(m->lat_counter, sizeof(unsigned long long) * 32);
   P3D_ALLOC(m->xchg, sizeof(unsigned) * 64);
-  if (L == 1024 && cfg->mode == P3D_MODE_BF16) {       // the whole-chip kernels' exchange buffers (mlp_simt.cu, mlp_mid.cu)
+  if (L == 1024 && (cfg->mode == P3D_MODE_BF16 || cfg->mode == P3D_MODE_FP16)) {   // the whole-chip kernels' exchange buffers (mlp_simt.cu, mlp_mid.cu)
     P3D_ALLOC(m->lat_act, sizeof(uint2) * 1024 * 8 * 128);
     P3D_ALLOC(m->mid_act, sizeof(unsigned long long) * 8 * 64 * 512);
   }
@@ -452,6 +453,9 @@ static int forward_on(p3d_model* m, const float* x, float* y, int64_t B, cudaStr
     return layered::forward_split(m, x, y, B, st);
   }
   const int L = m->L;
+  // fp16 mode: bf16 mode's paths on fp16 operands; widths no tensor-core tiling covers take the FFMA chain, whose
+  // contract is stricter (the bf16-only forward_small is not ported)
+  if (m->cfg.mode == P3D_MODE_FP16 && (L % 8) != 0) return simt::forward_fp32(m, x, y, B, st);
   if (B == 1 && L == 1024) {                            // single pose: whole-chip kernel (or the 16-CTA cluster kernel), one launch
     const int rc = simt::forward_latency_cluster(m, x, y, st);
     if (rc <= 0) return rc;                              // 1 = not schedulable here -> fall through
@@ -469,7 +473,7 @@ static int forward_on(p3d_model* m, const float* x, float* y, int64_t B, cudaStr
     return simt::forward_fp32(m, x, y, B, st);
   }
   P3D_TRY(ensure_xb(m, B, st));
-  P3D_TRY(prep::pack_input(x, m->xb, B, st));
+  P3D_TRY(prep::pack_input(x, m->xb, B, m->cfg.mode == P3D_MODE_FP16, st));
   return forward_packed(m, y, B, st);
 }
 

@@ -1,6 +1,7 @@
 // Shared host-side plumbing for libp3d: error reporting, launch accounting, model state.
 #pragma once
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <cuda_runtime.h>
 
 #include <atomic>
@@ -59,6 +60,26 @@ struct PerDeviceOnce {
   static unsigned long long bit() { int d = 0; cudaGetDevice(&d); return 1ull << (d & 63); }
   bool needed() const { return (mask.load(std::memory_order_acquire) & bit()) == 0; }
   void mark() { mask.fetch_or(bit(), std::memory_order_release); }
+};
+
+// The 16-bit operand type of the inference kernels: bf16 (P3D_MODE_BF16) or fp16 (P3D_MODE_FP16).  Both modes round
+// at the same points; the packed weights, packed input and 16-bit activations hold bf16 or fp16 bits accordingly.
+template <bool F16> struct Op16;
+template <> struct Op16<false> {
+  using T = __nv_bfloat16; using T2 = __nv_bfloat162;
+  static __device__ __forceinline__ T from(float v) { return __float2bfloat16_rn(v); }
+  static __device__ __forceinline__ float to(T v) { return __bfloat162float(v); }
+  static __device__ __forceinline__ T2 pack(float a, float b) { return __floats2bfloat162_rn(a, b); }
+  static __device__ __forceinline__ float lo(T2 v) { return __low2float(v); }
+  static __device__ __forceinline__ float hi(T2 v) { return __high2float(v); }
+};
+template <> struct Op16<true> {
+  using T = __half; using T2 = __half2;
+  static __device__ __forceinline__ T from(float v) { return __float2half_rn(v); }
+  static __device__ __forceinline__ float to(T v) { return __half2float(v); }
+  static __device__ __forceinline__ T2 pack(float a, float b) { return __floats2half2_rn(a, b); }
+  static __device__ __forceinline__ float lo(T2 v) { return __low2float(v); }
+  static __device__ __forceinline__ float hi(T2 v) { return __high2float(v); }
 };
 
 constexpr float kBnEps = 1e-3f;       // tf.layers.batch_normalization default
@@ -263,6 +284,8 @@ struct GemmArgs {
   void* out_bf16 = nullptr; int ld_out_bf16 = 0;
   const void* res_bf16 = nullptr; int ld_res_bf16 = 0;
   int relu = 0;
+  // fp16 operands (P3D_MODE_FP16 inference): A, B, out_bf16 and res_bf16 hold fp16; plain fp32 store or 16-bit output only
+  int f16 = 0;
   // programmatic dependent launch: the kernel may start before its stream predecessor has finished; B (weights)
   // must not depend on that predecessor - its first tiles are fetched ahead of the dependency wait
   int pdl = 0;
@@ -343,7 +366,7 @@ struct p3d_model {
   bool pack_valid = false;
   int rows_total = 0;      // sum of N over layers
   int kpad = 0;            // row pitch (elements) of wt_bf16 = max(L rounded up to 8, 64)
-  __nv_bfloat16* wt_bf16 = nullptr;  // [rows_total][kpad], K-major, BN+clip folded
+  __nv_bfloat16* wt_bf16 = nullptr;  // [rows_total][kpad], K-major, BN+clip folded; fp16 bits in P3D_MODE_FP16
   float* bias_fold = nullptr;        // [rows_total]
   float* wfold = nullptr;            // fp32 folded [K,N] per layer, concatenated
   double* norm2 = nullptr;           // [nlayers] ||W||_F^2

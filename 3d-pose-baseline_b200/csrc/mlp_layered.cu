@@ -2,7 +2,8 @@
 // persistent kernel does not tile (linear_size % 256 != 0): one tcgen05 GEMM per layer (tc_gemm.cu),
 // bias + ReLU (+ residual) fused in the epilogue, bf16 activations ping-ponging between two L2-resident
 // buffers.  Same graph as mlp_tc.cu (src/linear_model.py:102-125,154-201 at isTraining=False) and the same
-// rounding points (relu(.) rounded to bf16, residual added and rounded again), so both paths agree.
+// rounding points (relu(.) rounded to bf16, residual added and rounded again), so both paths agree.  P3D_MODE_FP16
+// models run the same chain on fp16 operands and activations (GemmArgs::f16).
 //
 // Why: a single 128-pose tile walks the six layers of the persistent kernel in ~100 us - one SM (pair) has
 // to stream all 8.6 MB of weights by itself.  Splitting every layer over N (L/64 CTAs) spreads the weight
@@ -32,6 +33,7 @@ static int build_plans(p3d_model* m, const __nv_bfloat16* xb, float* y, int64_t 
     g.B = m->wt_bf16 + static_cast<size_t>(ly.row_off) * kpad; g.ldb = kpad;    // folded W'^T, K-major
     g.bias = m->bias_fold + ly.row_off;
     g.pdl = 1;                                       // layer l+1 starts (and prefetches its weights) while layer l drains
+    g.f16 = m->cfg.mode == P3D_MODE_FP16 ? 1 : 0;
     if (last) {
       g.C = y; g.ldc = m->out_size;
     } else {
@@ -46,7 +48,7 @@ static int build_plans(p3d_model* m, const __nv_bfloat16* xb, float* y, int64_t 
 
 int forward(p3d_model* m, const __nv_bfloat16* xb, float* y, int64_t B, cudaStream_t st) {
   const int L = m->L;
-  P3D_REQUIRE((L % 8) == 0, "layered bf16 path needs linear_size %% 8 == 0 (got %d)", L);
+  P3D_REQUIRE((L % 8) == 0, "layered bf16 / fp16 path needs linear_size %% 8 == 0 (got %d)", L);
   P3D_REQUIRE(B <= 0x7fffffff, "layered path: batch too large");
   bool rebuild = (m->lay_B != B) || (m->lay_x != xb) || m->lay_plans.empty();
   if (m->lay_cap < B) {

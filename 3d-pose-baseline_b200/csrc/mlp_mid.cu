@@ -21,6 +21,8 @@
 //            captured into a CUDA graph gets a fresh tag on every replay
 //   rounding the same points as the tcgen05 paths (x, every ReLU output and every residual sum rounded to bf16, fp32
 //            accumulation): tests/helpers.py:emulate_bf16_forward
+//   fp16     P3D_MODE_FP16 models: F16 = true - fp16 weights, mma.sync .f16 operands, fp16 rounding and {2 x fp16, tag}
+//            exchange words, everything else as above
 #include "common.cuh"
 
 namespace p3d {
@@ -76,14 +78,19 @@ __device__ __forceinline__ void mma_bf16(float (&c)[4], uint32_t a0, uint32_t a1
   asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.bf16.bf16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
                : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3]) : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
 }
-__device__ __forceinline__ float bf16r(float v) { return __bfloat162float(__float2bfloat16_rn(v)); }
-__device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
-  const __nv_bfloat162 p = __floats2bfloat162_rn(lo, hi);
+__device__ __forceinline__ void mma_f16(float (&c)[4], uint32_t a0, uint32_t a1, uint32_t a2, uint32_t a3, uint32_t b0, uint32_t b1) {
+  asm volatile("mma.sync.aligned.m16n8k16.row.col.f32.f16.f16.f32 {%0, %1, %2, %3}, {%4, %5, %6, %7}, {%8, %9}, {%0, %1, %2, %3};"
+               : "+f"(c[0]), "+f"(c[1]), "+f"(c[2]), "+f"(c[3]) : "r"(a0), "r"(a1), "r"(a2), "r"(a3), "r"(b0), "r"(b1));
+}
+template <bool F16> __device__ __forceinline__ float r16(float v) { return Op16<F16>::to(Op16<F16>::from(v)); }
+template <bool F16> __device__ __forceinline__ uint32_t pack16(float lo, float hi) {
+  const typename Op16<F16>::T2 p = Op16<F16>::pack(lo, hi);
   return *reinterpret_cast<const uint32_t*>(&p);
 }
 
-template <int MT>      // m16 tiles per CTA: a row group is 16 MT poses
+template <int MT, bool F16 = false>      // m16 tiles per CTA: a row group is 16 MT poses
 __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
+  using O = Op16<F16>;
   constexpr int RG = 16 * MT;
   extern __shared__ __align__(128) uint8_t mg_smem[];
   uint8_t* base = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(mg_smem) + 127) & ~uintptr_t(127));
@@ -147,19 +154,19 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
       for (int q = 0; q < 4; ++q) {                             // 8 inputs per step
         const uint4 u0 = __ldg(w0 + q), u1 = __ldg(w1 + q);
         const float4 xa = __ldg(xr + 2 * q), xb = __ldg(xr + 2 * q + 1);
-        const float xs[8] = {bf16r(xa.x), bf16r(xa.y), bf16r(xa.z), bf16r(xa.w), bf16r(xb.x), bf16r(xb.y), bf16r(xb.z), bf16r(xb.w)};
-        const __nv_bfloat162* p0 = reinterpret_cast<const __nv_bfloat162*>(&u0);
-        const __nv_bfloat162* p1 = reinterpret_cast<const __nv_bfloat162*>(&u1);
+        const float xs[8] = {r16<F16>(xa.x), r16<F16>(xa.y), r16<F16>(xa.z), r16<F16>(xa.w), r16<F16>(xb.x), r16<F16>(xb.y), r16<F16>(xb.z), r16<F16>(xb.w)};
+        const typename O::T2* p0 = reinterpret_cast<const typename O::T2*>(&u0);
+        const typename O::T2* p1 = reinterpret_cast<const typename O::T2*>(&u1);
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
-          acc0 = fmaf(xs[2 * i], __low2float(p0[i]), acc0); acc0 = fmaf(xs[2 * i + 1], __high2float(p0[i]), acc0);
-          acc1 = fmaf(xs[2 * i], __low2float(p1[i]), acc1); acc1 = fmaf(xs[2 * i + 1], __high2float(p1[i]), acc1);
+          acc0 = fmaf(xs[2 * i], O::lo(p0[i]), acc0); acc0 = fmaf(xs[2 * i + 1], O::hi(p0[i]), acc0);
+          acc1 = fmaf(xs[2 * i], O::lo(p1[i]), acc1); acc1 = fmaf(xs[2 * i + 1], O::hi(p1[i]), acc1);
         }
       }
     }
-    const float v0 = bf16r(fmaxf(acc0 + __ldg(a.bias + n), 0.f)), v1 = bf16r(fmaxf(acc1 + __ldg(a.bias + n + 1), 0.f));
+    const float v0 = r16<F16>(fmaxf(acc0 + __ldg(a.bias + n), 0.f)), v1 = r16<F16>(fmaxf(acc1 + __ldg(a.bias + n + 1), 0.f));
     sres[er * NF + 2 * ej] = v0; sres[er * NF + 2 * ej + 1] = v1;             // block input of the first residual block
-    if (er < live) st_word(words(0, row0 + er) + fg * (NF / 2) + ej, pack_bf16(v0, v1), tag);
+    if (er < live) st_word(words(0, row0 + er) + fg * (NF / 2) + ej, pack16<F16>(v0, v1), tag);
   }
   MID_STAMP(1);
 
@@ -225,7 +232,10 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
         const uint32_t a0 = lds32(ra), a1 = lds32(ra + 8 * PITCH), a2 = lds32(ra + 16), a3 = lds32(ra + 8 * PITCH + 16);
 #pragma unroll
         for (int nt = 0; nt < 2; ++nt)
-          if (nt < ntiles) mma_bf16(acc[mt][nt], a0, a1, a2, a3, bf[nt][0], bf[nt][1]);
+          if (nt < ntiles) {
+            if constexpr (F16) mma_f16(acc[mt][nt], a0, a1, a2, a3, bf[nt][0], bf[nt][1]);
+            else mma_bf16(acc[mt][nt], a0, a1, a2, a3, bf[nt][0], bf[nt][1]);
+          }
       }
     }
   };
@@ -269,12 +279,12 @@ __global__ void __launch_bounds__(MGT, 1) mid_grid_kernel(const Args a) {
         s0 += p.x; s1 += p.y;
       }
       const int n = fg * NF + 2 * ej;
-      float v0 = bf16r(fmaxf(s0 + __ldg(a.bias + l * 1024 + n), 0.f)), v1 = bf16r(fmaxf(s1 + __ldg(a.bias + l * 1024 + n + 1), 0.f));
+      float v0 = r16<F16>(fmaxf(s0 + __ldg(a.bias + l * 1024 + n), 0.f)), v1 = r16<F16>(fmaxf(s1 + __ldg(a.bias + l * 1024 + n + 1), 0.f));
       if (!(l & 1)) {
-        if (a.residual) { v0 = bf16r(v0 + sres[er * NF + 2 * ej]); v1 = bf16r(v1 + sres[er * NF + 2 * ej + 1]); }
+        if (a.residual) { v0 = r16<F16>(v0 + sres[er * NF + 2 * ej]); v1 = r16<F16>(v1 + sres[er * NF + 2 * ej + 1]); }
         sres[er * NF + 2 * ej] = v0; sres[er * NF + 2 * ej + 1] = v1;
       }
-      if (er < live) st_word(words(l, row0 + er) + fg * (NF / 2) + ej, pack_bf16(v0, v1), tag);
+      if (er < live) st_word(words(l, row0 + er) + fg * (NF / 2) + ej, pack16<F16>(v0, v1), tag);
     }
     __syncthreads();                                           // the next gather overwrites the scratch
     MID_STAMP(1 + l);
@@ -319,12 +329,14 @@ int forward(p3d_model* m, const float* x, float* y, int rows, cudaStream_t st) {
   const int mt = rows > 32 ? 2 : 1;
   const int groups = (rows + 16 * mt - 1) / (16 * mt);
   if (m->num_sms < NFG * groups) return 1;
-  if (!m->mid_act) return 1;                            // allocated (2 MB, zero) by p3d_model_create for width 1024 / bf16
+  if (!m->mid_act) return 1;                            // allocated (2 MB, zero) by p3d_model_create for width 1024 / bf16 / fp16
   static PerDeviceOnce attr;
   if (attr.needed()) {
     P3D_TRY(refuse_in_capture(st, "forward: first use of the 9-64 pose whole-chip kernel on this device"));
     P3D_CUDA(cudaFuncSetAttribute(mid_grid_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(1)));
     P3D_CUDA(cudaFuncSetAttribute(mid_grid_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(2)));
+    P3D_CUDA(cudaFuncSetAttribute(mid_grid_kernel<1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(1)));
+    P3D_CUDA(cudaFuncSetAttribute(mid_grid_kernel<2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes(2)));
     attr.mark();
   }
   Args a;
@@ -339,8 +351,9 @@ int forward(p3d_model* m, const float* x, float* y, int rows, cudaStream_t st) {
   cudaLaunchAttribute at[1];
   at[0].id = cudaLaunchAttributeCooperative; at[0].val.cooperative = 1;     // every CTA polls what the others produce
   cfg.attrs = at; cfg.numAttrs = 1;
-  if (mt == 1) P3D_CUDA(cudaLaunchKernelEx(&cfg, mid_grid_kernel<1>, a));
-  else P3D_CUDA(cudaLaunchKernelEx(&cfg, mid_grid_kernel<2>, a));
+  const bool f16 = m->cfg.mode == P3D_MODE_FP16;
+  if (mt == 1) P3D_CUDA(cudaLaunchKernelEx(&cfg, f16 ? mid_grid_kernel<1, true> : mid_grid_kernel<1>, a));
+  else P3D_CUDA(cudaLaunchKernelEx(&cfg, f16 ? mid_grid_kernel<2, true> : mid_grid_kernel<2>, a));
   P3D_LAUNCH_CHECK();
   return P3D_OK;
 }

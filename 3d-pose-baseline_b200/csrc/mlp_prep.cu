@@ -5,8 +5,8 @@
 //   tf.layers.batch_normalization(training=False)   :112,181,193 (moving statistics, eps 1e-3)
 // into  W' = W * clip_scale * s,  b' = (b - moving_mean) * s + beta,  s = gamma / sqrt(moving_var + eps)
 // and writes them (a) fp32 [K,N] for the FFMA path and (b) bf16 transposed [N,Kpad] (K contiguous) for
-// the tcgen05 path, all layers stacked along rows; bf16x3 models also get (c) the split pair of (b), bf16(W') and
-// bf16(W' - bf16(W')), side by side in each row.
+// the tcgen05 path, all layers stacked along rows (fp16 instead of bf16 for P3D_MODE_FP16 models); bf16x3 models also
+// get (c) the split pair of (b), bf16(W') and bf16(W' - bf16(W')), side by side in each row.
 #include <cstring>
 
 #include "common.cuh"
@@ -48,6 +48,7 @@ struct FoldArgs {
   int K, N, kpad, seg3;
 };
 
+template <bool F16>
 __global__ void fold_pack_kernel(const FoldArgs a) {
   __shared__ float tile[32][33];
   const int n0 = blockIdx.x * 32, k0 = blockIdx.y * 32;
@@ -74,6 +75,10 @@ __global__ void fold_pack_kernel(const FoldArgs a) {
     const int n = n0 + nn, k = k0 + threadIdx.x;
     if (n < a.N && k < a.K) {
       const float v = tile[threadIdx.x][nn];
+      if constexpr (F16) {
+        reinterpret_cast<__half*>(a.wt)[static_cast<size_t>(n) * a.kpad + k] = __float2half_rn(v);
+        continue;
+      }
       const __nv_bfloat16 hi = __float2bfloat16_rn(v);
       a.wt[static_cast<size_t>(n) * a.kpad + k] = hi;
       if (a.wt3) {
@@ -96,8 +101,10 @@ __global__ void fold_pack_kernel(const FoldArgs a) {
   }
 }
 
-// x fp32 [B,32] -> bf16 [B,64], columns 32..63 zero (layer 0 runs as one K=64 swizzle atom)
+// x fp32 [B,32] -> bf16 (fp16: F16) [B,64], columns 32..63 zero (layer 0 runs as one K=64 swizzle atom)
+template <bool F16>
 __global__ void pack_input_kernel(const float* __restrict__ x, __nv_bfloat16* __restrict__ xb, long long B) {
+  using O = Op16<F16>;
   const long long idx = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x;   // one 8-element group
   if (idx >= B * 8) return;
   const long long row = idx >> 3;
@@ -106,8 +113,8 @@ __global__ void pack_input_kernel(const float* __restrict__ x, __nv_bfloat16* __
   if (g < 4) {
     const float4* xp = reinterpret_cast<const float4*>(x + row * kIn + g * 8);
     const float4 a = __ldg(xp), b = __ldg(xp + 1);
-    __nv_bfloat162 p0 = __floats2bfloat162_rn(a.x, a.y), p1 = __floats2bfloat162_rn(a.z, a.w);
-    __nv_bfloat162 p2 = __floats2bfloat162_rn(b.x, b.y), p3 = __floats2bfloat162_rn(b.z, b.w);
+    typename O::T2 p0 = O::pack(a.x, a.y), p1 = O::pack(a.z, a.w);
+    typename O::T2 p2 = O::pack(b.x, b.y), p3 = O::pack(b.z, b.w);
     o.x = *reinterpret_cast<uint32_t*>(&p0); o.y = *reinterpret_cast<uint32_t*>(&p1);
     o.z = *reinterpret_cast<uint32_t*>(&p2); o.w = *reinterpret_cast<uint32_t*>(&p3);
   }
@@ -169,16 +176,19 @@ int prepare(p3d_model* m, cudaStream_t st) {
     a.bias_fold = m->bias_fold + ly.row_off;
     a.K = ly.K; a.N = ly.N; a.kpad = m->kpad; a.seg3 = m->x3_seg;
     dim3 grid((ly.N + 31) / 32, (ly.K + 31) / 32), block(32, 8);
-    fold_pack_kernel<<<grid, block, 0, st>>>(a);
+    if (m->cfg.mode == P3D_MODE_FP16) fold_pack_kernel<true><<<grid, block, 0, st>>>(a);
+    else fold_pack_kernel<false><<<grid, block, 0, st>>>(a);
     P3D_LAUNCH_CHECK();
   }
   m->pack_valid = true;
   return P3D_OK;
 }
 
-int pack_input(const float* x, __nv_bfloat16* xb, int64_t B, cudaStream_t st) {
+int pack_input(const float* x, __nv_bfloat16* xb, int64_t B, bool f16, cudaStream_t st) {
   const long long groups = B * 8;
-  pack_input_kernel<<<static_cast<unsigned>((groups + 255) / 256), 256, 0, st>>>(x, xb, B);
+  const unsigned blocks = static_cast<unsigned>((groups + 255) / 256);
+  if (f16) pack_input_kernel<true><<<blocks, 256, 0, st>>>(x, xb, B);
+  else pack_input_kernel<false><<<blocks, 256, 0, st>>>(x, xb, B);
   P3D_LAUNCH_CHECK();
   return P3D_OK;
 }

@@ -418,7 +418,9 @@ __device__ __forceinline__ void bulk_load(void* dst, const void* src, uint32_t b
 __device__ __forceinline__ unsigned long long gtimer() { unsigned long long t; asm volatile("mov.u64 %0, %%globaltimer;" : "=l"(t)); return t; }
 #define LAT_STAMP(i) do { if (a.stamps && threadIdx.x == 0 && rank == 0) a.stamps[i] = gtimer(); } while (0)
 
+template <bool F16 = false>     // F16: fp16 weights (P3D_MODE_FP16)
 __global__ void __launch_bounds__(LNT, 1) latency_cluster_kernel(const LatArgs a) {
+  using O = Op16<F16>;
   constexpr int L = 1024;
   extern __shared__ __align__(128) uint8_t lat_smem[];
   __shared__ __align__(16) float sP[L];
@@ -476,8 +478,8 @@ __global__ void __launch_bounds__(LNT, 1) latency_cluster_kernel(const LatArgs a
     if (lane < 8) { const float4 h = *reinterpret_cast<const float4*>(sQ + lane * 4); hv4[0] = h.x; hv4[1] = h.y; hv4[2] = h.z; hv4[3] = h.w; }
 #pragma unroll
     for (int o = 0; o < LOPW; ++o) {
-      const __nv_bfloat162* w2 = reinterpret_cast<const __nv_bfloat162*>(&w0[o]);
-      float acc = hv4[0] * __low2float(w2[0]) + hv4[1] * __high2float(w2[0]) + hv4[2] * __low2float(w2[1]) + hv4[3] * __high2float(w2[1]);
+      const typename O::T2* w2 = reinterpret_cast<const typename O::T2*>(&w0[o]);
+      float acc = hv4[0] * O::lo(w2[0]) + hv4[1] * O::hi(w2[0]) + hv4[2] * O::lo(w2[1]) + hv4[3] * O::hi(w2[1]);
       for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
       const float v = fmaxf(acc + b0[o], 0.f);
       if (lane < LC) st_cluster_f32(sP + rank * 64 + o * LNW + warp, static_cast<uint32_t>(lane), v);
@@ -511,9 +513,9 @@ __global__ void __launch_bounds__(LNT, 1) latency_cluster_kernel(const LatArgs a
 #pragma unroll
       for (int i = 0; i < 8; ++i) {
         const uint2 wv = wrow[i * 32 + lane];                         // k = i*128 + lane*4 .. +3 : conflict-free
-        const __nv_bfloat162* w2 = reinterpret_cast<const __nv_bfloat162*>(&wv);
-        acc0 = fmaf(hreg[i].x, __low2float(w2[0]), acc0); acc1 = fmaf(hreg[i].y, __high2float(w2[0]), acc1);
-        acc0 = fmaf(hreg[i].z, __low2float(w2[1]), acc0); acc1 = fmaf(hreg[i].w, __high2float(w2[1]), acc1);
+        const typename O::T2* w2 = reinterpret_cast<const typename O::T2*>(&wv);
+        acc0 = fmaf(hreg[i].x, O::lo(w2[0]), acc0); acc1 = fmaf(hreg[i].y, O::hi(w2[0]), acc1);
+        acc0 = fmaf(hreg[i].z, O::lo(w2[1]), acc0); acc1 = fmaf(hreg[i].w, O::hi(w2[1]), acc1);
       }
       __syncwarp();
       if (lane == 0) lat_mbar_arrive(&wfree[slot]);                   // this warp is done with the slot
@@ -544,9 +546,9 @@ __global__ void __launch_bounds__(LNT, 1) latency_cluster_kernel(const LatArgs a
       for (int i = 0; i < 8; ++i) {
         const uint2 wv = __ldg(reinterpret_cast<const uint2*>(wrow + i * 128 + lane * 4));
         const float4 hv = *reinterpret_cast<const float4*>(src + i * 128 + lane * 4);
-        const __nv_bfloat162* w2 = reinterpret_cast<const __nv_bfloat162*>(&wv);
-        acc = fmaf(hv.x, __low2float(w2[0]), acc); acc = fmaf(hv.y, __high2float(w2[0]), acc);
-        acc = fmaf(hv.z, __low2float(w2[1]), acc); acc = fmaf(hv.w, __high2float(w2[1]), acc);
+        const typename O::T2* w2 = reinterpret_cast<const typename O::T2*>(&wv);
+        acc = fmaf(hv.x, O::lo(w2[0]), acc); acc = fmaf(hv.y, O::hi(w2[0]), acc);
+        acc = fmaf(hv.z, O::lo(w2[1]), acc); acc = fmaf(hv.w, O::hi(w2[1]), acc);
       }
       for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
       if (lane == 0) {
@@ -577,15 +579,17 @@ static int launch_latency_cluster(p3d_model* m, const float* x, float* y, const 
   if (ok < 0) {
     P3D_TRY(refuse_in_capture(st, "forward: probing the 16-CTA cluster kernel"));
     ok = 0;
-    if (cudaFuncSetAttribute(latency_cluster_kernel, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess &&
-        cudaFuncSetAttribute(latency_cluster_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, LAT_SMEM) == cudaSuccess) {
+    if (cudaFuncSetAttribute(latency_cluster_kernel<false>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess &&
+        cudaFuncSetAttribute(latency_cluster_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, LAT_SMEM) == cudaSuccess &&
+        cudaFuncSetAttribute(latency_cluster_kernel<true>, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess &&
+        cudaFuncSetAttribute(latency_cluster_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, LAT_SMEM) == cudaSuccess) {
       cudaLaunchConfig_t cfg{};
       cfg.gridDim = dim3(LC); cfg.blockDim = dim3(LNT); cfg.dynamicSmemBytes = LAT_SMEM;
       cudaLaunchAttribute attr[1];
       attr[0].id = cudaLaunchAttributeClusterDimension; attr[0].val.clusterDim.x = LC; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
       cfg.attrs = attr; cfg.numAttrs = 1;
       int nclusters = 0;
-      if (cudaOccupancyMaxActiveClusters(&nclusters, latency_cluster_kernel, &cfg) == cudaSuccess && nclusters >= 1) ok = 1;
+      if (cudaOccupancyMaxActiveClusters(&nclusters, latency_cluster_kernel<false>, &cfg) == cudaSuccess && nclusters >= 1) ok = 1;
     }
     cudaGetLastError();
     if (const char* e = getenv("P3D_LAT_CLUSTER")) ok = ok && atoi(e);
@@ -602,7 +606,8 @@ static int launch_latency_cluster(p3d_model* m, const float* x, float* y, const 
   cudaLaunchAttribute attr[1];
   attr[0].id = cudaLaunchAttributeClusterDimension; attr[0].val.clusterDim.x = LC; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr; cfg.numAttrs = 1;
-  P3D_CUDA(cudaLaunchKernelEx(&cfg, latency_cluster_kernel, a));
+  if (m->cfg.mode == P3D_MODE_FP16) P3D_CUDA(cudaLaunchKernelEx(&cfg, latency_cluster_kernel<true>, a));
+  else P3D_CUDA(cudaLaunchKernelEx(&cfg, latency_cluster_kernel<false>, a));
   P3D_LAUNCH_CHECK();
   return P3D_OK;
 }
@@ -639,8 +644,9 @@ __device__ __forceinline__ uint4 ld_ll2(const uint2* p) {
 }
 #define GLAT_STAMP(i) do { if (a.stamps && threadIdx.x == 0 && blockIdx.x == 0) a.stamps[i] = gtimer(); } while (0)
 
-template <int ROWS>      // poses served by one launch (1, 2, 4 or 8; a.rows <= ROWS of them are live)
+template <int ROWS, bool F16 = false>      // poses served by one launch (1, 2, 4 or 8; a.rows <= ROWS of them are live); F16: fp16 weights
 __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs a) {
+  using O = Op16<F16>;
   constexpr int L = 1024;
   extern __shared__ __align__(128) uint8_t glat_smem[];
   const int c = blockIdx.x, lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
@@ -684,14 +690,14 @@ __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs 
   {
     uint2 wv = make_uint2(0, 0);
     if (lane < 8) wv = __ldg(reinterpret_cast<const uint2*>(a.wt + static_cast<size_t>(n) * a.kpad + lane * 4));
-    const __nv_bfloat162* w2 = reinterpret_cast<const __nv_bfloat162*>(&wv);
+    const typename O::T2* w2 = reinterpret_cast<const typename O::T2*>(&wv);
     const float b = __ldg(a.bias + n);
 #pragma unroll
     for (int r = 0; r < ROWS; ++r) {
       float acc = 0.f;
       if (lane < 8 && r < a.rows) {
         const float4 h = __ldg(reinterpret_cast<const float4*>(a.x + r * kIn + lane * 4));
-        acc = h.x * __low2float(w2[0]) + h.y * __high2float(w2[0]) + h.z * __low2float(w2[1]) + h.w * __high2float(w2[1]);
+        acc = h.x * O::lo(w2[0]) + h.y * O::hi(w2[0]) + h.z * O::lo(w2[1]) + h.w * O::hi(w2[1]);
       }
       for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
       if (lane == 0) spub[r][warp] = fmaxf(acc + b, 0.f);
@@ -744,8 +750,8 @@ __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs 
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
       const uint2 wv = wrow[i * 32 + lane];                         // k = i*128 + lane*4 .. +3 : conflict-free
-      const __nv_bfloat162* w2 = reinterpret_cast<const __nv_bfloat162*>(&wv);
-      const float w0 = __low2float(w2[0]), w1 = __high2float(w2[0]), w2f = __low2float(w2[1]), w3 = __high2float(w2[1]);
+      const typename O::T2* w2 = reinterpret_cast<const typename O::T2*>(&wv);
+      const float w0 = O::lo(w2[0]), w1 = O::hi(w2[0]), w2f = O::lo(w2[1]), w3 = O::hi(w2[1]);
 #pragma unroll
       for (int r = 0; r < ROWS; ++r) {
         const float4 h = *reinterpret_cast<const float4*>(src + r * L + i * 128 + lane * 4);
@@ -782,9 +788,9 @@ __global__ void __launch_bounds__(GLT, 1) latency_grid_kernel(const GridLatArgs 
       for (int i = 0; i < 8; ++i) {
         const uint2 wv = wrow[i * 32 + lane];
         const float4 hv = *reinterpret_cast<const float4*>(src + warp * L + i * 128 + lane * 4);
-        const __nv_bfloat162* w2 = reinterpret_cast<const __nv_bfloat162*>(&wv);
-        acc = fmaf(hv.x, __low2float(w2[0]), acc); acc = fmaf(hv.y, __high2float(w2[0]), acc);
-        acc = fmaf(hv.z, __low2float(w2[1]), acc); acc = fmaf(hv.w, __high2float(w2[1]), acc);
+        const typename O::T2* w2 = reinterpret_cast<const typename O::T2*>(&wv);
+        acc = fmaf(hv.x, O::lo(w2[0]), acc); acc = fmaf(hv.y, O::hi(w2[0]), acc);
+        acc = fmaf(hv.z, O::lo(w2[1]), acc); acc = fmaf(hv.w, O::hi(w2[1]), acc);
       }
       for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
       if (lane == 0) a.y[warp * a.out + c] = acc + __ldg(a.bias + l * L + c);
@@ -804,13 +810,16 @@ static int launch_latency_grid(p3d_model* m, const float* x, float* y, int rows,
   if (R < rmin) R = rmin;
   const int smem = 128 + nhid * (GLF * 2048) + 2048 + 2 * R * 1024 * 4 + 8 * (nhid + 1) + 64;
   using K = void (*)(const GridLatArgs);
-  const K fn = R == 1 ? latency_grid_kernel<1> : (R == 2 ? latency_grid_kernel<2> : (R == 4 ? latency_grid_kernel<4> : latency_grid_kernel<8>));
-  if (!m->lat_act) return 1;                           // allocated (8 MB, zero) by p3d_model_create for width 1024 / bf16
+  const bool f16 = m->cfg.mode == P3D_MODE_FP16;
+  const K fn = f16 ? (R == 1 ? latency_grid_kernel<1, true> : (R == 2 ? latency_grid_kernel<2, true> : (R == 4 ? latency_grid_kernel<4, true> : latency_grid_kernel<8, true>)))
+                   : (R == 1 ? latency_grid_kernel<1> : (R == 2 ? latency_grid_kernel<2> : (R == 4 ? latency_grid_kernel<4> : latency_grid_kernel<8>)));
+  if (!m->lat_act) return 1;                           // allocated (8 MB, zero) by p3d_model_create for width 1024 / bf16 / fp16
   static PerDeviceOnce attr;
   if (attr.needed()) {
     P3D_TRY(refuse_in_capture(st, "forward: first use of the whole-chip kernel on this device"));
     const int cap = 128 + 6 * (GLF * 2048) + 2048 + 2 * 8 * 1024 * 4 + 256;
-    for (K k : {static_cast<K>(latency_grid_kernel<1>), static_cast<K>(latency_grid_kernel<2>), static_cast<K>(latency_grid_kernel<4>), static_cast<K>(latency_grid_kernel<8>)})
+    for (K k : {static_cast<K>(latency_grid_kernel<1>), static_cast<K>(latency_grid_kernel<2>), static_cast<K>(latency_grid_kernel<4>), static_cast<K>(latency_grid_kernel<8>),
+                static_cast<K>(latency_grid_kernel<1, true>), static_cast<K>(latency_grid_kernel<2, true>), static_cast<K>(latency_grid_kernel<4, true>), static_cast<K>(latency_grid_kernel<8, true>)})
       P3D_CUDA(cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, cap));
     attr.mark();
   }
@@ -841,7 +850,7 @@ int forward_latency_cluster(p3d_model* m, const float* x, float* y, cudaStream_t
 // the 16-CTA cluster kernel: fused into the whole-chip kernel (128 CTAs reading the keypoints from mapped host memory, 48
 // output CTAs writing y / pose there behind system-scope fences and counting themselves) a frame took 181 us instead of 49.
 int forward_latency_cluster_rt(p3d_model* m, const rt::Fused& f, float* y, cudaStream_t st) {
-  if (m->L != 1024 || m->cfg.mode != P3D_MODE_BF16) return 1;
+  if (m->L != 1024 || (m->cfg.mode != P3D_MODE_BF16 && m->cfg.mode != P3D_MODE_FP16)) return 1;
   return launch_latency_cluster(m, nullptr, y, &f, st);
 }
 

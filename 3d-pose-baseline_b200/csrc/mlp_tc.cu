@@ -13,7 +13,7 @@
 //                           layer transitions are a larger share)
 //   warp 1   MMA issuer   : tcgen05.mma 128x256x16 (one elected lane, warp-uniform operands), fp32
 //                           accumulators in TMEM, 2 x 256 columns double buffered against the epilogue
-//   warps 4-7 epilogue    : tcgen05.ld -> +bias -> ReLU -> bf16 -> swizzled smem tile -> TMA store
+//   warps 4-7 epilogue    : tcgen05.ld -> +bias -> ReLU -> bf16 (fp16: F16) -> swizzled smem tile -> TMA store
 //                           (cp.reduce.async.bulk .add when the block's residual is added: the L2
 //                           performs  P += tile  so the residual is never re-read by the SM), or fp32 y
 // Layers are chained through per-256-column "chunk done" mbarriers: the producer may load the K
@@ -90,8 +90,8 @@ struct Params {
   float* y;                  // [B][out_valid]
 };
 
-__device__ __forceinline__ uint32_t pack_bf16x2(float a, float b) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
+template <bool F16> __device__ __forceinline__ uint32_t pack_16x2(float a, float b) {    // F16: cvt.rn.f16x2.f32
+  typename Op16<F16>::T2 v = Op16<F16>::pack(a, b);
   return *reinterpret_cast<uint32_t*>(&v);
 }
 
@@ -102,7 +102,7 @@ __device__ __forceinline__ uint64_t desc_at(uint32_t smem_addr) {
   return (static_cast<uint64_t>(hi) << 32) | lo;
 }
 
-template <int CG>
+template <int CG, bool F16 = false>
 __global__ void __launch_bounds__(NTHREADS, 1)
 mlp_forward_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_constant__ CUtensorMap tm_act,
                       const __grid_constant__ CUtensorMap tm_w, const __grid_constant__ CUtensorMap tm_wout,
@@ -203,8 +203,8 @@ mlp_forward_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_con
   } else if (warp == 1 && leader) {
     // ------------------------------------------------------------ MMA issuer (warp-uniform loop, one elected lane issues)
     int stage = 0; uint32_t phase = 0; uint32_t q = 0;
-    const uint32_t idesc_hidden = umma_idesc_bf16_f32(BM * CG, BN);
-    const uint32_t idesc_out = umma_idesc_bf16_f32(BM * CG, p.out_n);
+    const uint32_t idesc_hidden = umma_idesc_16_f32<F16>(BM * CG, BN);
+    const uint32_t idesc_out = umma_idesc_16_f32<F16>(BM * CG, p.out_n);
     const uint32_t a_base = smem_u32(sA), b_base = smem_u32(sB);
     for (int gt = group_id; gt < ngtiles; gt += ngroups) {
       for (int l = 0; l < nlayers; ++l) {
@@ -308,9 +308,9 @@ mlp_forward_tc_kernel(const __grid_constant__ CUtensorMap tm_x, const __grid_con
               const float* bs = sBias + s * 64;
 #pragma unroll
               for (int j = 0; j < 16; ++j) {
-                o[j] = pack_bf16x2(fmaxf(__uint_as_float(v0[2 * j]) + bs[2 * j], 0.f),
+                o[j] = pack_16x2<F16>(fmaxf(__uint_as_float(v0[2 * j]) + bs[2 * j], 0.f),
                                    fmaxf(__uint_as_float(v0[2 * j + 1]) + bs[2 * j + 1], 0.f));
-                o[16 + j] = pack_bf16x2(fmaxf(__uint_as_float(v1[2 * j]) + bs[32 + 2 * j], 0.f),
+                o[16 + j] = pack_16x2<F16>(fmaxf(__uint_as_float(v1[2 * j]) + bs[32 + 2 * j], 0.f),
                                         fmaxf(__uint_as_float(v1[2 * j + 1]) + bs[32 + 2 * j + 1], 0.f));
               }
               mbar_wait(stg_free, (nslab & 1) ^ 1, 5);    // the store warp has read the previous slab out of the staging tile
@@ -424,23 +424,23 @@ static EncodeTiledFn get_encode_fn() {
   return fn;
 }
 
-// bf16 row-major [rows][pitch_elems] tensor, box = [box_rows][64 cols], 128B swizzle
+// bf16 (f16: fp16) row-major [rows][pitch_elems] tensor, box = [box_rows][64 cols], 128B swizzle
 static int make_tmap(CUtensorMap* out, const void* base, uint64_t rows, uint64_t cols, uint64_t pitch_elems,
-                     uint32_t box_rows) {
+                     uint32_t box_rows, bool f16 = false) {
   EncodeTiledFn fn = get_encode_fn();
   if (!fn) { set_error("cuTensorMapEncodeTiled entry point not available"); return P3D_ERR_CUDA; }
   cuuint64_t gdim[2] = {cols, rows};
   cuuint64_t gstride[1] = {pitch_elems * 2};
   cuuint32_t box[2] = {static_cast<cuuint32_t>(BK), box_rows};
   cuuint32_t estr[2] = {1, 1};
-  CUresult r = fn(out, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gdim, gstride, box, estr,
+  CUresult r = fn(out, f16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void*>(base), gdim, gstride, box, estr,
                   CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                   CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) { set_error("cuTensorMapEncodeTiled failed with CUresult %d", (int)r); return P3D_ERR_CUDA; }
   return P3D_OK;
 }
 
-template <int CG>
+template <int CG, bool F16>
 static int launch_forward(p3d_model* m, const __nv_bfloat16* xb, float* y, int64_t B, cudaStream_t st) {
   using T = Tile<CG>;
   const int L = m->L;
@@ -452,7 +452,9 @@ static int launch_forward(p3d_model* m, const __nv_bfloat16* xb, float* y, int64
   const int out_n = (m->out_size + 15) / 16 * 16;
   CUtensorMap tm_x, tm_act, tm_w, tm_wout;
   P3D_TRY(make_tmap(&tm_x, xb, static_cast<uint64_t>(B), 64, 64, BM));
-  P3D_TRY(make_tmap(&tm_act, m->act_scratch, 2ull * grid * BM, L, L, BM));
+  // the residual is added by cp.reduce.async.bulk.tensor .add, whose arithmetic follows the map's data type: an fp16
+  // model's activation map must say FLOAT16 (the loads are bit copies either way)
+  P3D_TRY(make_tmap(&tm_act, m->act_scratch, 2ull * grid * BM, L, L, BM, F16));
   P3D_TRY(make_tmap(&tm_w, m->wt_bf16, static_cast<uint64_t>(nlayers - 1) * L, m->kpad, m->kpad, T::B_ROWS));
   P3D_TRY(make_tmap(&tm_wout, m->wt_bf16 + static_cast<size_t>(nlayers - 1) * L * m->kpad, out_n, m->kpad, m->kpad, out_n / CG));
   Params p;
@@ -461,7 +463,7 @@ static int launch_forward(p3d_model* m, const __nv_bfloat16* xb, float* y, int64
   p.bias = m->bias_fold; p.y = y;
   static PerDeviceOnce attr_set;
   if (attr_set.needed()) {
-    P3D_CUDA(cudaFuncSetAttribute(mlp_forward_tc_kernel<CG>, cudaFuncAttributeMaxDynamicSharedMemorySize, T::SMEM_BYTES));
+    P3D_CUDA(cudaFuncSetAttribute(mlp_forward_tc_kernel<CG, F16>, cudaFuncAttributeMaxDynamicSharedMemorySize, T::SMEM_BYTES));
     attr_set.mark();
   }
   cudaLaunchConfig_t cfg{};
@@ -502,7 +504,7 @@ static int launch_forward(p3d_model* m, const __nv_bfloat16* xb, float* y, int64
   }
   cudaEvent_t e0 = nullptr, e1 = nullptr;
   if (prof::enabled() && !cap) prof::begin(st, &e0, &e1);     // timing events are read on the host: eager launches only
-  P3D_CUDA(cudaLaunchKernelEx(&cfg, mlp_forward_tc_kernel<CG>, tm_x, tm_act, tm_w, tm_wout, p));
+  P3D_CUDA(cudaLaunchKernelEx(&cfg, mlp_forward_tc_kernel<CG, F16>, tm_x, tm_act, tm_w, tm_wout, p));
   P3D_LAUNCH_CHECK();
   if (e0) prof::end(st, e0, e1);
   return P3D_OK;
@@ -523,7 +525,8 @@ int forward_bf16(p3d_model* m, const __nv_bfloat16* xb, float* y, int64_t B, cud
     const char* e = getenv("P3D_TC_CG");       // 1 = single-CTA tiles, 2 = CTA pairs (default)
     cg = (e && e[0] == '1') ? 1 : 2;
   }
-  return cg == 1 ? launch_forward<1>(m, xb, y, B, st) : launch_forward<2>(m, xb, y, B, st);
+  if (m->cfg.mode == P3D_MODE_FP16) return cg == 1 ? launch_forward<1, true>(m, xb, y, B, st) : launch_forward<2, true>(m, xb, y, B, st);
+  return cg == 1 ? launch_forward<1, false>(m, xb, y, B, st) : launch_forward<2, false>(m, xb, y, B, st);
 }
 
 int debug_umma_gemm(const void* A, const void* W, float* C, int N, int K, cudaStream_t st) {

@@ -286,5 +286,13 @@ __device__ __forceinline__ void tmem_st_32x32b_x32(uint32_t taddr, const uint32_
 }
 __device__ __forceinline__ void tmem_st_wait() { asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory"); }
 
+// umma_idesc_bf16_f32 with A=B=fp16: a_format (bits 7-9) and b_format (bits 10-12) 0 = F16; the same kind::f16 MMA
+__host__ __device__ constexpr uint32_t umma_idesc_f16_f32(uint32_t M, uint32_t N) {
+  return (1u << 4) | ((N >> 3) << 17) | ((M >> 4) << 24);
+}
+template <bool F16> __host__ __device__ constexpr uint32_t umma_idesc_16_f32(uint32_t M, uint32_t N) {
+  return F16 ? umma_idesc_f16_f32(M, N) : umma_idesc_bf16_f32(M, N);
+}
+
 }  // namespace ptx
 }  // namespace p3d

@@ -292,11 +292,15 @@ __device__ __forceinline__ void totals_wait(const Params& p, int n0, int et, dou
 // bf16 hi / lo halves to out_b).  RES: a residual operand is added.  CS: column sums of the result and its
 // square are accumulated (BatchNorm statistics of a forward layer on the unfused path).  SEG: segment schedule of the
 // split-precision (bf16x3) GEMMs, inference and training - the K loop runs three passes, reading the (A, B) segments
-// (hi, hi), (lo, hi), (hi, lo) into one accumulator; either operand K-major or MN-major, K split or not.
-template <int OUT, bool RES, int CS, bool SEG = false>
+// (hi, hi), (lo, hi), (hi, lo) into one accumulator; either operand K-major or MN-major, K split or not.  F16: fp16
+// operands (P3D_MODE_FP16 inference: the fp32 store and the 16-bit activation store, OUT 0 / 2), where OUT = 2 stores
+// and reads fp16 activations.
+template <int OUT, bool RES, int CS, bool SEG = false, bool F16 = false>
 __global__ void __launch_bounds__((OUT == 3 || OUT == 4) ? FUSED_NTHREADS : NTHREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
   static_assert(CS == 0 || OUT < 2, "column sums are taken of the fp32 stores only");
+  static_assert(!F16 || ((OUT == 0 || OUT == 2) && !SEG && CS == 0), "fp16 operands: the inference epilogues only");
+  using O16 = Op16<F16>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
   const int STAGES = p.stages;
@@ -404,7 +408,7 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
     // eight descriptors per k-block from byte addresses cost ~110 SASS instructions between the barrier and the first
     // tcgen05.mma, against 4 x 56 cycles of tensor work at N <= 64; measured: 16.9 -> 14.7 us for a 4096 x 1024 x 1024
     // GEMM, 48 -> 40 us for the six-layer batch-64 inference chain.)
-    const uint32_t idesc = umma_idesc_bf16_f32(BM, p.bn) | (p.a_mn ? (1u << 15) : 0u) | (p.b_mn ? (1u << 16) : 0u);
+    const uint32_t idesc = umma_idesc_16_f32<F16>(BM, p.bn) | (p.a_mn ? (1u << 15) : 0u) | (p.b_mn ? (1u << 16) : 0u);
     const uint32_t a_base = smem_u32(sA), b_base = smem_u32(sB);
     const uint32_t a_step = p.a_mn ? 2048u : 32u, b_step = p.b_mn ? 2048u : 32u;   // bytes per K=16 slice
     const uint64_t a0 = p.a_mn ? desc_mn(a_base) : desc_k(a_base), b0 = p.b_mn ? desc_mn(b_base) : desc_k(b_base);
@@ -869,15 +873,15 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
           float o[4] = {alpha * t4[i].x + b4.x, alpha * t4[i].y + b4.y, alpha * t4[i].z + b4.z, alpha * t4[i].w + b4.w};
           if (OUT == 2) {
             // bf16 activations of the layered inference path: same rounding points as the fused persistent kernel
-            // (relu(.) rounded to bf16, then the residual added and rounded again)
-            __nv_bfloat16 ob[4];
+            // (relu(.) rounded to bf16 / fp16, then the residual added and rounded again)
+            typename O16::T ob[4];
 #pragma unroll
-            for (int j = 0; j < 4; ++j) ob[j] = __float2bfloat16_rn(p.relu ? fmaxf(o[j], 0.f) : o[j]);
+            for (int j = 0; j < 4; ++j) ob[j] = O16::from(p.relu ? fmaxf(o[j], 0.f) : o[j]);
             if (use_res) {
-              __nv_bfloat16 rv[4];
+              typename O16::T rv[4];
               memcpy(rv, &rb[i], 8);
 #pragma unroll
-              for (int j = 0; j < 4; ++j) ob[j] = __float2bfloat16_rn(__bfloat162float(ob[j]) + __bfloat162float(rv[j]));
+              for (int j = 0; j < 4; ++j) ob[j] = O16::from(O16::to(ob[j]) + O16::to(rv[j]));
             }
             uint2 q; memcpy(&q, ob, 8);
             if (live) *reinterpret_cast<uint2*>(p.out_b + static_cast<size_t>(m) * p.ldob + n) = q;
@@ -929,9 +933,10 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
             if (n + j >= p.N) continue;
             float o = alpha * tv[j] + bias[j];
             if (OUT == 2) {
-              __nv_bfloat16 ob = __float2bfloat16_rn(p.relu ? fmaxf(o, 0.f) : o);
-              if (use_res) ob = __float2bfloat16_rn(__bfloat162float(ob) + __bfloat162float(p.res_b[static_cast<size_t>(m) * p.ldrb + n + j]));
-              p.out_b[static_cast<size_t>(m) * p.ldob + n + j] = ob;
+              using T16 = typename O16::T;
+              T16 ob = O16::from(p.relu ? fmaxf(o, 0.f) : o);
+              if (use_res) ob = O16::from(O16::to(ob) + O16::to(reinterpret_cast<const T16*>(p.res_b)[static_cast<size_t>(m) * p.ldrb + n + j]));
+              reinterpret_cast<T16*>(p.out_b)[static_cast<size_t>(m) * p.ldob + n + j] = ob;
             } else if (OUT == 5) {
               float r = p.relu ? fmaxf(o, 0.f) : o;
               if (use_res) r += p.res[static_cast<size_t>(m) * p.ldres + n + j];
@@ -1058,7 +1063,7 @@ static int make_map(CUtensorMap* out, const void* base, uint64_t inner, uint64_t
 }
 
 // A: a_mn ? [K][M] : [M][K];  B: b_mn ? [K][N] : [N][K]  (bf16, pitches lda/ldb in elements)
-struct PlanData { CUtensorMap ta, tb; Params p; dim3 grid; int pdl; int fused_mode; int coop; };
+struct PlanData { CUtensorMap ta, tb; Params p; dim3 grid; int pdl; int fused_mode; int coop; int f16; };
 static_assert(sizeof(PlanData) <= sizeof(GemmPlan::blob), "GemmPlan::blob too small");
 
 // tile width: the widest BN that still gives the grid about one CTA per SM; a split-K problem keeps the
@@ -1156,6 +1161,9 @@ int plan(const GemmArgs& g, GemmPlan* out) {
   p.ft = g.fused;
   d->fused_mode = g.fused_mode;
   d->coop = 0;
+  d->f16 = g.f16;
+  P3D_REQUIRE(!g.f16 || (!seg && !g.fused_mode && !g.colsum && !g.split_k && !g.accumulate && !(g.C && g.out_bf16)),
+              "tc_gemm: fp16 operands take the inference epilogues only (fp32 store or 16-bit activations)");
   if (g.fused_mode) {
     P3D_REQUIRE(g.fused_mode == 3 || g.fused_mode == 4, "tc_gemm: unknown fused mode %d", g.fused_mode);
     P3D_REQUIRE(splits == 1 && (g.N % 32) == 0 && g.ldc == g.N && !g.out_bf16 && !g.colsum && !g.pdl,
@@ -1193,6 +1201,12 @@ int launch(const GemmPlan& pl, cudaStream_t st) {
   P3D_TCG_PICK(1, false, 0) P3D_TCG_PICK(1, true, 0)
   P3D_TCG_PICK(2, false, 0) P3D_TCG_PICK(2, true, 0)
 #undef P3D_TCG_PICK
+  if (d->f16) {      // fp16 inference: the output layer (fp32 store) and the hidden layers (16-bit activations)
+    fn = nullptr;
+    if (!seg && out == 0 && !res && cs == 0) fn = tc_gemm_kernel<0, false, 0, false, true>;
+    if (!seg && out == 2 && !res) fn = tc_gemm_kernel<2, false, 0, false, true>;
+    if (!seg && out == 2 && res) fn = tc_gemm_kernel<2, true, 0, false, true>;
+  }
 #define P3D_TCG_PICK_SEG(O, R) if (seg && out == O && res == R && cs == 0) fn = tc_gemm_kernel<O, R, 0, true>;
   P3D_TCG_PICK_SEG(0, false) P3D_TCG_PICK_SEG(5, false) P3D_TCG_PICK_SEG(5, true)
   P3D_TCG_PICK_SEG(0, true) P3D_TCG_PICK_SEG(1, false)       // bf16x3 training: data gradient + residual, split-K weight gradient
@@ -1207,7 +1221,8 @@ int launch(const GemmPlan& pl, cudaStream_t st) {
                       tc_gemm_kernel<2, false, 0>, tc_gemm_kernel<2, true, 0>,
                       tc_gemm_kernel<3, false, 0>, tc_gemm_kernel<4, false, 0>,
                       tc_gemm_kernel<0, false, 0, true>, tc_gemm_kernel<5, false, 0, true>, tc_gemm_kernel<5, true, 0, true>,
-                      tc_gemm_kernel<0, true, 0, true>, tc_gemm_kernel<1, false, 0, true>};
+                      tc_gemm_kernel<0, true, 0, true>, tc_gemm_kernel<1, false, 0, true>,
+                      tc_gemm_kernel<0, false, 0, false, true>, tc_gemm_kernel<2, false, 0, false, true>, tc_gemm_kernel<2, true, 0, false, true>};
     for (KernelFn f : all) P3D_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     attr.mark();
   }

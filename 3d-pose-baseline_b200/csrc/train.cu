@@ -521,8 +521,9 @@ void free_workspace(p3d_model* m) {
 }
 
 constexpr int kOutPad = 48;   // bf16 pitch of dy / W4 rows: 96 B keeps TMA's 16-byte pitch rule for out = 42 too
-// bf16 mode runs the step's GEMMs on the tensor cores (tc_gemm.cu); fp32 mode keeps the FFMA GEMMs
-static inline bool use_tc(const p3d_model* m) { return m->cfg.mode == P3D_MODE_BF16 && (m->L % 8) == 0; }
+// bf16 mode runs the step's GEMMs on the tensor cores (tc_gemm.cu); fp32 mode keeps the FFMA GEMMs.  fp16 mode chooses
+// inference arithmetic only: it trains on the bf16 route.
+static inline bool use_tc(const p3d_model* m) { return (m->cfg.mode == P3D_MODE_BF16 || m->cfg.mode == P3D_MODE_FP16) && (m->L % 8) == 0; }
 // P3D_TRAIN_MATMUL_BF16X3 (fp32 / bf16x3 models): the step's GEMMs as three split-bf16 products on the tensor cores;
 // widths the tcgen05 GEMM does not tile keep FFMA
 static inline bool use_x3(const p3d_model* m) {
@@ -1233,7 +1234,8 @@ int p3d_model_train_epoch(p3d_model* m, const float* X, const float* T, int64_t 
 int p3d_model_set_train_matmul(p3d_model* m, int kind) {
   P3D_REQUIRE(m, "set_train_matmul: null model");
   P3D_REQUIRE(kind == P3D_TRAIN_MATMUL_DEFAULT || kind == P3D_TRAIN_MATMUL_BF16X3, "set_train_matmul: unknown kind %d", kind);
-  P3D_REQUIRE(m->cfg.mode != P3D_MODE_BF16, "set_train_matmul: bf16-mode models train on their own tcgen05 bf16 route");
+  P3D_REQUIRE(m->cfg.mode != P3D_MODE_BF16 && m->cfg.mode != P3D_MODE_FP16,
+              "set_train_matmul: bf16- and fp16-mode models train on their own tcgen05 bf16 route");
   if (kind == m->train_matmul) return P3D_OK;
   P3D_CUDA(cudaSetDevice(m->cfg.device));
   train::drop_graphs(m->tw);        // captured with the other route's launches; the next step captures again

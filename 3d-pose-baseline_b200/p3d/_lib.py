@@ -39,7 +39,7 @@ class Camera(C.Structure):
                 ("k", C.c_double * 3), ("p", C.c_double * 2)]
 
 
-MODE_BF16, MODE_FP32, MODE_BF16X3 = 0, 1, 2
+MODE_BF16, MODE_FP32, MODE_BF16X3, MODE_FP16 = 0, 1, 2, 3
 TRAIN_MATMUL_DEFAULT, TRAIN_MATMUL_BF16X3 = 0, 1
 
 # name -> (restype, argtypes): every symbol include/p3d.h declares

@@ -5,8 +5,9 @@ are replaced by libp3d.so (hand-written sm_100a CUDA).  There is no TensorFlow, 
 
 Differences that are visible to a caller, all additive:
   * `session` is accepted and ignored (there is no tf.Session).
-  * keyword-only extras: `mode` ('bf16' tensor-core path, 'fp32', or 'bf16x3': fp32 accuracy on the tensor cores
-    for inference, trained like 'fp32'), `train_matmul` (None: the mode's own training route; 'bf16x3' with mode
+  * keyword-only extras: `mode` ('bf16' tensor-core path, 'fp32', 'bf16x3': fp32 accuracy on the tensor cores
+    for inference, trained like 'fp32', or 'fp16': bf16's paths on fp16 operands, <= 2e-3 row-wise error,
+    trained like 'bf16'), `train_matmul` (None: the mode's own training route; 'bf16x3' with mode
     'fp32' or 'bf16x3': the training step's MatMuls as three split-bf16 tensor-core products), `device`, `seed`, `dist`.
   * `step()` also accepts torch CUDA tensors (fp32) and then returns torch tensors without any host copy.
   * summaries are `Summary(tag, value)` tuples that serialize to the TF `Summary` protobuf on demand; with a
@@ -146,15 +147,15 @@ class LinearModel(object):
         self._lr0 = float(learning_rate)
         self._seed = int(seed) if seed is not None else int.from_bytes(os.urandom(4), "little")
         self._handle = None
-        modes = {"bf16": _lib.MODE_BF16, "fp32": _lib.MODE_FP32, "bf16x3": _lib.MODE_BF16X3}
+        modes = {"bf16": _lib.MODE_BF16, "fp32": _lib.MODE_FP32, "bf16x3": _lib.MODE_BF16X3, "fp16": _lib.MODE_FP16}
         if mode not in modes:
-            raise ValueError("mode must be 'bf16', 'fp32' or 'bf16x3'")
+            raise ValueError("mode must be 'bf16', 'fp32', 'bf16x3' or 'fp16'")
         # the arithmetic of the training step's MatMuls (p3d_model_set_train_matmul); with `dist`, every rank passes the
         # same value
         if train_matmul not in (None, "bf16x3"):
             raise ValueError("train_matmul must be None or 'bf16x3'")
-        if train_matmul is not None and mode == "bf16":
-            raise ValueError("train_matmul='bf16x3' needs mode 'fp32' or 'bf16x3' (bf16 models train on bf16 tensor cores)")
+        if train_matmul is not None and mode in ("bf16", "fp16"):
+            raise ValueError("train_matmul='bf16x3' needs mode 'fp32' or 'bf16x3' (bf16 and fp16 models train on bf16 tensor cores)")
         self.train_matmul = train_matmul
         # Summary writers for train and test runs (linear_model.py:80-82)
         if summaries_dir:

@@ -58,6 +58,13 @@ extern "C" {
  * MatMuls on the tensor cores too; the whole-chip bf16 kernels and the one-launch realtime frame are not used (frames
  * take the staged route). */
 #define P3D_MODE_BF16X3 2
+/* fp16 operands wherever P3D_MODE_BF16 uses bf16: every inference path of bf16 mode (the fused kernel, the per-layer
+ * GEMMs, the whole-chip kernels for 1-64 poses and the one-launch realtime frame), the same rounding points, fp32
+ * accumulation, the same tensor-core rate.  Contract: <= 2e-3 row-wise relative error against the fp64 oracle (bf16
+ * mode: ~6e-3), provided every folded weight, input and activation stays inside fp16's range (|v| <= 65504).
+ * linear_size % 8 != 0 runs the fp32 FFMA path.  Training steps and epochs are those of P3D_MODE_BF16 (the same
+ * kernels on the bf16 tensor cores); p3d_model_set_train_matmul returns P3D_ERR_ARG. */
+#define P3D_MODE_FP16 3
 
 const char* p3d_last_error(void);
 int p3d_version(void);
@@ -138,7 +145,8 @@ int p3d_model_train_epoch(p3d_model* m, const float* X, const float* T, int64_t 
                           float keep_prob, uint64_t seed, float* losses, float* lr_last_or_null, void* stream);
 
 /* Which arithmetic runs the MatMuls of a training step (steps and epochs), chosen per model:
- *   P3D_TRAIN_MATMUL_DEFAULT: the mode's own route - tcgen05 bf16 (P3D_MODE_BF16), FFMA (P3D_MODE_FP32, P3D_MODE_BF16X3).
+ *   P3D_TRAIN_MATMUL_DEFAULT: the mode's own route - tcgen05 bf16 (P3D_MODE_BF16, P3D_MODE_FP16), FFMA (P3D_MODE_FP32,
+ *                             P3D_MODE_BF16X3).
  *   P3D_TRAIN_MATMUL_BF16X3 : every MatMul of the step (forward, data and weight gradients) on tcgen05 as three split-bf16
  *                             products hi*hi + lo*hi + hi*lo with fp32 accumulation; activations, BatchNorm, dropout,
  *                             the loss and Adam stay fp32 as on the FFMA route.  fp32-class, not bit-equal to FFMA: at
@@ -146,7 +154,7 @@ int p3d_model_train_epoch(p3d_model* m, const float* X, const float* T, int64_t 
  *                             the split operands move pre-activations by ~1e-5 relative, which flips the ReLU of a few
  *                             dozen units near zero (gradients within ~3e-3 relative L2) - hence opt-in.  Widths with
  *                             linear_size % 8 != 0 keep the FFMA route.
- * Valid on P3D_MODE_FP32 and P3D_MODE_BF16X3 models; a P3D_MODE_BF16 model returns P3D_ERR_ARG.  A host call without a
+ * Valid on P3D_MODE_FP32 and P3D_MODE_BF16X3 models; a P3D_MODE_BF16 or P3D_MODE_FP16 model returns P3D_ERR_ARG.  A host call without a
  * stream: it must not be made while a training step of the model is in flight.  Switching drops the model's captured
  * training-step graphs (the next step captures again).  Data-parallel ranks must all set the same kind. */
 #define P3D_TRAIN_MATMUL_DEFAULT 0
@@ -198,7 +206,7 @@ typedef struct p3d_realtime p3d_realtime;
 int p3d_realtime_create(p3d_model* m, const double* mean2d_host, const double* std2d_host, const int32_t* use2d_host,
                         const double* mean3d_host, const double* std3d_host, const int32_t* use3d_host, p3d_realtime** out);
 void p3d_realtime_destroy(p3d_realtime* r);
-/* One frame, HOST buffers, synchronous.  With linear_size 1024 in bf16 mode this is a single kernel launch that reads
+/* One frame, HOST buffers, synchronous.  With linear_size 1024 in bf16 or fp16 mode this is a single kernel launch that reads
  * the keypoints from and writes the results to mapped pinned memory (no cudaMemcpy, no stream synchronise).
  * enc_in_host[32] and y_host[out] (the normalised input / prediction) are optional. */
 int p3d_realtime_step_host(p3d_realtime* r, const double* xy36_host, float* enc_in_host_or_null, float* y_host_or_null,
