@@ -124,7 +124,8 @@ struct TrainWorkspace {
   double* red = nullptr;    // [nhidden][2][L] backward sums (dgamma, dbeta) + misc scalars
   unsigned* gcount = nullptr;   // [2 nhidden][2] arrival counter + completion flag of the grid-synchronised fused epilogues
   float* scal = nullptr;    // small device scalars: loss, lr, clip dots...
-  // bf16 operands of the tensor-core path (P3D_MODE_BF16)
+  // bf16 operands of the tensor-core path (P3D_MODE_BF16); fp16 bits on the P3D_TRAIN_MATMUL_FP16 route (dzb / dyb then
+  // hold the gradient scaled by a power of two)
   __nv_bfloat16* xb = nullptr;    // [B][32]
   __nv_bfloat16* hb = nullptr;    // [nhidden][B][L]
   __nv_bfloat16* dzb = nullptr;   // [B][L]
@@ -266,6 +267,8 @@ struct FusedTrain {
   double* xsum = nullptr;                 // optional scalar summed over the ranks on the same exchange (the step's loss sum)
   float pg_scale = 1.f;                   // 1 / world: gradients every rank computes in full (dgamma, dbeta, bias) are
                                           // pre-divided so that the flat gradient all-reduce (a sum) restores them once
+  float gscale = 1.f;                     // mode 4 with fp16 operands: dz is stored as fp16(gscale * dz), a power of two
+                                          // (fills the struct's tail padding: no other member moves)
 };
 // tcgen05 GEMM (tc_gemm.cu): C[M,N] (+)= alpha * A B^T-form product of bf16 operands, fp32 result.
 struct GemmArgs {
@@ -284,7 +287,8 @@ struct GemmArgs {
   void* out_bf16 = nullptr; int ld_out_bf16 = 0;
   const void* res_bf16 = nullptr; int ld_res_bf16 = 0;
   int relu = 0;
-  // fp16 operands (P3D_MODE_FP16 inference): A, B, out_bf16 and res_bf16 hold fp16; plain fp32 store or 16-bit output only
+  // fp16 operands (P3D_MODE_FP16 inference, P3D_TRAIN_MATMUL_FP16 training): A, B, out_bf16, res_bf16 and the fused
+  // epilogues' 16-bit outputs hold fp16; not with the segment schedule
   int f16 = 0;
   // programmatic dependent launch: the kernel may start before its stream predecessor has finished; B (weights)
   // must not depend on that predecessor - its first tiles are fetched ahead of the dependency wait

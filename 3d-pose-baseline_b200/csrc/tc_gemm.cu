@@ -293,13 +293,14 @@ __device__ __forceinline__ void totals_wait(const Params& p, int n0, int et, dou
 // square are accumulated (BatchNorm statistics of a forward layer on the unfused path).  SEG: segment schedule of the
 // split-precision (bf16x3) GEMMs, inference and training - the K loop runs three passes, reading the (A, B) segments
 // (hi, hi), (lo, hi), (hi, lo) into one accumulator; either operand K-major or MN-major, K split or not.  F16: fp16
-// operands (P3D_MODE_FP16 inference: the fp32 store and the 16-bit activation store, OUT 0 / 2), where OUT = 2 stores
-// and reads fp16 activations.
+// operands - P3D_MODE_FP16 inference (OUT 0 / 2, where OUT = 2 stores and reads fp16 activations) and the
+// P3D_TRAIN_MATMUL_FP16 training route (OUT 0 / 1 / 3 / 4, CS), where OUT = 3 stores fp16 h and OUT = 4 stores dz as
+// fp16(ft.gscale * dz).  The 2^-k that takes a scaled gradient operand back out is the caller's alpha.
 template <int OUT, bool RES, int CS, bool SEG = false, bool F16 = false>
 __global__ void __launch_bounds__((OUT == 3 || OUT == 4) ? FUSED_NTHREADS : NTHREADS, 1)
 tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_b, const Params p) {
   static_assert(CS == 0 || OUT < 2, "column sums are taken of the fp32 stores only");
-  static_assert(!F16 || ((OUT == 0 || OUT == 2) && !SEG && CS == 0), "fp16 operands: the inference epilogues only");
+  static_assert(!F16 || (OUT != 5 && !SEG), "fp16 operands: not with the segment schedule");
   using O16 = Op16<F16>;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -714,9 +715,9 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
             }
             r[0] += hr[i].x; r[1] += hr[i].y; r[2] += hr[i].z; r[3] += hr[i].w;
             if (p.ft.h) *reinterpret_cast<float4*>(p.ft.h + off) = make_float4(r[0], r[1], r[2], r[3]);
-            __nv_bfloat162 lo = __floats2bfloat162_rn(r[0], r[1]), hi = __floats2bfloat162_rn(r[2], r[3]);
+            typename O16::T2 lo = O16::pack(r[0], r[1]), hi = O16::pack(r[2], r[3]);
             uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
-            *reinterpret_cast<uint2*>(static_cast<__nv_bfloat16*>(p.ft.hb) + off) = pk;
+            *reinterpret_cast<uint2*>(static_cast<typename O16::T*>(p.ft.hb) + off) = pk;
           }
         }
       } else {
@@ -791,9 +792,13 @@ tc_gemm_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__
             float d[4];
 #pragma unroll
             for (int j = 0; j < 4; ++j) d[j] = has_bn ? gr[j] * (o[i][j] - P[j] - xh[i][j] * Q[j]) : o[i][j];
-            __nv_bfloat162 lo = __floats2bfloat162_rn(d[0], d[1]), hi = __floats2bfloat162_rn(d[2], d[3]);
+            if constexpr (F16) {        // the gradient operand is scaled by 2^k into fp16's normal range (exact)
+#pragma unroll
+              for (int j = 0; j < 4; ++j) d[j] *= p.ft.gscale;
+            }
+            typename O16::T2 lo = O16::pack(d[0], d[1]), hi = O16::pack(d[2], d[3]);
             uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
-            *reinterpret_cast<uint2*>(static_cast<__nv_bfloat16*>(p.ft.dzb) + static_cast<size_t>(m) * p.N + n) = pk;
+            *reinterpret_cast<uint2*>(static_cast<typename O16::T*>(p.ft.dzb) + static_cast<size_t>(m) * p.N + n) = pk;
           }
         }
       }
@@ -1162,8 +1167,8 @@ int plan(const GemmArgs& g, GemmPlan* out) {
   d->fused_mode = g.fused_mode;
   d->coop = 0;
   d->f16 = g.f16;
-  P3D_REQUIRE(!g.f16 || (!seg && !g.fused_mode && !g.colsum && !g.split_k && !g.accumulate && !(g.C && g.out_bf16)),
-              "tc_gemm: fp16 operands take the inference epilogues only (fp32 store or 16-bit activations)");
+  P3D_REQUIRE(!g.f16 || (!seg && !(g.C && g.out_bf16) && !(g.out_bf16 && (g.colsum || g.split_k || g.accumulate))),
+              "tc_gemm: fp16 operands take the fp32, reduction, 16-bit activation and fused training epilogues");
   if (g.fused_mode) {
     P3D_REQUIRE(g.fused_mode == 3 || g.fused_mode == 4, "tc_gemm: unknown fused mode %d", g.fused_mode);
     P3D_REQUIRE(splits == 1 && (g.N % 32) == 0 && g.ldc == g.N && !g.out_bf16 && !g.colsum && !g.pdl,
@@ -1206,13 +1211,17 @@ int launch(const GemmPlan& pl, cudaStream_t st) {
     if (!seg && out == 0 && !res && cs == 0) fn = tc_gemm_kernel<0, false, 0, false, true>;
     if (!seg && out == 2 && !res) fn = tc_gemm_kernel<2, false, 0, false, true>;
     if (!seg && out == 2 && res) fn = tc_gemm_kernel<2, true, 0, false, true>;
+    // fp16 training route: forward with BN column sums, data gradient + residual, split-K weight gradient
+    if (!seg && out == 0 && !res && cs == 1) fn = tc_gemm_kernel<0, false, 1, false, true>;
+    if (!seg && out == 0 && res && cs == 0) fn = tc_gemm_kernel<0, true, 0, false, true>;
+    if (!seg && out == 1 && !res) fn = tc_gemm_kernel<1, false, 0, false, true>;
   }
 #define P3D_TCG_PICK_SEG(O, R) if (seg && out == O && res == R && cs == 0) fn = tc_gemm_kernel<O, R, 0, true>;
   P3D_TCG_PICK_SEG(0, false) P3D_TCG_PICK_SEG(5, false) P3D_TCG_PICK_SEG(5, true)
   P3D_TCG_PICK_SEG(0, true) P3D_TCG_PICK_SEG(1, false)       // bf16x3 training: data gradient + residual, split-K weight gradient
 #undef P3D_TCG_PICK_SEG
-  if (d->fused_mode == 3) fn = tc_gemm_kernel<3, false, 0>;
-  if (d->fused_mode == 4) fn = tc_gemm_kernel<4, false, 0>;
+  if (d->fused_mode == 3) fn = d->f16 ? tc_gemm_kernel<3, false, 0, false, true> : tc_gemm_kernel<3, false, 0>;
+  if (d->fused_mode == 4) fn = d->f16 ? tc_gemm_kernel<4, false, 0, false, true> : tc_gemm_kernel<4, false, 0>;
   P3D_REQUIRE(fn != nullptr, "tc_gemm: unsupported epilogue combination (out %d res %d colsum %d)", out, (int)res, (int)cs);
   static PerDeviceOnce attr;
   if (attr.needed()) {
@@ -1222,7 +1231,9 @@ int launch(const GemmPlan& pl, cudaStream_t st) {
                       tc_gemm_kernel<3, false, 0>, tc_gemm_kernel<4, false, 0>,
                       tc_gemm_kernel<0, false, 0, true>, tc_gemm_kernel<5, false, 0, true>, tc_gemm_kernel<5, true, 0, true>,
                       tc_gemm_kernel<0, true, 0, true>, tc_gemm_kernel<1, false, 0, true>,
-                      tc_gemm_kernel<0, false, 0, false, true>, tc_gemm_kernel<2, false, 0, false, true>, tc_gemm_kernel<2, true, 0, false, true>};
+                      tc_gemm_kernel<0, false, 0, false, true>, tc_gemm_kernel<2, false, 0, false, true>, tc_gemm_kernel<2, true, 0, false, true>,
+                      tc_gemm_kernel<0, false, 1, false, true>, tc_gemm_kernel<0, true, 0, false, true>, tc_gemm_kernel<1, false, 0, false, true>,
+                      tc_gemm_kernel<3, false, 0, false, true>, tc_gemm_kernel<4, false, 0, false, true>};
     for (KernelFn f : all) P3D_CUDA(cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES));
     attr.mark();
   }

@@ -9,6 +9,8 @@
 // the row index), the forward GEMM's epilogue also produces the BatchNorm column sums.  P3D_MODE_FP32: FFMA GEMMs.
 // P3D_TRAIN_MATMUL_BF16X3 (fp32 / bf16x3 models, opt-in): the FFMA route's kernels, with every GEMM replaced by three
 // split-bf16 tcgen05 products (tc_gemm.cu segment schedule) on split-pair copies of x, h, dz, dy and W.
+// P3D_TRAIN_MATMUL_FP16 (bf16 / fp16 models, opt-in): the bf16 route with fp16 in the same 16-bit operand buffers; the
+// gradient operands dy / dz are stored scaled by 2^k (grad_exp) and their GEMMs take 2^-k into alpha.
 // Data parallel (one process per GPU): rows are sharded, BN statistics and their backward sums are
 // all-reduced (SyncBN - required for parity with the single-device reference), and the flat gradient
 // buffer is all-reduced once with NCCL before the (replicated) Adam update.
@@ -98,8 +100,11 @@ __device__ __forceinline__ void store_split4(__nv_bfloat16* p, int lo, const flo
 
 // W -> bf16 operand copy (row pitch ldwb >= N) and ||W||_F^2, every layer in ONE launch; ws: the split pair of W instead
 // (bf16x3 training route, rows [hi | lo] of pitch 2 seg at off_ws).  The norm is summed in the same order either way.
-__global__ void wprep_kernel(const float* __restrict__ theta, const LayerTabEntry* __restrict__ tab, __nv_bfloat16* __restrict__ wb,
+// F16: the operand copy is fp16 (P3D_TRAIN_MATMUL_FP16).
+template <bool F16>
+__global__ void wprep_kernel(const float* __restrict__ theta, const LayerTabEntry* __restrict__ tab, typename Op16<F16>::T* __restrict__ wb,
                              double* __restrict__ norm2, __nv_bfloat16* __restrict__ ws) {
+  using O = Op16<F16>;
   const LayerTabEntry e = tab[blockIdx.y];
   const long long n = static_cast<long long>(e.K) * e.N;
   const float* w = theta + e.off_w;
@@ -110,7 +115,7 @@ __global__ void wprep_kernel(const float* __restrict__ theta, const LayerTabEntr
       const float4 v = *reinterpret_cast<const float4*>(w + i);
       acc += static_cast<double>(v.x) * v.x + static_cast<double>(v.y) * v.y + static_cast<double>(v.z) * v.z + static_cast<double>(v.w) * v.w;
       if (wb) {
-        __nv_bfloat162 lo = __floats2bfloat162_rn(v.x, v.y), hi = __floats2bfloat162_rn(v.z, v.w);
+        typename O::T2 lo = O::pack(v.x, v.y), hi = O::pack(v.z, v.w);
         uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
         *reinterpret_cast<uint2*>(wb + e.off_wb + i) = pk;
       }
@@ -124,7 +129,7 @@ __global__ void wprep_kernel(const float* __restrict__ theta, const LayerTabEntr
     for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < n; i += static_cast<long long>(gridDim.x) * blockDim.x) {
       const float v = w[i];
       acc += static_cast<double>(v) * v;
-      if (wb) { const long long r = i / e.N; wb[e.off_wb + r * e.ldwb + (i - r * e.N)] = __float2bfloat16_rn(v); }
+      if (wb) { const long long r = i / e.N; wb[e.off_wb + r * e.ldwb + (i - r * e.N)] = O::from(v); }
       if (ws) {
         const long long r = i / e.N;
         __nv_bfloat16* row = ws + e.off_ws + r * 2 * e.seg + (i - r * e.N);
@@ -217,8 +222,10 @@ struct ActArgs {
   __nv_bfloat16* hs; int seg;     // bf16x3 training route: split pair of h, rows [hi | lo] of pitch 2 seg (else null)
 };
 
-// h = dropout(relu(bn(z))) (+res); one thread per 4 columns; also materialises the keep-mask
+// h = dropout(relu(bn(z))) (+res); one thread per 4 columns; also materialises the keep-mask.  F16: hb holds fp16.
+template <bool F16>
 __global__ void fwd_act_kernel(const ActArgs a) {
+  using O = Op16<F16>;
   const int L4 = a.L / 4;
   const long long total = a.B * L4;
   const float keep = a.sc->keep, inv_keep = a.sc->inv_keep;
@@ -255,30 +262,33 @@ __global__ void fwd_act_kernel(const ActArgs a) {
     }
     if (a.h) *reinterpret_cast<float4*>(a.h + r * a.L + c) = make_float4(v[0], v[1], v[2], v[3]);
     if (a.hb) {      // operand of the next layer's tcgen05 GEMMs (forward and weight gradient)
-      __nv_bfloat162 lo = __floats2bfloat162_rn(v[0], v[1]), hi = __floats2bfloat162_rn(v[2], v[3]);
+      typename O::T2 lo = O::pack(v[0], v[1]), hi = O::pack(v[2], v[3]);
       uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
-      *reinterpret_cast<uint2*>(a.hb + r * a.L + c) = pk;
+      *reinterpret_cast<uint2*>(reinterpret_cast<typename O::T*>(a.hb) + r * a.L + c) = pk;
     }
     if (a.hs) store_split4(a.hs + r * 2 * a.seg + c, a.seg, v);     // operand of the next layer's bf16x3 GEMMs
   }
 }
 
-// fp32 -> bf16 with a (possibly wider) destination pitch; pad columns are left untouched (zero)
-__global__ void to_bf16_kernel(const float* __restrict__ src, __nv_bfloat16* __restrict__ dst, long long rows, int cols, int ld_dst) {
+// fp32 -> bf16 (F16: fp16) with a (possibly wider) destination pitch; pad columns are left untouched (zero)
+template <bool F16>
+__global__ void to_bf16_kernel(const float* __restrict__ src, typename Op16<F16>::T* __restrict__ dst, long long rows, int cols, int ld_dst) {
   const long long total = rows * cols;
   for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
        i += static_cast<long long>(gridDim.x) * blockDim.x) {
     const long long r = i / cols;
     const int c = static_cast<int>(i - r * cols);
-    dst[r * ld_dst + c] = __float2bfloat16_rn(src[i]);
+    dst[r * ld_dst + c] = Op16<F16>::from(src[i]);
   }
 }
 
 // dy = 2 (y - t) / (Bg*out), loss accumulator += sum (y-t)^2
-// dyb: bf16 operand copy of dy with row pitch ld_b; lo_b > 0: the split pair instead, lo half at column lo_b + c
+// dyb: bf16 operand copy of dy with row pitch ld_b; lo_b > 0: the split pair instead, lo half at column lo_b + c.
+// F16: dyb = fp16(gs * dy), gs the power of two that lifts the gradient out of fp16's subnormals (no split pair).
+template <bool F16>
 __global__ void loss_dy_kernel(const float* __restrict__ y, const float* __restrict__ t, size_t n, float scale,
-                               float* __restrict__ dy, double* __restrict__ acc, __nv_bfloat16* __restrict__ dyb, int out, int ld_b,
-                               int lo_b) {
+                               float* __restrict__ dy, double* __restrict__ acc, typename Op16<F16>::T* __restrict__ dyb, int out, int ld_b,
+                               int lo_b, float gs) {
   double s = 0;
   for (size_t i = blockIdx.x * static_cast<size_t>(blockDim.x) + threadIdx.x; i < n; i += static_cast<size_t>(gridDim.x) * blockDim.x) {
     const float d = y[i] - t[i];
@@ -286,9 +296,13 @@ __global__ void loss_dy_kernel(const float* __restrict__ y, const float* __restr
     if (dyb) {
       const size_t r = i / out;
       const float v = scale * d;
-      const __nv_bfloat16 h = __float2bfloat16_rn(v);
-      dyb[r * ld_b + (i - r * out)] = h;
-      if (lo_b) dyb[r * ld_b + lo_b + (i - r * out)] = __float2bfloat16_rn(v - __bfloat162float(h));
+      if constexpr (F16) {
+        dyb[r * ld_b + (i - r * out)] = Op16<true>::from(v * gs);
+      } else {
+        const __nv_bfloat16 h = __float2bfloat16_rn(v);
+        dyb[r * ld_b + (i - r * out)] = h;
+        if (lo_b) dyb[r * ld_b + lo_b + (i - r * out)] = __float2bfloat16_rn(v - __bfloat162float(h));
+      }
     }
     s += static_cast<double>(d) * d;
   }
@@ -311,11 +325,15 @@ struct BwdArgs {
   const float* dh; const float* z; const float* mean; const float* rstd; const float* gamma; const float* beta;
   const uint8_t* mask; float* dz; __nv_bfloat16* dzb; double* sums; const StepScalars* sc; long long B; int L; int has_bn; int dropout;
   __nv_bfloat16* dzs; int seg;    // bf16x3 training route, layers without BN: split pair of dz (else null)
+  float gs;                       // F16: dzb = fp16(gs * dz), a power of two
 };
 
 // pass A: da = dh * dropout * relu'(a); column sums of da and da*xhat (for BN backward / dgamma, dbeta).
 // Block = 32 x 8 threads, every thread owns 4 consecutive columns (float4) of RCH4 / 8 rows.
+// F16: dzb holds fp16(gs * dz).
+template <bool F16>
 __global__ void __launch_bounds__(256) bwd_act_kernel(const BwdArgs a) {
+  using O = Op16<F16>;
   __shared__ double s1[8][33][4], s2[8][33][4];
   const int c = (blockIdx.x * 32 + threadIdx.x) * 4;
   const long long r0 = static_cast<long long>(blockIdx.y) * RCH4;
@@ -351,9 +369,11 @@ __global__ void __launch_bounds__(256) bwd_act_kernel(const BwdArgs a) {
       }
       if (a.dz) *reinterpret_cast<float4*>(a.dz + o) = make_float4(da[0], da[1], da[2], da[3]);
       if (a.dzb) {       // final dz only when the layer has no BN
-        __nv_bfloat162 lo = __floats2bfloat162_rn(da[0], da[1]), hi = __floats2bfloat162_rn(da[2], da[3]);
+        typename O::T2 lo, hi;
+        if constexpr (F16) { lo = O::pack(da[0] * a.gs, da[1] * a.gs); hi = O::pack(da[2] * a.gs, da[3] * a.gs); }
+        else { lo = O::pack(da[0], da[1]); hi = O::pack(da[2], da[3]); }
         uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
-        *reinterpret_cast<uint2*>(a.dzb + o) = pk;
+        *reinterpret_cast<uint2*>(reinterpret_cast<typename O::T*>(a.dzb) + o) = pk;
       }
       if (a.dzs) store_split4(a.dzs + static_cast<size_t>(r) * 2 * a.seg + c, a.seg, da);
     }
@@ -374,13 +394,16 @@ __global__ void __launch_bounds__(256) bwd_act_kernel(const BwdArgs a) {
 
 // pass B (BN layers): dz = gamma * rstd * (da - mean(da) - xhat * mean(da*xhat)), means over the GLOBAL batch;
 // also writes dgamma / dbeta (pre-divided by the world size: the flat gradient all-reduce restores them).
+template <bool F16>
 __global__ void bwd_bn_kernel(float* __restrict__ dz, const float* __restrict__ z, const float* __restrict__ mean,
                               const float* __restrict__ rstd, const float* __restrict__ gamma,
-                              const double* __restrict__ sums, float invB, long long B, int L, __nv_bfloat16* __restrict__ dzb,
+                              const double* __restrict__ sums, float invB, long long B, int L, typename Op16<F16>::T* __restrict__ dzb,
                               int write_f32, double pg_scale, float* __restrict__ ggamma, float* __restrict__ gbeta,
                               const float* __restrict__ dh, const uint8_t* __restrict__ mask, const float* __restrict__ beta,
-                              const StepScalars* __restrict__ sc, __nv_bfloat16* __restrict__ dzs, int seg) {
+                              const StepScalars* __restrict__ sc, __nv_bfloat16* __restrict__ dzs, int seg, float gs) {
   // dzs: the split pair of dz (bf16x3 training route), rows [hi | lo] of pitch 2 seg
+  // F16: dzb holds fp16(gs * dz)
+  using O = Op16<F16>;
   // dh != null: da is recomputed from (dh, z, mask) instead of being read back - pass A then never stores it
   const int L4 = L / 4;
   const long long total = B * L4;
@@ -421,7 +444,9 @@ __global__ void bwd_bn_kernel(float* __restrict__ dz, const float* __restrict__ 
     }
     if (write_f32) *reinterpret_cast<float4*>(dz + o) = make_float4(v[0], v[1], v[2], v[3]);
     if (dzb) {
-      __nv_bfloat162 lo = __floats2bfloat162_rn(v[0], v[1]), hi = __floats2bfloat162_rn(v[2], v[3]);
+      typename O::T2 lo, hi;
+      if constexpr (F16) { lo = O::pack(v[0] * gs, v[1] * gs); hi = O::pack(v[2] * gs, v[3] * gs); }
+      else { lo = O::pack(v[0], v[1]); hi = O::pack(v[2], v[3]); }
       uint2 pk; pk.x = *reinterpret_cast<uint32_t*>(&lo); pk.y = *reinterpret_cast<uint32_t*>(&hi);
       *reinterpret_cast<uint2*>(dzb + o) = pk;
     }
@@ -522,7 +547,7 @@ void free_workspace(p3d_model* m) {
 
 constexpr int kOutPad = 48;   // bf16 pitch of dy / W4 rows: 96 B keeps TMA's 16-byte pitch rule for out = 42 too
 // bf16 mode runs the step's GEMMs on the tensor cores (tc_gemm.cu); fp32 mode keeps the FFMA GEMMs.  fp16 mode chooses
-// inference arithmetic only: it trains on the bf16 route.
+// inference arithmetic only: it trains on the bf16 route (on fp16 operands with P3D_TRAIN_MATMUL_FP16, use_f16).
 static inline bool use_tc(const p3d_model* m) { return (m->cfg.mode == P3D_MODE_BF16 || m->cfg.mode == P3D_MODE_FP16) && (m->L % 8) == 0; }
 // P3D_TRAIN_MATMUL_BF16X3 (fp32 / bf16x3 models): the step's GEMMs as three split-bf16 products on the tensor cores;
 // widths the tcgen05 GEMM does not tile keep FFMA
@@ -530,6 +555,15 @@ static inline bool use_x3(const p3d_model* m) {
   return m->train_matmul == P3D_TRAIN_MATMUL_BF16X3 && m->cfg.mode != P3D_MODE_BF16 && (m->L % 8) == 0;
 }
 static inline int seg_of(int n) { return (n + 63) / 64 * 64; }   // lo-segment column of a split pair of width n
+// P3D_TRAIN_MATMUL_FP16 (bf16 / fp16 models): the bf16 route's kernels with fp16 in every 16-bit operand buffer
+static inline bool use_f16(const p3d_model* m) { return use_tc(m) && m->train_matmul == P3D_TRAIN_MATMUL_FP16; }
+// Scale of the fp16 route's gradient operands: 2^k with k = floor(log2(Bg * out)), so that 2^k dy = 2^k 2 (y - t) / (Bg out)
+// lies in (y - t, 2 (y - t)] - out of fp16's subnormals at any batch.  Every gradient operand (dy, dz) is linear in dy:
+// they are stored as fp16(2^k g) and the GEMMs that read them take 2^-k into their fp32 alpha (both exact).
+static inline int grad_exp(int64_t Bg, int out) {
+  const unsigned long long n = static_cast<unsigned long long>(Bg) * static_cast<unsigned long long>(out);
+  return 63 - __builtin_clzll(n);
+}
 
 static void drop_graphs(TrainWorkspace& w) {
   for (auto& ge : w.graphs) if (ge.exec) cudaGraphExecDestroy(static_cast<cudaGraphExec_t>(ge.exec));   // they hold the old pointers
@@ -658,6 +692,9 @@ static int fwd_bwd_fused(p3d_model* m, const float* t, int64_t B, bool dropout, 
   const float invB = 1.f / static_cast<float>(Bg);
   const int Bi = static_cast<int>(B);
   const bool dp = m->world > 1;
+  const bool f16 = use_f16(m);
+  const int gk = f16 ? grad_exp(Bg, out) : 0;
+  const float gs = std::ldexp(1.f, gk), ginv = std::ldexp(1.f, -gk);   // 1 and 1 on the bf16 route
   // grid-synchronised form: per layer and direction [2][L] doubles of column sums (w.stats forward, w.red backward,
   // both zeroed at the top of the step) and an arrival counter + completion flag
   auto grid_operands = [&](tcg::FusedTrain& f, double* sums, int which) {
@@ -673,7 +710,7 @@ static int fwd_bwd_fused(p3d_model* m, const float* t, int64_t B, bool dropout, 
     g.A = li == 0 ? w.xb : w.hb + (li - 1) * bl; g.lda = li == 0 ? kIn : L;
     g.B = w.wb + ly.off_w; g.ldb = L; g.b_mn = 1;
     g.C = w.z + li * bl; g.ldc = L; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + li : nullptr;
-    g.fused_mode = 3;
+    g.fused_mode = 3; g.f16 = f16;
     tcg::FusedTrain& f = g.fused;
     f.sc = sc; f.has_bn = ly.has_bn; f.dropout = dropout; f.layer = li; f.invB = invB;
     if (ly.has_bn) {
@@ -694,11 +731,15 @@ static int fwd_bwd_fused(p3d_model* m, const float* t, int64_t B, bool dropout, 
     g.M = Bi; g.N = out; g.K = L;
     g.A = w.hb + (nh - 1) * bl; g.lda = L;
     g.B = w.wb + ly.off_w; g.ldb = kOutPad; g.b_mn = 1;
-    g.C = y; g.ldc = out; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + nh : nullptr;
+    g.C = y; g.ldc = out; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + nh : nullptr; g.f16 = f16;
     P3D_TRY(tcg::gemm(g, st));
   }
   const size_t ny = static_cast<size_t>(B) * out;
-  loss_dy_kernel<<<egrid(static_cast<long long>(ny)), 256, 0, st>>>(y, t, ny, 2.0f * invB / out, w.dy, lossacc, w.dyb, out, kOutPad, 0);
+  if (f16)
+    loss_dy_kernel<true><<<egrid(static_cast<long long>(ny)), 256, 0, st>>>(y, t, ny, 2.0f * invB / out, w.dy, lossacc,
+                                                                            reinterpret_cast<__half*>(w.dyb), out, kOutPad, 0, gs);
+  else
+    loss_dy_kernel<false><<<egrid(static_cast<long long>(ny)), 256, 0, st>>>(y, t, ny, 2.0f * invB / out, w.dy, lossacc, w.dyb, out, kOutPad, 0, 1.f);
   P3D_LAUNCH_CHECK();
   // ---------------------------------------------------------------- backward
   // (data parallel: the loss sum rides on the first backward exchange, see fused_dgrad)
@@ -717,11 +758,11 @@ static int fwd_bwd_fused(p3d_model* m, const float* t, int64_t B, bool dropout, 
     g.M = Bi; g.N = L; g.K = K;
     g.A = A; g.lda = lda;
     g.B = w.wb + lw.off_w; g.ldb = ldb;
-    g.C = w.dz; g.ldc = L; g.alpha_dev = clip ? scale + li : nullptr;
+    g.C = w.dz; g.ldc = L; g.alpha_dev = clip ? scale + li : nullptr; g.alpha = ginv;
     if (add) { g.res = DH[keep]; g.ldres = L; }
-    g.fused_mode = 4;
+    g.fused_mode = 4; g.f16 = f16;
     tcg::FusedTrain& f = g.fused;
-    f.sc = sc; f.has_bn = lt.has_bn; f.dropout = dropout; f.layer = tl; f.invB = invB;
+    f.sc = sc; f.has_bn = lt.has_bn; f.dropout = dropout; f.layer = tl; f.invB = invB; f.gscale = gs;
     f.z = w.z + tl * bl; f.mask = w.maskbuf + tl * bl; f.dzb = dz_out;
     f.dh_out = save ? DH[slot] : nullptr;
     if (lt.has_bn) {
@@ -759,7 +800,7 @@ static int fwd_bwd_fused(p3d_model* m, const float* t, int64_t B, bool dropout, 
     gw.M = L; gw.N = out; gw.K = Bi;
     gw.A = w.hb + (nh - 1) * bl; gw.lda = L; gw.a_mn = 1;
     gw.B = w.dyb; gw.ldb = kOutPad; gw.b_mn = 1;
-    gw.C = m->grad + ly.off_w; gw.ldc = out; gw.split_k = 1;
+    gw.C = m->grad + ly.off_w; gw.ldc = out; gw.split_k = 1; gw.alpha = ginv; gw.f16 = f16;
     cudaEvent_t e4;
     P3D_TRY(fork_wgrad(gw, &e4));
     colsum_kernel<<<colgrid(out, B), dim3(32, 8), 0, st>>>(w.dy, B, out, m->grad + ly.off_b);
@@ -772,7 +813,7 @@ static int fwd_bwd_fused(p3d_model* m, const float* t, int64_t B, bool dropout, 
     gw.M = ly.K; gw.N = L; gw.K = Bi;
     gw.A = li == 0 ? w.xb : w.hb + (li - 1) * bl; gw.lda = li == 0 ? kIn : L; gw.a_mn = 1;
     gw.B = dzb[db]; gw.ldb = L; gw.b_mn = 1;
-    gw.C = m->grad + ly.off_w; gw.ldc = L; gw.split_k = 1;
+    gw.C = m->grad + ly.off_w; gw.ldc = L; gw.split_k = 1; gw.alpha = ginv; gw.f16 = f16;
     P3D_TRY(fork_wgrad(gw, &wg_done[db]));
     if (li > 0) {
       if (wg_done[1 - db]) P3D_CUDA(cudaStreamWaitEvent(st, wg_done[1 - db], 0));   // the buffer about to be overwritten is free
@@ -804,6 +845,9 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
   const bool tc = use_tc(m);
   const bool x3 = use_x3(m);        // bf16x3 split products on tcgen05 (unfused route, FFMA's elementwise kernels)
   const bool lowp = tc || x3;       // the GEMMs read the bf16 operand buffers, not the fp32 activations
+  const bool f16 = use_f16(m);      // tc with fp16 operands; gradient operands scaled by gs, their GEMMs' alpha takes ginv
+  const int gk = f16 ? grad_exp(Bg, out) : 0;
+  const float gs = std::ldexp(1.f, gk), ginv = std::ldexp(1.f, -gk);
   const int seg = seg_of(L), ld = 2 * seg;
   const size_t bls = static_cast<size_t>(B) * ld;   // one layer of split activations
   using tcg::GemmArgs;
@@ -820,7 +864,8 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
   if (clip || lowp) {
     // one launch over all layers: ||W||_F^2 (clip_by_norm) and, on the tensor-core paths, this step's bf16 copy (or
     // split pair) of the UNCLIPPED W in its natural [K][N] layout (W4 rows padded); the clip scale is the GEMMs' alpha
-    wprep_kernel<<<dim3(148, nlay), 256, 0, st>>>(m->theta, tab, tc ? w.wb : nullptr, clip ? m->norm2 : nullptr, x3 ? w.ws : nullptr);
+    if (f16) wprep_kernel<true><<<dim3(148, nlay), 256, 0, st>>>(m->theta, tab, reinterpret_cast<__half*>(w.wb), clip ? m->norm2 : nullptr, nullptr);
+    else wprep_kernel<false><<<dim3(148, nlay), 256, 0, st>>>(m->theta, tab, tc ? w.wb : nullptr, clip ? m->norm2 : nullptr, x3 ? w.ws : nullptr);
     P3D_LAUNCH_CHECK();
   }
   if (clip) {
@@ -828,7 +873,8 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
     P3D_LAUNCH_CHECK();
   }
   if (tc) {
-    to_bf16_kernel<<<egrid(static_cast<long long>(B) * kIn / 4 + 1), 256, 0, st>>>(x, w.xb, B, kIn, kIn);
+    if (f16) to_bf16_kernel<true><<<egrid(static_cast<long long>(B) * kIn / 4 + 1), 256, 0, st>>>(x, reinterpret_cast<__half*>(w.xb), B, kIn, kIn);
+    else to_bf16_kernel<false><<<egrid(static_cast<long long>(B) * kIn / 4 + 1), 256, 0, st>>>(x, w.xb, B, kIn, kIn);
     P3D_LAUNCH_CHECK();
   }
   if (x3) P3D_TRY(prep::pack_input_split(x, w.xs, B, st));      // [B][128]: hi columns 0..31, lo 64..95
@@ -853,7 +899,7 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       g.A = li == 0 ? w.xb : w.hb + (li - 1) * bl; g.lda = lda;
       g.B = w.wb + ly.off_w; g.ldb = L; g.b_mn = 1;
       g.C = z; g.ldc = L; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + li : nullptr;
-      g.colsum = ly.has_bn ? stats : nullptr;
+      g.colsum = ly.has_bn ? stats : nullptr; g.f16 = f16;
       P3D_TRY(tcg::gemm(g, st));
     } else if (x3) {
       GemmArgs g;   // z = (x|h) W * clip + b: A K-major, W MN-major, both split pairs
@@ -894,7 +940,8 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
     a.hs = x3 ? w.hs + li * bls : nullptr; a.seg = seg;
     a.sc = sc; a.layer = li;
     a.row0 = row0; a.B = B; a.L = L; a.has_bn = ly.has_bn; a.dropout = dropout;
-    fwd_act_kernel<<<egrid(static_cast<long long>(bl / 4)), 256, 0, st>>>(a);
+    if (f16) fwd_act_kernel<true><<<egrid(static_cast<long long>(bl / 4)), 256, 0, st>>>(a);
+    else fwd_act_kernel<false><<<egrid(static_cast<long long>(bl / 4)), 256, 0, st>>>(a);
     P3D_LAUNCH_CHECK();
   }
   {
@@ -904,7 +951,7 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       g.M = static_cast<int>(B); g.N = out; g.K = L;
       g.A = w.hb + (nh - 1) * bl; g.lda = L;
       g.B = w.wb + ly.off_w; g.ldb = kOutPad; g.b_mn = 1;
-      g.C = y; g.ldc = out; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + nh : nullptr;
+      g.C = y; g.ldc = out; g.bias = m->theta + ly.off_b; g.alpha_dev = clip ? scale + nh : nullptr; g.f16 = f16;
       P3D_TRY(tcg::gemm(g, st));
     } else if (x3) {
       GemmArgs g;   // y = h W4 * clip + b4 (W4 split pair: [L][128], segment 64)
@@ -919,9 +966,13 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
     }
   }
   const size_t ny = static_cast<size_t>(B) * out;
-  loss_dy_kernel<<<egrid(static_cast<long long>(ny)), 256, 0, st>>>(y, t, ny, static_cast<float>(2.0 * invBg / out), w.dy, lossacc,
-                                                                          tc ? w.dyb : (x3 ? w.dys : nullptr), out, tc ? kOutPad : 128,
-                                                                          x3 ? 64 : 0);
+  if (f16)
+    loss_dy_kernel<true><<<egrid(static_cast<long long>(ny)), 256, 0, st>>>(y, t, ny, static_cast<float>(2.0 * invBg / out), w.dy, lossacc,
+                                                                            reinterpret_cast<__half*>(w.dyb), out, kOutPad, 0, gs);
+  else
+    loss_dy_kernel<false><<<egrid(static_cast<long long>(ny)), 256, 0, st>>>(y, t, ny, static_cast<float>(2.0 * invBg / out), w.dy, lossacc,
+                                                                             tc ? w.dyb : (x3 ? w.dys : nullptr), out, tc ? kOutPad : 128,
+                                                                             x3 ? 64 : 0, 1.f);
   P3D_LAUNCH_CHECK();
   P3D_TRY(allreduce(m, lossacc, 1, ncclDouble, st));
   // ---------------------------------------------------------------- backward
@@ -934,7 +985,7 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       gw.M = L; gw.N = out; gw.K = static_cast<int>(B);
       gw.A = w.hb + (nh - 1) * bl; gw.lda = L; gw.a_mn = 1;
       gw.B = w.dyb; gw.ldb = kOutPad; gw.b_mn = 1;
-      gw.C = m->grad + ly.off_w; gw.ldc = out; gw.split_k = 1;
+      gw.C = m->grad + ly.off_w; gw.ldc = out; gw.split_k = 1; gw.alpha = ginv; gw.f16 = f16;
       P3D_TRY(tcg::gemm(gw, st));
     } else if (x3) {
       GemmArgs gw;   // dW4 = h^T dy: both split pairs MN-major, K = batch rows, split-K
@@ -954,7 +1005,7 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       gd.M = static_cast<int>(B); gd.N = L; gd.K = out;
       gd.A = w.dyb; gd.lda = kOutPad;
       gd.B = w.wb + ly.off_w; gd.ldb = kOutPad;
-      gd.C = G[cur]; gd.ldc = L; gd.alpha_dev = clip ? scale + nh : nullptr;
+      gd.C = G[cur]; gd.ldc = L; gd.alpha_dev = clip ? scale + nh : nullptr; gd.alpha = ginv; gd.f16 = f16;
       P3D_TRY(tcg::gemm(gd, st));
     } else if (x3) {
       GemmArgs gd;   // dh = dy W4^T * clip: both K-major (W4 rows are the output rows), K = out
@@ -977,19 +1028,26 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
     a.mask = maskbuf + li * bl; a.dz = (lowp && ly.has_bn) ? nullptr : w.dz;   // tensor-core + BN: pass B recomputes da
     a.dzb = (tc && !ly.has_bn) ? w.dzb : nullptr; a.sums = w.red + 2ull * li * L; a.sc = sc;
     a.dzs = (x3 && !ly.has_bn) ? w.dzs : nullptr; a.seg = seg;
-    a.B = B; a.L = L; a.has_bn = ly.has_bn; a.dropout = dropout;
-    bwd_act_kernel<<<dim3((L / 4 + 31) / 32, static_cast<unsigned>((B + RCH4 - 1) / RCH4)), dim3(32, 8), 0, st>>>(a);
+    a.B = B; a.L = L; a.has_bn = ly.has_bn; a.dropout = dropout; a.gs = gs;
+    const dim3 ga((L / 4 + 31) / 32, static_cast<unsigned>((B + RCH4 - 1) / RCH4));
+    if (f16) bwd_act_kernel<true><<<ga, dim3(32, 8), 0, st>>>(a);
+    else bwd_act_kernel<false><<<ga, dim3(32, 8), 0, st>>>(a);
     P3D_LAUNCH_CHECK();
     if (ly.has_bn) {
       P3D_TRY(allreduce(m, a.sums, 2ull * L, ncclDouble, st));
       // dz (bf16 only on the tensor-core path) + dgamma / dbeta.  The sums are already global after the all-reduce,
       // so every rank holds the full dgamma/dbeta: pre-divide by world so that the flat gradient all-reduce (a sum)
       // restores them exactly once.
-      bwd_bn_kernel<<<egrid(static_cast<long long>(bl / 4)), 256, 0, st>>>(w.dz, a.z, a.mean, a.rstd, a.gamma, a.sums, static_cast<float>(invBg), B, L,
-                                                                           tc ? w.dzb : nullptr, lowp ? 0 : 1, 1.0 / m->world,
-                                                                           m->grad + ly.off_gamma, m->grad + ly.off_beta,
-                                                                           lowp ? a.dh : nullptr, dropout ? a.mask : nullptr, a.beta, sc,
-                                                                           x3 ? w.dzs : nullptr, seg);
+      if (f16)
+        bwd_bn_kernel<true><<<egrid(static_cast<long long>(bl / 4)), 256, 0, st>>>(w.dz, a.z, a.mean, a.rstd, a.gamma, a.sums, static_cast<float>(invBg), B, L,
+                                                                                   reinterpret_cast<__half*>(w.dzb), 0, 1.0 / m->world, m->grad + ly.off_gamma, m->grad + ly.off_beta,
+                                                                                   a.dh, dropout ? a.mask : nullptr, a.beta, sc, nullptr, seg, gs);
+      else
+        bwd_bn_kernel<false><<<egrid(static_cast<long long>(bl / 4)), 256, 0, st>>>(w.dz, a.z, a.mean, a.rstd, a.gamma, a.sums, static_cast<float>(invBg), B, L,
+                                                                                    tc ? w.dzb : nullptr, lowp ? 0 : 1, 1.0 / m->world,
+                                                                                    m->grad + ly.off_gamma, m->grad + ly.off_beta,
+                                                                                    lowp ? a.dh : nullptr, dropout ? a.mask : nullptr, a.beta, sc,
+                                                                                    x3 ? w.dzs : nullptr, seg, 1.f);
       P3D_LAUNCH_CHECK();
       // the bias feeding a BN layer has an exactly-zero gradient (it is removed by the mean subtraction)
     } else {
@@ -1003,7 +1061,7 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
       gw.M = ly.K; gw.N = L; gw.K = static_cast<int>(B);
       gw.A = li == 0 ? w.xb : w.hb + (li - 1) * bl; gw.lda = lda; gw.a_mn = 1;
       gw.B = w.dzb; gw.ldb = L; gw.b_mn = 1;
-      gw.C = m->grad + ly.off_w; gw.ldc = L; gw.split_k = 1;
+      gw.C = m->grad + ly.off_w; gw.ldc = L; gw.split_k = 1; gw.alpha = ginv; gw.f16 = f16;
       P3D_TRY(tcg::gemm(gw, st));
     } else if (x3) {
       GemmArgs gw;   // dW = in^T dz: both split pairs MN-major, K = batch rows, split-K
@@ -1025,7 +1083,7 @@ static int train_body(p3d_model* m, const float* x, const float* t, int64_t B, b
         gd.M = static_cast<int>(B); gd.N = L; gd.K = L;
         gd.A = w.dzb; gd.lda = L;
         gd.B = w.wb + ly.off_w; gd.ldb = L;
-        gd.C = G[nxt]; gd.ldc = L; gd.alpha_dev = clip ? scale + li : nullptr;
+        gd.C = G[nxt]; gd.ldc = L; gd.alpha_dev = clip ? scale + li : nullptr; gd.alpha = ginv; gd.f16 = f16;
         if (add) { gd.res = G[keepi]; gd.ldres = L; }
         P3D_TRY(tcg::gemm(gd, st));
       } else if (x3) {
@@ -1233,9 +1291,13 @@ int p3d_model_train_epoch(p3d_model* m, const float* X, const float* T, int64_t 
 
 int p3d_model_set_train_matmul(p3d_model* m, int kind) {
   P3D_REQUIRE(m, "set_train_matmul: null model");
-  P3D_REQUIRE(kind == P3D_TRAIN_MATMUL_DEFAULT || kind == P3D_TRAIN_MATMUL_BF16X3, "set_train_matmul: unknown kind %d", kind);
-  P3D_REQUIRE(m->cfg.mode != P3D_MODE_BF16 && m->cfg.mode != P3D_MODE_FP16,
-              "set_train_matmul: bf16- and fp16-mode models train on their own tcgen05 bf16 route");
+  P3D_REQUIRE(kind == P3D_TRAIN_MATMUL_DEFAULT || kind == P3D_TRAIN_MATMUL_BF16X3 || kind == P3D_TRAIN_MATMUL_BF16 ||
+              kind == P3D_TRAIN_MATMUL_FP16, "set_train_matmul: unknown kind %d", kind);
+  // bf16 / fp16 models choose between their tcgen05 routes by name; fp32 / bf16x3 models between FFMA and bf16x3
+  const bool tc_mode = m->cfg.mode == P3D_MODE_BF16 || m->cfg.mode == P3D_MODE_FP16;
+  const bool tc_kind = kind == P3D_TRAIN_MATMUL_BF16 || kind == P3D_TRAIN_MATMUL_FP16;
+  P3D_REQUIRE(tc_mode == tc_kind, tc_mode ? "set_train_matmul: bf16- and fp16-mode models take P3D_TRAIN_MATMUL_BF16 or _FP16"
+                                          : "set_train_matmul: fp32- and bf16x3-mode models take P3D_TRAIN_MATMUL_DEFAULT or _BF16X3");
   if (kind == m->train_matmul) return P3D_OK;
   P3D_CUDA(cudaSetDevice(m->cfg.device));
   train::drop_graphs(m->tw);        // captured with the other route's launches; the next step captures again

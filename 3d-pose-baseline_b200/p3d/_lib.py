@@ -40,7 +40,7 @@ class Camera(C.Structure):
 
 
 MODE_BF16, MODE_FP32, MODE_BF16X3, MODE_FP16 = 0, 1, 2, 3
-TRAIN_MATMUL_DEFAULT, TRAIN_MATMUL_BF16X3 = 0, 1
+TRAIN_MATMUL_DEFAULT, TRAIN_MATMUL_BF16X3, TRAIN_MATMUL_BF16, TRAIN_MATMUL_FP16 = 0, 1, 2, 3
 
 # name -> (restype, argtypes): every symbol include/p3d.h declares
 PROTOTYPES = {

@@ -8,7 +8,8 @@ Differences that are visible to a caller, all additive:
   * keyword-only extras: `mode` ('bf16' tensor-core path, 'fp32', 'bf16x3': fp32 accuracy on the tensor cores
     for inference, trained like 'fp32', or 'fp16': bf16's paths on fp16 operands, <= 2e-3 row-wise error,
     trained like 'bf16'), `train_matmul` (None: the mode's own training route; 'bf16x3' with mode
-    'fp32' or 'bf16x3': the training step's MatMuls as three split-bf16 tensor-core products), `device`, `seed`, `dist`.
+    'fp32' or 'bf16x3': the training step's MatMuls as three split-bf16 tensor-core products; 'fp16' with mode 'bf16'
+    or 'fp16': the bf16 route's kernels on fp16 operands, gradients scaled by a power of two), `device`, `seed`, `dist`.
   * `step()` also accepts torch CUDA tensors (fp32) and then returns torch tensors without any host copy.
   * summaries are `Summary(tag, value)` tuples that serialize to the TF `Summary` protobuf on demand; with a
     `summaries_dir` the train/test writers append real TensorBoard event files (p3d/summary.py), without one they
@@ -152,10 +153,12 @@ class LinearModel(object):
             raise ValueError("mode must be 'bf16', 'fp32', 'bf16x3' or 'fp16'")
         # the arithmetic of the training step's MatMuls (p3d_model_set_train_matmul); with `dist`, every rank passes the
         # same value
-        if train_matmul not in (None, "bf16x3"):
-            raise ValueError("train_matmul must be None or 'bf16x3'")
-        if train_matmul is not None and mode in ("bf16", "fp16"):
+        if train_matmul not in (None, "bf16x3", "fp16"):
+            raise ValueError("train_matmul must be None, 'bf16x3' or 'fp16'")
+        if train_matmul == "bf16x3" and mode in ("bf16", "fp16"):
             raise ValueError("train_matmul='bf16x3' needs mode 'fp32' or 'bf16x3' (bf16 and fp16 models train on bf16 tensor cores)")
+        if train_matmul == "fp16" and mode not in ("bf16", "fp16"):
+            raise ValueError("train_matmul='fp16' needs mode 'bf16' or 'fp16' (the tensor-core training route)")
         self.train_matmul = train_matmul
         # Summary writers for train and test runs (linear_model.py:80-82)
         if summaries_dir:
@@ -170,8 +173,9 @@ class LinearModel(object):
         h = C.c_void_p()
         check(lib.p3d_model_create(C.byref(cfg), C.byref(h)))
         self._handle = h
-        if train_matmul == "bf16x3":
-            check(lib.p3d_model_set_train_matmul(self._handle, _lib.TRAIN_MATMUL_BF16X3))
+        if train_matmul is not None:
+            kinds = {"bf16x3": _lib.TRAIN_MATMUL_BF16X3, "fp16": _lib.TRAIN_MATMUL_FP16}
+            check(lib.p3d_model_set_train_matmul(self._handle, kinds[train_matmul]))
         self.global_step = _Evaluable(lambda: int(lib.p3d_model_global_step(self._handle)))
         self.learning_rate = _Evaluable(self._decayed_lr)
         self._names = self._query_names()

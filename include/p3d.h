@@ -63,7 +63,8 @@ extern "C" {
  * accumulation, the same tensor-core rate.  Contract: <= 2e-3 row-wise relative error against the fp64 oracle (bf16
  * mode: ~6e-3), provided every folded weight, input and activation stays inside fp16's range (|v| <= 65504).
  * linear_size % 8 != 0 runs the fp32 FFMA path.  Training steps and epochs are those of P3D_MODE_BF16 (the same
- * kernels on the bf16 tensor cores); p3d_model_set_train_matmul returns P3D_ERR_ARG. */
+ * kernels on the bf16 tensor cores) unless p3d_model_set_train_matmul(P3D_TRAIN_MATMUL_FP16) runs them on fp16
+ * operands. */
 #define P3D_MODE_FP16 3
 
 const char* p3d_last_error(void);
@@ -146,19 +147,36 @@ int p3d_model_train_epoch(p3d_model* m, const float* X, const float* T, int64_t 
 
 /* Which arithmetic runs the MatMuls of a training step (steps and epochs), chosen per model:
  *   P3D_TRAIN_MATMUL_DEFAULT: the mode's own route - tcgen05 bf16 (P3D_MODE_BF16, P3D_MODE_FP16), FFMA (P3D_MODE_FP32,
- *                             P3D_MODE_BF16X3).
+ *                             P3D_MODE_BF16X3).  Valid on P3D_MODE_FP32 and P3D_MODE_BF16X3 models.
  *   P3D_TRAIN_MATMUL_BF16X3 : every MatMul of the step (forward, data and weight gradients) on tcgen05 as three split-bf16
  *                             products hi*hi + lo*hi + hi*lo with fp32 accumulation; activations, BatchNorm, dropout,
  *                             the loss and Adam stay fp32 as on the FFMA route.  fp32-class, not bit-equal to FFMA: at
  *                             batch 64 gradients are within 2e-5 of each tensor's max of the fp64 graph; at batch 4096
  *                             the split operands move pre-activations by ~1e-5 relative, which flips the ReLU of a few
  *                             dozen units near zero (gradients within ~3e-3 relative L2) - hence opt-in.  Widths with
- *                             linear_size % 8 != 0 keep the FFMA route.
- * Valid on P3D_MODE_FP32 and P3D_MODE_BF16X3 models; a P3D_MODE_BF16 or P3D_MODE_FP16 model returns P3D_ERR_ARG.  A host call without a
- * stream: it must not be made while a training step of the model is in flight.  Switching drops the model's captured
- * training-step graphs (the next step captures again).  Data-parallel ranks must all set the same kind. */
+ *                             linear_size % 8 != 0 keep the FFMA route.  Valid on P3D_MODE_FP32 and P3D_MODE_BF16X3
+ *                             models.
+ *   P3D_TRAIN_MATMUL_BF16   : the tcgen05 bf16 route by name - what P3D_MODE_BF16 and P3D_MODE_FP16 models train on
+ *                             without a call.  Valid on P3D_MODE_BF16 and P3D_MODE_FP16 models.
+ *   P3D_TRAIN_MATMUL_FP16   : the bf16 route's kernels with fp16 in every 16-bit MatMul operand (x, h, the unclipped W,
+ *                             dy, dz); fp32 accumulation, fp32 z / BatchNorm / dropout / loss / Adam / master weights, the
+ *                             clip scale in the GEMMs' alpha, as on the bf16 route.  Gradient operands are stored as
+ *                             fp16(2^k g), k = floor(log2(global_B * out)), and every GEMM that reads one multiplies by
+ *                             2^-k in its fp32 epilogue (both exact), so dh, dgamma, dbeta, the SyncBN sums and every
+ *                             fp32 gradient are unscaled.  Accuracy (tests/test_oracle_fp16_train.py: NumPy emulation,
+ *                             width 256, 2 blocks, trained BN, max_norm, dropout 0.5, batches 64 / 4096 / 32768): the
+ *                             worst weight gradient 2.8-3.9x closer to the fp64 graph than the bf16 route's (relative L2
+ *                             2.5-3.1e-2 against 8.0-9.8e-2), the median one 2.8-4.7x, forward outputs 7.7-9x closer.
+ *                             Contract: every operand and every scaled gradient stays inside fp16's range (|v| <= 65504).
+ *                             Widths with linear_size % 8 != 0 keep the FFMA route.  Valid on P3D_MODE_BF16 and
+ *                             P3D_MODE_FP16 models; inference keeps following the mode.
+ * Any other kind for a model's mode returns P3D_ERR_ARG.  A host call without a stream: it must not be made while a
+ * training step of the model is in flight.  Switching drops the model's captured training-step graphs (the next step
+ * captures again).  Data-parallel ranks must all set the same kind. */
 #define P3D_TRAIN_MATMUL_DEFAULT 0
 #define P3D_TRAIN_MATMUL_BF16X3 1
+#define P3D_TRAIN_MATMUL_BF16 2
+#define P3D_TRAIN_MATMUL_FP16 3
 int p3d_model_set_train_matmul(p3d_model* m, int kind);
 /* Data parallel: a NCCL communicator owned by the library (SyncBN statistics + one gradient
  * all-reduce per step).  id_host = 128-byte ncclUniqueId made by rank 0 and broadcast by the caller. */
