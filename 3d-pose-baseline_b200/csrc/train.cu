@@ -1181,6 +1181,10 @@ static bool graphs_enabled() {
   static const bool on = [] { const char* e = getenv("P3D_TRAIN_GRAPH"); return !(e && e[0] == '0'); }();
   return on;
 }
+static bool dp_graphs_enabled() {
+  static const bool on = [] { const char* e = getenv("P3D_TRAIN_GRAPH_DP"); return !(e && e[0] == '0'); }();
+  return on;
+}
 
 // model.step(isTraining=True)
 int train_step(p3d_model* m, const float* x, const float* t, int64_t B, float keep, uint64_t seed, const uint8_t* mask_in,
@@ -1190,8 +1194,7 @@ int train_step(p3d_model* m, const float* x, const float* t, int64_t B, float ke
   P3D_TRY(l2persist_release(m->cfg.device));     // the fused inference kernel's L2 set-aside goes back to normal traffic
   P3D_TRY(push_scalars(m, keep, seed, st));
   // data parallel: the NCCL all-reduces (SyncBN sums, gradient) are captured into the graph with everything else
-  static const bool dp_graph = [] { const char* e = getenv("P3D_TRAIN_GRAPH_DP"); return !(e && e[0] == '0'); }();
-  if (graphs_enabled() && (m->world == 1 || dp_graph) && mask_in == nullptr) {
+  if (graphs_enabled() && (m->world == 1 || dp_graphs_enabled()) && mask_in == nullptr) {
     const size_t out = static_cast<size_t>(m->out_size);
     P3D_CUDA(cudaMemcpyAsync(w.gx, x, sizeof(float) * B * kIn, cudaMemcpyDeviceToDevice, st));
     P3D_CUDA(cudaMemcpyAsync(w.gt, t, sizeof(float) * B * out, cudaMemcpyDeviceToDevice, st));
@@ -1229,26 +1232,36 @@ __global__ void store_loss_kernel(const float* gscal, float* losses, long long i
 }
 
 // The batch loop of predict_3dpose.train() (src/predict_3dpose.py:231-259) over a device-resident training set.
+// Data parallel: every rank holds the whole set and steps its row block [lo, lo + Bl) of each global batch of B rows
+// (LinearModel's shard_rows arithmetic) through the same graph p3d_model_train_step replays for that shard.
 int train_epoch(p3d_model* m, const float* X, const float* T, int64_t n, const long long* perm, int64_t B, float keep, uint64_t seed,
                 float* losses, float* lr_last, cudaStream_t st) {
-  P3D_REQUIRE(m->world == 1, "train_epoch: data-parallel models step through p3d_model_train_step");
-  P3D_TRY(ensure_workspace(m, B));
+  P3D_REQUIRE(B >= m->world, "train_epoch: batch_size %lld leaves a rank of %d without rows", static_cast<long long>(B), m->world);
+  const int64_t base = B / m->world, rem = B % m->world;
+  const int64_t lo = m->rank * base + (m->rank < rem ? m->rank : rem);
+  const int64_t Bl = base + (m->rank < rem ? 1 : 0);
+  P3D_TRY(ensure_workspace(m, Bl));
   P3D_TRY(l2persist_release(m->cfg.device));
   TrainWorkspace& w = m->tw;
   const int64_t nb = n / B;                                   // the n % B tail is dropped (linear_model.py:311-313)
-  int g = static_cast<int>((B * (kIn + m->out_size) + 255) / 256);
+  int g = static_cast<int>((Bl * (kIn + m->out_size) + 255) / 256);
   if (g > 148 * 4) g = 148 * 4;
+  const bool graph = graphs_enabled() && (m->world == 1 || dp_graphs_enabled());
   for (int64_t b = 0; b < nb; ++b) {
     P3D_TRY(push_scalars(m, keep, seed, st));
-    gather_batch_kernel<<<g, 256, 0, st>>>(X, T, perm, b * B, static_cast<int>(B), m->out_size, w.gx, w.gt);
+    gather_batch_kernel<<<g, 256, 0, st>>>(X, T, perm, b * B + lo, static_cast<int>(Bl), m->out_size, w.gx, w.gt);
     P3D_LAUNCH_CHECK();
-    if (graphs_enabled()) P3D_TRY(train_step_staged(m, B, keep, seed, st));
-    else P3D_TRY(train_body(m, w.gx, w.gt, B, keep < 1.f, nullptr, B, 0, w.gscal, w.gscal + 1, w.gy, st));
+    if (graph) P3D_TRY(train_step_staged(m, Bl, keep, seed, st, B, lo));
+    else P3D_TRY(train_body(m, w.gx, w.gt, Bl, keep < 1.f, nullptr, B, lo, w.gscal, w.gscal + 1, w.gy, st));
     store_loss_kernel<<<1, 1, 0, st>>>(w.gscal, losses, b, lr_last);
     P3D_LAUNCH_CHECK();
     m->global_step += 1;
   }
   m->pack_valid = false;
+  if (nb > 0) {        // as train_step leaves them: the last batch's global outputs for p3d_model_gathered_outputs
+    m->dp_Bg = B;
+    m->dp_y_gathered = m->world > 1 && p2p::grad_ready(m) && B * m->out_size <= p2p::YMAX;
+  }
   return mark_model_work(m, st);
 }
 

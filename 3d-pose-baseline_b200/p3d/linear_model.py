@@ -434,24 +434,40 @@ class LinearModel(object):
         get_all_batches builds, linear_model.py:266-300; NumPy or torch CUDA), permuted (np.random.permutation
         as in :309 unless `perm` is given or shuffle=False), cut into n // batch_size batches (the tail is
         dropped, :311-313) and stepped on the device, one replayed CUDA graph per batch.
-        Returns (losses[n_batches], last learning rate) - NumPy for NumPy inputs, torch otherwise."""
+        Returns (losses[n_batches], last learning rate) - NumPy for NumPy inputs, torch otherwise.
+
+        Data parallel (`dist`): a collective like step().  Every rank is handed the whole training set, as step() hands
+        every rank the global batch; batch_size is the global batch and each rank steps its row block of every batch.
+        Rank 0's permutation (its `perm`, or its np.random.permutation draw) is broadcast and used by all ranks, as rank
+        0's dropout seed is.  Ranks that disagree on n, batch_size, dropout_keep_prob or whether the order is permuted
+        all raise ValueError before anything runs.  The losses are those of the global batches, the same on every rank."""
         torch = _lib.require_cuda()
-        if self.world > 1:
-            raise RuntimeError("train_epoch is single-GPU; data-parallel training steps through step()")
         is_torch = hasattr(encoder_inputs, "is_cuda")
         dev = torch.device("cuda", self.device)
         with torch.cuda.device(self.device):
             X = (encoder_inputs if is_torch else torch.from_numpy(np.ascontiguousarray(encoder_inputs, dtype=np.float32))).to(dev, torch.float32).contiguous()
             T = (decoder_outputs if is_torch else torch.from_numpy(np.ascontiguousarray(decoder_outputs, dtype=np.float32))).to(dev, torch.float32).contiguous()
             n = int(X.shape[0])
+            err = None
             if X.dim() != 2 or X.shape[1] != self.input_size or T.shape != (n, self.output_size):
-                raise ValueError("expected [n,%d] inputs and [n,%d] outputs" % (self.input_size, self.output_size))
+                err = "expected [n,%d] inputs and [n,%d] outputs" % (self.input_size, self.output_size)
+            elif self.world > 1 and perm is not None and np.shape(perm) != (n,):
+                err = "perm must have shape [%d]" % n
+            if self.world > 1:
+                self._dp_epoch_agree(n, dropout_keep_prob, perm is not None or shuffle, err)
+            elif err:
+                raise ValueError(err)
             nb = n // self.batch_size
             pd = None
             if perm is not None:
                 pd = torch.as_tensor(np.asarray(perm, dtype=np.int64)).to(dev)
             elif shuffle:
                 pd = torch.from_numpy(np.random.permutation(n).astype(np.int64)).to(dev)
+            if self.world > 1 and pd is not None:
+                nccl = self._dist.get_backend() == "nccl"
+                pb = pd if nccl else pd.cpu()
+                self._dist.broadcast(pb, src=0)
+                pd = pb if nccl else pb.to(dev)
             losses = torch.zeros(max(nb, 1), dtype=torch.float32, device=dev)
             lr = torch.zeros(1, dtype=torch.float32, device=dev)
             if nb:
@@ -462,6 +478,25 @@ class LinearModel(object):
         if is_torch:
             return losses, lr[0]
         return losses.cpu().numpy(), float(lr.item())
+
+    def _dp_epoch_agree(self, n, keep, permuted, err):
+        """Before a data-parallel epoch launches anything: raise ValueError on EVERY rank when any rank rejected its
+        arguments (`err`) or the ranks disagree on the sizes - one rank stepping other batches than the rest would leave
+        them in peer waits with no timeout.  One all_reduce(MAX) over (v, -v) gives the maximum and the minimum."""
+        import torch
+        v = [float(n), float(self.batch_size), float(np.float32(keep)), 1.0 if permuted else 0.0, 1.0 if err else 0.0]
+        dev = torch.device("cuda", self.device) if self._dist.get_backend() == "nccl" else "cpu"
+        t = torch.tensor(v + [-a for a in v], dtype=torch.float64, device=dev)
+        self._dist.all_reduce(t, op=self._dist.ReduceOp.MAX)
+        hi, lo = t[:5].tolist(), [-a for a in t[5:].tolist()]
+        if err:
+            raise ValueError(err)
+        if hi[4] > 0:
+            raise ValueError("train_epoch: another rank rejected its arguments")
+        if hi != lo:
+            names = ("n", "batch_size", "dropout_keep_prob", "shuffle or perm")
+            diff = ", ".join("%s %.10g..%.10g" % (k, a, b) for k, a, b in zip(names, lo, hi) if a != b)
+            raise ValueError("train_epoch: the ranks disagree on %s; every rank must pass the same" % diff)
 
     # ------------------------------------------------------------------ batching (host side, linear_model.py:247-300)
     def get_all_batches(self, data_x, data_y, camera_frame, training=True):

@@ -141,7 +141,12 @@ int p3d_model_train_step(p3d_model* m, const float* x, const float* t, int64_t B
  * perm_or_null[n] its np.random.permutation (int64, device; NULL = natural order), the n % batch_size tail is
  * dropped (:311-313).  Every batch is gathered on the device and stepped as a replayed CUDA graph - no host
  * synchronisation inside.  losses[n / batch_size] (device) receives each step's loss, lr_last_or_null the last
- * learning rate.  Single GPU (data-parallel models call p3d_model_train_step per batch). */
+ * learning rate.  Data parallel (after attach_nccl): every rank passes the whole training set and the same n,
+ * batch_size (the GLOBAL batch, >= world), keep_prob, seed, X, T and perm; each rank gathers and steps its row block of
+ * every batch (LinearModel's shard_rows: the first batch_size % world ranks take one row more) through the graph
+ * p3d_model_train_step replays for that shard, and losses receive the GLOBAL batch losses, identical on every rank.
+ * Like p3d_model_train_step it is then a collective: its exchanges wait for the peers with no timeout by default
+ * (P3D_SYNC_TIMEOUT_S=<s> makes a longer wait trap), so a rank that passes other sizes leaves the others waiting. */
 int p3d_model_train_epoch(p3d_model* m, const float* X, const float* T, int64_t n, const int64_t* perm_or_null, int64_t batch_size,
                           float keep_prob, uint64_t seed, float* losses, float* lr_last_or_null, void* stream);
 
