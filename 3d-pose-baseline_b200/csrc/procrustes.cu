@@ -36,9 +36,73 @@ __device__ __forceinline__ double warp_sum(double v) {
   return v;
 }
 
-__global__ void __launch_bounds__(PB, 4) procrustes_mpjpe_kernel(const float* __restrict__ pred, const float* __restrict__ gt,
-                                                              const __grid_constant__ EvalArgs a, float* __restrict__ dists,
-                                                              double* __restrict__ joint_sum, long long N) {
+// ---- segmented evaluation (p3d_mpjpe_segments): KINDS = 0 is the unsegmented kernel; otherwise the bitmask of
+// distances summed per segment (1 plain, 2 Procrustes-aligned), always with the squared error of the normalised rows.
+// Per segment s the sums are [2J+1] doubles: J plain joint sums, J aligned joint sums, the squared-error sum.
+constexpr int MAX_SEG = 1024;
+struct SegTable {              // segment s holds the global rows [off[s], off[s+1]); row i of the call is global row0 + i
+  long long off[MAX_SEG + 1];
+  long long row0;
+  int S;
+};
+template <class A> struct SegArgs : A { SegTable t; };
+template <class A, int KINDS> using ArgsOf = typename std::conditional<KINDS == 0, A, SegArgs<A>>::type;
+
+// The segment of global row g (the last s with off[s] <= g).  Called with a warp-uniform g: every read of the
+// parameter bank is a broadcast.
+__device__ __forceinline__ int seg_find(const SegTable& t, long long g, int hint) {
+  if (hint >= 0 && t.off[hint] <= g && g < t.off[hint + 1]) return hint;
+  int lo = 0, hi = t.S - 1;
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) >> 1;
+    if (t.off[mid] <= g) lo = mid; else hi = mid - 1;
+  }
+  return lo;
+}
+
+// A tile that straddles segments: one warp sum per distinct segment of the live lanes (lane segment ls),
+// dst[ls * stride + i] += v[i] for i < n.
+template <int NV, typename F>
+__device__ __forceinline__ void seg_scatter(const F* v, int n, bool live, int ls, double* dst, int stride) {
+  const int lane = threadIdx.x & 31;
+  unsigned pending = __ballot_sync(0xffffffffu, live);
+  while (pending) {
+    const int u = __shfl_sync(0xffffffffu, ls, __ffs(pending) - 1);
+    const bool mine = live && ls == u;
+    pending &= ~__ballot_sync(0xffffffffu, mine);
+#pragma unroll
+    for (int i = 0; i < NV; ++i) {
+      if (i < n) {
+        const double s = warp_sum(mine ? static_cast<double>(v[i]) : 0.0);
+        if (lane == 0) atomicAdd(dst + static_cast<long long>(u) * stride + i, s);
+      }
+    }
+  }
+}
+
+// Per-warp segment state of a 32-pose tile whose first pose is global row g0 and which holds nlive poses: the segment
+// of the tile's first pose, whether the whole tile lies in it, and this lane's own segment.
+struct TileSeg {
+  int s, ls;
+  bool whole;
+};
+__device__ __forceinline__ TileSeg tile_segment(const SegTable& t, long long g0, int nlive, int lane, int hint) {
+  TileSeg r;
+  r.s = seg_find(t, g0, hint);
+  r.whole = g0 + nlive - 1 < t.off[r.s + 1];
+  r.ls = r.s;
+  if (!r.whole && lane < nlive)
+    while (t.off[r.ls + 1] <= g0 + lane) ++r.ls;
+  return r;
+}
+
+// KINDS != 0 (segmented): each warp keeps the sums of its current segment per lane (fp64) and flushes them whenever
+// its segment changes; joint_sum is then the [S][2J+1] table.  Two kinds hold two more per-lane arrays: 2 blocks/SM.
+template <int KINDS = 0>
+__global__ void __launch_bounds__(PB, KINDS == 0 ? 4 : (KINDS == 3 ? 2 : 3))
+    procrustes_mpjpe_kernel(const float* __restrict__ pred, const float* __restrict__ gt,
+                            const __grid_constant__ ArgsOf<EvalArgs, KINDS> a, float* __restrict__ dists,
+                            double* __restrict__ joint_sum, long long N) {
   extern __shared__ float sm[];
   const int W = a.width, WP = a.width + 1;      // padded row pitch: conflict-free per-lane rows
   float* sp = sm;
@@ -48,8 +112,36 @@ __global__ void __launch_bounds__(PB, 4) procrustes_mpjpe_kernel(const float* __
   double jacc[MAXJ];
 #pragma unroll
   for (int j = 0; j < MAXJ; ++j) jacc[j] = 0.0;
+  // segmented: jacc sums the first requested kind, kacc the plain distance when both are, qacc the squared error
+  constexpr int NK = KINDS == 3 ? MAXJ : 1;
+  double kacc[NK], qacc = 0.0;
+#pragma unroll
+  for (int j = 0; j < NK; ++j) kacc[j] = 0.0;
+  int cur = -1, since_flush = 0;
+  auto flush = [&](int s) {
+    const int J = a.J, st = 2 * J + 1;
+    double* dst = joint_sum + static_cast<long long>(s) * st;
+#pragma unroll
+    for (int j = 0; j < MAXJ; ++j) {
+      if (j < J) {
+        const double u = warp_sum(jacc[j]);
+        if (lane == 0) atomicAdd(dst + (KINDS == 1 ? 0 : J) + j, u);
+        if constexpr (KINDS == 3) {
+          const double v = warp_sum(kacc[j]);
+          if (lane == 0) atomicAdd(dst + j, v);
+        }
+      }
+      jacc[j] = 0.0;
+      if (j < NK) kacc[j] = 0.0;
+    }
+    const double q = warp_sum(qacc);
+    if (lane == 0) atomicAdd(dst + 2 * J, q);
+    qacc = 0.0;
+  };
   const long long ntiles = (N + PB - 1) / PB;
-  for (long long tile = blockIdx.x; tile < ntiles; tile += gridDim.x) {
+  const long long per = (ntiles + gridDim.x - 1) / gridDim.x;      // segmented: contiguous tiles per block (see fp32)
+  const long long tend = KINDS == 0 ? ntiles : (blockIdx.x * per + per < ntiles ? blockIdx.x * per + per : ntiles);
+  for (long long tile = KINDS == 0 ? blockIdx.x : blockIdx.x * per; tile < tend; tile += KINDS == 0 ? gridDim.x : 1) {
     const long long p0 = tile * PB;
     const int np = static_cast<int>((N - p0 < PB) ? (N - p0) : PB);
     const int tot = np * W;
@@ -77,13 +169,22 @@ __global__ void __launch_bounds__(PB, 4) procrustes_mpjpe_kernel(const float* __
     const float* mp = sp + tid * WP;
     const float* mg = sg + tid * WP;
     const int J = a.J, J0 = a.with_hip;          // joints J0..J-1 come from the arrays, joint 0 is the hip
-    double dj[MAXJ];
+    double dj[MAXJ], dk[NK], sq = 0.0;
 #pragma unroll
     for (int j = 0; j < MAXJ; ++j) dj[j] = 0.0;
+#pragma unroll
+    for (int j = 0; j < NK; ++j) dk[j] = 0.0;
+    constexpr int ALIGN_KIND = KINDS & 2;
     if (live) {
       double T[9] = {1, 0, 0, 0, 1, 0, 0, 0, 1};
       double b = 1.0, c0 = 0.0, c1 = 0.0, c2 = 0.0;
-      if (a.use_procrustes) {
+      if constexpr (KINDS != 0) {
+        for (int k = 0; k < W; ++k) {
+          const double e = static_cast<double>(mp[k]) - static_cast<double>(mg[k]);
+          sq += e * e;
+        }
+      }
+      if (KINDS == 0 ? a.use_procrustes : ALIGN_KIND) {
         // means (X = ground truth, Y = prediction)
         double mx[3] = {0, 0, 0}, my[3] = {0, 0, 0};
         if (J0) { for (int d = 0; d < 3; ++d) { mx[d] = a.hip[d]; my[d] = a.hip[d]; } }
@@ -136,7 +237,11 @@ __global__ void __launch_bounds__(PB, 4) procrustes_mpjpe_kernel(const float* __
             }
           }
           double o0 = y[0], o1 = y[1], o2 = y[2];
-          if (a.use_procrustes) {     // out = b * out.dot(T) + c  (predict_3dpose.py:419)
+          if constexpr (KINDS == 3) {
+            const double e0 = y[0] - x[0], e1 = y[1] - x[1], e2 = y[2] - x[2];
+            dk[j] = static_cast<double>(sqrtf(static_cast<float>(e0 * e0 + e1 * e1 + e2 * e2)));
+          }
+          if (KINDS == 0 ? a.use_procrustes : ALIGN_KIND) {     // out = b * out.dot(T) + c  (predict_3dpose.py:419)
             o0 = b * (y[0] * T[0] + y[1] * T[3] + y[2] * T[6]) + c0;
             o1 = b * (y[0] * T[1] + y[1] * T[4] + y[2] * T[7]) + c1;
             o2 = b * (y[0] * T[2] + y[1] * T[5] + y[2] * T[8]) + c2;
@@ -154,24 +259,49 @@ __global__ void __launch_bounds__(PB, 4) procrustes_mpjpe_kernel(const float* __
         for (int j = 0; j < MAXJ; ++j) if (j < J) dp[j] = static_cast<float>(dj[j]);
       }
     }
+    if constexpr (KINDS == 0) {
 #pragma unroll
-    for (int j = 0; j < MAXJ; ++j) {
-      const double v = (live && j < J) ? dj[j] : 0.0;
-      jacc[j] += v;
+      for (int j = 0; j < MAXJ; ++j) {
+        const double v = (live && j < J) ? dj[j] : 0.0;
+        jacc[j] += v;
+      }
+    } else if (warp * 32 < np) {
+      const int nlive = np - warp * 32 < 32 ? np - warp * 32 : 32;
+      const TileSeg ts = tile_segment(a.t, a.t.row0 + p0 + warp * 32, nlive, lane, cur);
+      if (cur >= 0 && (!ts.whole || ts.s != cur)) { flush(cur); since_flush = 0; }
+      cur = ts.whole ? ts.s : -1;
+      if (ts.whole) {
+#pragma unroll
+        for (int j = 0; j < MAXJ; ++j) {
+          jacc[j] += dj[j];
+          if (j < NK) kacc[j] += dk[j];
+        }
+        qacc += sq;
+        if (++since_flush == 64) { flush(cur); since_flush = 0; }
+      } else {
+        const int st = 2 * J + 1;
+        seg_scatter<MAXJ>(dj, J, live, ts.ls, joint_sum + (KINDS == 1 ? 0 : J), st);
+        if (KINDS == 3) seg_scatter<NK>(dk, J, live, ts.ls, joint_sum, st);
+        seg_scatter<1>(&sq, 1, live, ts.ls, joint_sum + 2 * J, st);
+      }
     }
     __syncthreads();
   }
-  // block reduction: shuffles within the warp, shared memory across warps, one atomic per joint
+  if constexpr (KINDS != 0) {
+    if (cur >= 0) flush(cur);
+  } else {
+    // block reduction: shuffles within the warp, shared memory across warps, one atomic per joint
 #pragma unroll
-  for (int j = 0; j < MAXJ; ++j) {
-    const double s = warp_sum(jacc[j]);
-    if (lane == 0) sacc[warp][j] = s;
-  }
-  __syncthreads();
-  if (tid < a.J) {
-    double s = 0;
-    for (int w = 0; w < PB / 32; ++w) s += sacc[w][tid];
-    atomicAdd(joint_sum + tid, s);
+    for (int j = 0; j < MAXJ; ++j) {
+      const double s = warp_sum(jacc[j]);
+      if (lane == 0) sacc[warp][j] = s;
+    }
+    __syncthreads();
+    if (tid < a.J) {
+      double s = 0;
+      for (int w = 0; w < PB / 32; ++w) s += sacc[w][tid];
+      atomicAdd(joint_sum + tid, s);
+    }
   }
 }
 
@@ -196,10 +326,13 @@ constexpr int EV_WARPS = 4;
 #define EV_BLOCKS 3   // 4 blocks (128 registers) spills and is 40% slower; 3 blocks = 168 registers, no hot spills
 #endif
 
-template <int W, int J0>
-__global__ void __launch_bounds__(EV_WARPS * 32, EV_BLOCKS) mpjpe_f32_kernel(const float* __restrict__ pred, const float* __restrict__ gt,
-                                                                    const __grid_constant__ EvalArgsF a, float* __restrict__ dists,
-                                                                    double* __restrict__ joint_sum, long long N) {
+// KINDS != 0 (segmented): the fp32 per-lane sums belong to the warp's current segment and are flushed whenever it
+// changes; a tile that straddles segments goes straight to the atomics, one warp sum per distinct segment.  joint_sum
+// is then the [S][2J+1] table.  Both kinds hold J more accumulators: 2 blocks/SM (DESIGN 3.4).
+template <int W, int J0, int KINDS = 0>
+__global__ void __launch_bounds__(EV_WARPS * 32, KINDS == 3 ? 2 : EV_BLOCKS)
+    mpjpe_f32_kernel(const float* __restrict__ pred, const float* __restrict__ gt, const __grid_constant__ ArgsOf<EvalArgsF, KINDS> a,
+                     float* __restrict__ dists, double* __restrict__ joint_sum, long long N) {
   using LY = EvalLayout<W>;
   constexpr int J = W / 3 + J0;
   constexpr int ROW_BYTES = LY::PITCH * 4;
@@ -211,11 +344,17 @@ __global__ void __launch_bounds__(EV_WARPS * 32, EV_BLOCKS) mpjpe_f32_kernel(con
   const uint32_t sbuf = static_cast<uint32_t>(__cvta_generic_to_shared(buf));
   const long long ntiles = (N + 31) / 32;
   const long long nwarps = static_cast<long long>(gridDim.x) * EV_WARPS;
+  // segmented: each warp walks a contiguous range of tiles, so its segment changes about once per boundary it meets
+  // instead of at nearly every tile of a strided walk
+  const long long gwarp = static_cast<long long>(blockIdx.x) * EV_WARPS + wib;
+  const long long per = (ntiles + nwarps - 1) / nwarps;
+  const long long tend = KINDS == 0 ? ntiles : (gwarp * per + per < ntiles ? gwarp * per + per : ntiles);
+  const long long tstep = KINDS == 0 ? nwarps : 1;
   const uint8_t* gbytes = reinterpret_cast<const uint8_t*>(gt);
   const uint8_t* pbytes = reinterpret_cast<const uint8_t*>(pred);
 
   auto issue = [&](long long tile) {
-    if (tile < ntiles) {
+    if (tile < tend) {
       const long long base = tile * 32 * W * 4;
       const long long rem = N * W * 4 - base;             // valid bytes of this tile (rows are multiples of CB)
 #pragma unroll
@@ -231,22 +370,26 @@ __global__ void __launch_bounds__(EV_WARPS * 32, EV_BLOCKS) mpjpe_f32_kernel(con
     asm volatile("cp.async.commit_group;" ::: "memory");
   };
 
-  float acc[J];
+  // per-lane sums: J joint sums; segmented, J per requested kind and the squared error last
+  constexpr int NA = KINDS == 0 ? J : ((KINDS & 1) + (KINDS >> 1)) * J + 1;
+  constexpr int STRIDE = 2 * J + 1;
+  float acc[NA];
 #pragma unroll
-  for (int j = 0; j < J; ++j) acc[j] = 0.f;
-  auto flush = [&]() {
+  for (int j = 0; j < NA; ++j) acc[j] = 0.f;
+  auto flush = [&](double* dst) {
 #pragma unroll
-    for (int j = 0; j < J; ++j) {
+    for (int j = 0; j < NA; ++j) {
       const double s = warp_sum(static_cast<double>(acc[j]));
-      if (lane == 0) atomicAdd(joint_sum + j, s);
+      const int slot = KINDS == 0 ? j : (j == NA - 1 ? 2 * J : (KINDS == 2 ? J + j : j));
+      if (lane == 0) atomicAdd(dst + slot, s);
       acc[j] = 0.f;
     }
   };
 
-  long long tile = static_cast<long long>(blockIdx.x) * EV_WARPS + wib;
+  long long tile = KINDS == 0 ? gwarp : gwarp * per;
   issue(tile);
-  int since_flush = 0;
-  for (; tile < ntiles; tile += nwarps) {
+  int since_flush = 0, cur = -1;
+  for (; tile < tend; tile += tstep) {
     asm volatile("cp.async.wait_group 0;" ::: "memory");
     __syncwarp();
     float g[W], p[W];
@@ -269,22 +412,54 @@ __global__ void __launch_bounds__(EV_WARPS * 32, EV_BLOCKS) mpjpe_f32_kernel(con
       }
     }
     __syncwarp();                       // every lane holds its row: the slab can take the next tile
-    issue(tile + nwarps);
+    issue(tile + tstep);
     const long long pose = tile * 32 + lane;
     const bool live = pose < N;
-    float dj[J];
-    pose_errors_f32<W, J0>(g, p, a.sd, a.mc, a.hipc, a.use_procrustes, dj);
-    if (dists && live) {
-      float* dp = dists + pose * J;
+    if constexpr (KINDS == 0) {
+      float dj[J];
+      pose_errors_f32<W, J0>(g, p, a.sd, a.mc, a.hipc, a.use_procrustes, dj);
+      if (dists && live) {
+        float* dp = dists + pose * J;
 #pragma unroll
-      for (int j = 0; j < J; ++j) dp[j] = dj[j];
+        for (int j = 0; j < J; ++j) dp[j] = dj[j];
+      }
+#pragma unroll
+      for (int j = 0; j < J; ++j) acc[j] += live ? dj[j] : 0.f;
+      if (++since_flush == 64) { flush(joint_sum); since_flush = 0; }   // bounds the fp32 partial sums (<= 64 terms per lane)
+    } else {
+      const int nlive = N - tile * 32 < 32 ? static_cast<int>(N - tile * 32) : 32;
+      const TileSeg ts = tile_segment(a.t, a.t.row0 + tile * 32, nlive, lane, cur);
+      if (cur >= 0 && (!ts.whole || ts.s != cur)) { flush(joint_sum + static_cast<long long>(cur) * STRIDE); since_flush = 0; }
+      cur = ts.whole ? ts.s : -1;
+      // whole tile: into the lane sums; straddling tile: straight to the segments' atomics
+      auto take = [&](const float* v, int at, int n, int slot) {
+        if (ts.whole) {
+#pragma unroll
+          for (int i = 0; i < J; ++i)
+            if (i < n) acc[at + i] += live ? v[i] : 0.f;
+        } else {
+          seg_scatter<J>(v, n, live, ts.ls, joint_sum + slot, STRIDE);
+        }
+      };
+      float sq = 0.f;
+#pragma unroll
+      for (int k = 0; k < W; ++k) { const float e = p[k] - g[k]; sq = fmaf(e, e, sq); }
+      float dj[J];
+      if constexpr ((KINDS & 1) != 0) {
+        pose_errors_f32<W, J0>(g, p, a.sd, a.mc, a.hipc, 0, dj);
+        take(dj, 0, J, 0);
+      }
+      if constexpr ((KINDS & 2) != 0) {     // last: the aligned form overwrites g and p
+        pose_errors_f32<W, J0>(g, p, a.sd, a.mc, a.hipc, 1, dj);
+        take(dj, (KINDS & 1) ? J : 0, J, J);
+      }
+      take(&sq, NA - 1, 1, 2 * J);
+      if (ts.whole && ++since_flush == 64) { flush(joint_sum + static_cast<long long>(cur) * STRIDE); since_flush = 0; }
     }
-#pragma unroll
-    for (int j = 0; j < J; ++j) acc[j] += live ? dj[j] : 0.f;
-    if (++since_flush == 64) { flush(); since_flush = 0; }   // bounds the fp32 partial sums (<= 64 terms per lane)
   }
   asm volatile("cp.async.wait_group 0;" ::: "memory");
-  flush();
+  if constexpr (KINDS == 0) flush(joint_sum);
+  else if (cur >= 0) flush(joint_sum + static_cast<long long>(cur) * STRIDE);
 }
 
 // Batched procrustes.compute_similarity_transform on raw fp64 poses; one thread per pose.
@@ -332,18 +507,15 @@ __global__ void similarity_transform_kernel(const double* __restrict__ X, const 
 using namespace p3d;
 using namespace p3d::evalk;
 
-extern "C" {
+namespace {
 
-int p3d_procrustes_mpjpe_f64(const float* pred_n, const float* gt_n, const double* mean3d, const double* std3d, int predict_14,
-                         int use_procrustes, int64_t N, float* dists, double* joint_sum, void* stream) {
-  P3D_REQUIRE(pred_n && gt_n && mean3d && std3d && joint_sum && N >= 0, "procrustes_mpjpe: null argument");
-  if (N == 0) return P3D_OK;
-  static const int j16[16] = {1, 2, 3, 6, 7, 8, 12, 13, 14, 15, 17, 18, 19, 25, 26, 27};
-  static const int j14[14] = {1, 2, 3, 6, 7, 8, 13, 15, 17, 18, 19, 25, 26, 27};
-  EvalArgs a;
+const int kJ16[16] = {1, 2, 3, 6, 7, 8, 12, 13, 14, 15, 17, 18, 19, 25, 26, 27};
+const int kJ14[14] = {1, 2, 3, 6, 7, 8, 13, 15, 17, 18, 19, 25, 26, 27};
+
+void fill_args_f64(EvalArgs& a, const double* mean3d, const double* std3d, int predict_14, int use_procrustes) {
   memset(&a, 0, sizeof(a));
   const int nj = predict_14 ? 14 : 16;
-  const int* jt = predict_14 ? j14 : j16;
+  const int* jt = predict_14 ? kJ14 : kJ16;
   for (int j = 0; j < nj; ++j)
     for (int d = 0; d < 3; ++d) { a.mean[j * 3 + d] = mean3d[jt[j] * 3 + d]; a.stdv[j * 3 + d] = std3d[jt[j] * 3 + d]; }
   for (int d = 0; d < 3; ++d) a.hip[d] = mean3d[d];
@@ -351,15 +523,90 @@ int p3d_procrustes_mpjpe_f64(const float* pred_n, const float* gt_n, const doubl
   a.with_hip = predict_14 ? 0 : 1;      // dtu3d = [0,1,2] U dim_to_use_3d unless predict_14 (predict_3dpose.py:405)
   a.J = nj + a.with_hip;
   a.use_procrustes = use_procrustes ? 1 : 0;
-  const size_t smem = sizeof(float) * 2 * PB * (a.width + 1);
-  static PerDeviceOnce attr;
-  if (attr.needed()) {
-    P3D_CUDA(cudaFuncSetAttribute(procrustes_mpjpe_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
-    attr.mark();
+}
+
+void fill_args_f32(EvalArgsF& a, const double* mean3d, const double* std3d, int predict_14, int use_procrustes) {
+  const int nj = predict_14 ? 14 : 16;
+  const int* jt = predict_14 ? kJ14 : kJ16;
+  const int J = nj + (predict_14 ? 0 : 1);
+  // mean over the J joints of the un-normalised MEAN pose (the hip, data_mean_3d[0:3], is joint 0 unless predict_14)
+  double mbar[3] = {0, 0, 0};
+  for (int d = 0; d < 3; ++d) {
+    for (int j = 0; j < nj; ++j) mbar[d] += mean3d[jt[j] * 3 + d];
+    if (!predict_14) mbar[d] += mean3d[d];
+    mbar[d] /= J;
   }
+  memset(&a, 0, sizeof(a));
+  for (int j = 0; j < nj; ++j)
+    for (int d = 0; d < 3; ++d) {
+      a.sd[j * 3 + d] = static_cast<float>(std3d[jt[j] * 3 + d]);
+      a.mc[j * 3 + d] = static_cast<float>(mean3d[jt[j] * 3 + d] - mbar[d]);
+    }
+  for (int d = 0; d < 3; ++d) a.hipc[d] = static_cast<float>(mean3d[d] - mbar[d]);
+  a.use_procrustes = use_procrustes ? 1 : 0;
+}
+
+template <int KINDS>
+void launch_f64(const float* pred_n, const float* gt_n, const ArgsOf<EvalArgs, KINDS>& a, float* dists, double* sums,
+                int64_t N, cudaStream_t st) {
+  const size_t smem = sizeof(float) * 2 * PB * (a.width + 1);
   const long long ntiles = (N + PB - 1) / PB;
   const int grid = ntiles < 148 * 4 ? (int)ntiles : 148 * 4;
-  procrustes_mpjpe_kernel<<<grid, PB, smem, (cudaStream_t)stream>>>(pred_n, gt_n, a, dists, joint_sum, N);
+  procrustes_mpjpe_kernel<KINDS><<<grid, PB, smem, st>>>(pred_n, gt_n, a, dists, sums, N);
+}
+
+template <int W, int J0, int KINDS>
+int launch_f32(const float* pred_n, const float* gt_n, const ArgsOf<EvalArgsF, KINDS>& a, float* dists, double* sums,
+               int64_t N, cudaStream_t st) {
+  constexpr int smem = EV_WARPS * 2 * 32 * EvalLayout<W>::PITCH * 4;
+  constexpr int blocks = KINDS == 3 ? 2 : EV_BLOCKS;     // the kernel's __launch_bounds__
+  static PerDeviceOnce attr;
+  if (attr.needed()) {
+    P3D_CUDA(cudaFuncSetAttribute(mpjpe_f32_kernel<W, J0, KINDS>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    attr.mark();
+  }
+  const long long ntiles = (N + 31) / 32;
+  const long long nblocks = (ntiles + EV_WARPS - 1) / EV_WARPS;
+  const int grid = nblocks < 148 * blocks ? (int)nblocks : 148 * blocks;
+  mpjpe_f32_kernel<W, J0, KINDS><<<grid, EV_WARPS * 32, smem, st>>>(pred_n, gt_n, a, dists, sums, N);
+  return P3D_OK;
+}
+
+// Argument checks of p3d_mpjpe_segments[_f64]; fills the segment table of the launch.
+int segment_table(const float* pred_n, const float* gt_n, const double* mean3d, const double* std3d, int kinds, int64_t N,
+                  int64_t row0, const int64_t* offsets, int S, const double* sums, const char* fn, SegTable& t) {
+  P3D_REQUIRE(pred_n && gt_n && mean3d && std3d && offsets && sums && N >= 0, "%s: null argument or N < 0", fn);
+  P3D_REQUIRE(S >= 1 && S <= MAX_SEG, "%s: S = %d segments, must be 1..%d", fn, S, MAX_SEG);
+  P3D_REQUIRE(kinds >= 1 && kinds <= 3, "%s: kinds = %d, must be 1 (plain), 2 (aligned) or 3 (both)", fn, kinds);
+  P3D_REQUIRE(((reinterpret_cast<uintptr_t>(pred_n) | reinterpret_cast<uintptr_t>(gt_n)) & 15) == 0,
+              "%s: pred/gt must be 16-byte aligned", fn);
+  for (int s = 0; s < S; ++s)
+    P3D_REQUIRE(offsets[s] <= offsets[s + 1], "%s: offsets descend at segment %d (%lld > %lld)", fn, s,
+                (long long)offsets[s], (long long)offsets[s + 1]);
+  P3D_REQUIRE(row0 >= offsets[0] && row0 + N <= offsets[S], "%s: rows [%lld, %lld) lie outside the segments [%lld, %lld)", fn,
+              (long long)row0, (long long)(row0 + N), (long long)offsets[0], (long long)offsets[S]);
+  for (int s = 0; s <= S; ++s) t.off[s] = offsets[s];
+  t.row0 = row0;
+  t.S = S;
+  return P3D_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+int p3d_procrustes_mpjpe_f64(const float* pred_n, const float* gt_n, const double* mean3d, const double* std3d, int predict_14,
+                         int use_procrustes, int64_t N, float* dists, double* joint_sum, void* stream) {
+  P3D_REQUIRE(pred_n && gt_n && mean3d && std3d && joint_sum && N >= 0, "procrustes_mpjpe: null argument");
+  if (N == 0) return P3D_OK;
+  EvalArgs a;
+  fill_args_f64(a, mean3d, std3d, predict_14, use_procrustes);
+  static PerDeviceOnce attr;
+  if (attr.needed()) {
+    P3D_CUDA(cudaFuncSetAttribute(procrustes_mpjpe_kernel<0>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+    attr.mark();
+  }
+  launch_f64<0>(pred_n, gt_n, a, dists, joint_sum, N, (cudaStream_t)stream);
   P3D_LAUNCH_CHECK();
   return P3D_OK;
 }
@@ -370,42 +617,57 @@ int p3d_procrustes_mpjpe(const float* pred_n, const float* gt_n, const double* m
   if (N == 0) return P3D_OK;
   P3D_REQUIRE(((reinterpret_cast<uintptr_t>(pred_n) | reinterpret_cast<uintptr_t>(gt_n)) & 15) == 0,
               "procrustes_mpjpe: pred/gt must be 16-byte aligned");
-  static const int j16[16] = {1, 2, 3, 6, 7, 8, 12, 13, 14, 15, 17, 18, 19, 25, 26, 27};
-  static const int j14[14] = {1, 2, 3, 6, 7, 8, 13, 15, 17, 18, 19, 25, 26, 27};
-  const int nj = predict_14 ? 14 : 16;
-  const int* jt = predict_14 ? j14 : j16;
-  const int J = nj + (predict_14 ? 0 : 1);
-  // mean over the J joints of the un-normalised MEAN pose (the hip, data_mean_3d[0:3], is joint 0 unless predict_14)
-  double mbar[3] = {0, 0, 0};
-  for (int d = 0; d < 3; ++d) {
-    for (int j = 0; j < nj; ++j) mbar[d] += mean3d[jt[j] * 3 + d];
-    if (!predict_14) mbar[d] += mean3d[d];
-    mbar[d] /= J;
-  }
   EvalArgsF a;
-  memset(&a, 0, sizeof(a));
-  for (int j = 0; j < nj; ++j)
-    for (int d = 0; d < 3; ++d) {
-      a.sd[j * 3 + d] = static_cast<float>(std3d[jt[j] * 3 + d]);
-      a.mc[j * 3 + d] = static_cast<float>(mean3d[jt[j] * 3 + d] - mbar[d]);
-    }
-  for (int d = 0; d < 3; ++d) a.hipc[d] = static_cast<float>(mean3d[d] - mbar[d]);
-  a.use_procrustes = use_procrustes ? 1 : 0;
-  const long long ntiles = (N + 31) / 32;
-  const long long nblocks = (ntiles + EV_WARPS - 1) / EV_WARPS;
-  const int grid = nblocks < 148 * EV_BLOCKS ? (int)nblocks : 148 * EV_BLOCKS;
+  fill_args_f32(a, mean3d, std3d, predict_14, use_procrustes);
   cudaStream_t st = (cudaStream_t)stream;
+  const int rc = predict_14 ? launch_f32<42, 0, 0>(pred_n, gt_n, a, dists, joint_sum, N, st)
+                            : launch_f32<48, 1, 0>(pred_n, gt_n, a, dists, joint_sum, N, st);
+  if (rc != P3D_OK) return rc;
+  P3D_LAUNCH_CHECK();
+  return P3D_OK;
+}
+
+int p3d_mpjpe_segments(const float* pred_n, const float* gt_n, const double* mean3d, const double* std3d, int predict_14,
+                       int kinds, int64_t N, int64_t row0, const int64_t* offsets, int S, double* sums, void* stream) {
+  SegArgs<EvalArgsF> a;
+  const int rc = segment_table(pred_n, gt_n, mean3d, std3d, kinds, N, row0, offsets, S, sums, "mpjpe_segments", a.t);
+  if (rc != P3D_OK) return rc;
+  if (N == 0) return P3D_OK;
+  fill_args_f32(a, mean3d, std3d, predict_14, 0);
+  cudaStream_t st = (cudaStream_t)stream;
+  int r;
   if (!predict_14) {
-    constexpr int smem = EV_WARPS * 2 * 32 * EvalLayout<48>::PITCH * 4;
-    static PerDeviceOnce attr;
-    if (attr.needed()) { P3D_CUDA(cudaFuncSetAttribute(mpjpe_f32_kernel<48, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); attr.mark(); }
-    mpjpe_f32_kernel<48, 1><<<grid, EV_WARPS * 32, smem, st>>>(pred_n, gt_n, a, dists, joint_sum, N);
+    r = kinds == 1 ? launch_f32<48, 1, 1>(pred_n, gt_n, a, nullptr, sums, N, st)
+      : kinds == 2 ? launch_f32<48, 1, 2>(pred_n, gt_n, a, nullptr, sums, N, st)
+                   : launch_f32<48, 1, 3>(pred_n, gt_n, a, nullptr, sums, N, st);
   } else {
-    constexpr int smem = EV_WARPS * 2 * 32 * EvalLayout<42>::PITCH * 4;
-    static PerDeviceOnce attr;
-    if (attr.needed()) { P3D_CUDA(cudaFuncSetAttribute(mpjpe_f32_kernel<42, 0>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem)); attr.mark(); }
-    mpjpe_f32_kernel<42, 0><<<grid, EV_WARPS * 32, smem, st>>>(pred_n, gt_n, a, dists, joint_sum, N);
+    r = kinds == 1 ? launch_f32<42, 0, 1>(pred_n, gt_n, a, nullptr, sums, N, st)
+      : kinds == 2 ? launch_f32<42, 0, 2>(pred_n, gt_n, a, nullptr, sums, N, st)
+                   : launch_f32<42, 0, 3>(pred_n, gt_n, a, nullptr, sums, N, st);
   }
+  if (r != P3D_OK) return r;
+  P3D_LAUNCH_CHECK();
+  return P3D_OK;
+}
+
+int p3d_mpjpe_segments_f64(const float* pred_n, const float* gt_n, const double* mean3d, const double* std3d, int predict_14,
+                           int kinds, int64_t N, int64_t row0, const int64_t* offsets, int S, double* sums, void* stream) {
+  SegArgs<EvalArgs> a;
+  const int rc = segment_table(pred_n, gt_n, mean3d, std3d, kinds, N, row0, offsets, S, sums, "mpjpe_segments_f64", a.t);
+  if (rc != P3D_OK) return rc;
+  if (N == 0) return P3D_OK;
+  fill_args_f64(a, mean3d, std3d, predict_14, 0);
+  static PerDeviceOnce attr;
+  if (attr.needed()) {
+    P3D_CUDA(cudaFuncSetAttribute(procrustes_mpjpe_kernel<1>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+    P3D_CUDA(cudaFuncSetAttribute(procrustes_mpjpe_kernel<2>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+    P3D_CUDA(cudaFuncSetAttribute(procrustes_mpjpe_kernel<3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 64 * 1024));
+    attr.mark();
+  }
+  cudaStream_t st = (cudaStream_t)stream;
+  if (kinds == 1) launch_f64<1>(pred_n, gt_n, a, nullptr, sums, N, st);
+  else if (kinds == 2) launch_f64<2>(pred_n, gt_n, a, nullptr, sums, N, st);
+  else launch_f64<3>(pred_n, gt_n, a, nullptr, sums, N, st);
   P3D_LAUNCH_CHECK();
   return P3D_OK;
 }

@@ -82,6 +82,10 @@ PROTOTYPES = {
                                      c_void_p, c_void_p]),
     "p3d_procrustes_mpjpe_f64": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p,
                                      c_void_p, c_void_p]),
+    "p3d_mpjpe_segments": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int64, c_void_p,
+                                   c_int, c_void_p, c_void_p]),
+    "p3d_mpjpe_segments_f64": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_int, c_int, c_int64, c_int64, c_void_p,
+                                       c_int, c_void_p, c_void_p]),
     "p3d_similarity_transform_f64": (c_int, [c_void_p, c_void_p, c_int, c_int, c_int64, c_void_p, c_void_p, c_void_p,
                                              c_void_p, c_void_p, c_void_p]),
     "p3d_debug_stream_mix": (c_int, [c_void_p, c_void_p, c_int64, c_int64, c_void_p]),

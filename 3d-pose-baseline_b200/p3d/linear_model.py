@@ -501,6 +501,20 @@ class LinearModel(object):
     # ------------------------------------------------------------------ batching (host side, linear_model.py:247-300)
     def get_all_batches(self, data_x, data_y, camera_frame, training=True):
         """Obtain a list of all the batches, randomly permuted when training (linear_model.py:247-300)."""
+        encoder_inputs, decoder_outputs = self.stack_pairs(data_x, data_y, camera_frame)
+        n = encoder_inputs.shape[0]
+        if training:
+            perm = np.random.permutation(n)
+            encoder_inputs, decoder_outputs = encoder_inputs[perm, :], decoder_outputs[perm, :]
+        n_extra = n % self.batch_size
+        if n_extra > 0:
+            encoder_inputs, decoder_outputs = encoder_inputs[:-n_extra, :], decoder_outputs[:-n_extra, :]
+        n_batches = n // self.batch_size
+        return np.split(encoder_inputs, n_batches), np.split(decoder_outputs, n_batches)
+
+    def stack_pairs(self, data_x, data_y, camera_frame):
+        """The first half of get_all_batches: every 2D entry and its 3D entry (the '-sh' suffix of stacked-hourglass
+        detections dropped in the camera frame, '<action>.h5' in the world frame) concatenated, float64, in order."""
         n = sum(v.shape[0] for v in data_x.values())
         encoder_inputs = np.zeros((n, self.input_size), dtype=float)
         decoder_outputs = np.zeros((n, self.output_size), dtype=float)
@@ -513,14 +527,7 @@ class LinearModel(object):
             encoder_inputs[idx:idx + n2d, :] = data_x[key2d]
             decoder_outputs[idx:idx + n2d, :] = data_y[key3d]
             idx += n2d
-        if training:
-            perm = np.random.permutation(n)
-            encoder_inputs, decoder_outputs = encoder_inputs[perm, :], decoder_outputs[perm, :]
-        n_extra = n % self.batch_size
-        if n_extra > 0:
-            encoder_inputs, decoder_outputs = encoder_inputs[:-n_extra, :], decoder_outputs[:-n_extra, :]
-        n_batches = n // self.batch_size
-        return np.split(encoder_inputs, n_batches), np.split(decoder_outputs, n_batches)
+        return encoder_inputs, decoder_outputs
 
     # ------------------------------------------------------------------ graph handles (linear_model.py:128-148)
     # The reference's callers hold on to graph tensors of the model.  There is no graph here; the attributes exist and

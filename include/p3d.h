@@ -299,6 +299,21 @@ int p3d_procrustes_mpjpe(const float* pred_n, const float* gt_n, const double* m
 int p3d_procrustes_mpjpe_f64(const float* pred_n, const float* gt_n, const double* mean3d_host, const double* std3d_host,
                              int predict_14, int use_procrustes, int64_t N, float* dists_or_null, double* joint_sum,
                              void* stream);
+/* Segmented evaluation: row i of pred_n/gt_n ([N,48|42], normalised, 16-byte aligned) is global row row0 + i; segment s
+ * holds global rows [offsets_host[s], offsets_host[s+1]).  offsets ascending, S in 1..1024, offsets[0] <= row0,
+ * row0 + N <= offsets[S].  kinds: bit 0 plain distance, bit 1 Procrustes-aligned.  sums: DEVICE doubles [S][2*J + 1]
+ * = {J plain joint sums, J aligned joint sums, squared-error sum}, ACCUMULATED into (caller zeroes); unrequested kinds
+ * are left untouched.  The squared error is sum((pred_n - gt_n)^2) over the row's out columns (the evaluation loss
+ * times out per pose).  One launch whatever S is; the offsets travel in the kernel's parameters, so a captured launch
+ * stays valid.  Equal offsets (empty segments) are allowed; descending ones, S out of range, kinds outside 1..3,
+ * rows outside the table and unaligned rows return P3D_ERR_ARG.  The arithmetic per pose is that of
+ * p3d_procrustes_mpjpe (fp32) and p3d_procrustes_mpjpe_f64 (_f64). */
+int p3d_mpjpe_segments(const float* pred_n, const float* gt_n, const double* mean3d_host, const double* std3d_host,
+                       int predict_14, int kinds, int64_t N, int64_t row0, const int64_t* offsets_host, int S,
+                       double* sums, void* stream);
+int p3d_mpjpe_segments_f64(const float* pred_n, const float* gt_n, const double* mean3d_host, const double* std3d_host,
+                           int predict_14, int kinds, int64_t N, int64_t row0, const int64_t* offsets_host, int S,
+                           double* sums, void* stream);
 /* Batched procrustes.compute_similarity_transform on raw poses X,Y[N,J,3] f64 (J<=17):
  * d[N], Z[N,J,3], T[N,9], b[N], c[N,3]; any output may be NULL. */
 int p3d_similarity_transform_f64(const double* X, const double* Y, int J, int compute_optimal_scale, int64_t N,
