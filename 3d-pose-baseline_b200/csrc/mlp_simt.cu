@@ -612,6 +612,224 @@ static int launch_latency_cluster(p3d_model* m, const float* x, float* y, const 
   return P3D_OK;
 }
 
+// ----------------------------------------------------------------------------- multi-person realtime frame
+// The realtime cluster kernel above for a.rows = 2 .. MAXP people of one frame.  Same cluster, same weight ring, same
+// flag; each CTA keeps every person's activation vector (MAXP x 8 KB of sP | sQ, dynamic shared memory behind the ring),
+// so the ring gives up a slot at MAXP = 8 to stay inside 227 KB.  A warp holds one weight row's words in registers
+// (releasing the ring slot once the first person's products have used them) and reads each person's activations from
+// shared memory.  Per person the operation order is exactly the single-person
+// kernel's, so every person's enc / y / pose equal what a one-person frame computes, bit for bit.
+template <int MAXP> constexpr int people_slots() { return MAXP <= 4 ? LSLOTS : 5; }
+template <int MAXP> constexpr int people_smem() { return people_slots<MAXP>() * LPART_BYTES + 2 * MAXP * 1024 * 4 + 1024; }
+
+template <int MAXP, bool F16>
+__global__ void __launch_bounds__(LNT, 1) latency_people_kernel(const LatArgs a) {
+  using O = Op16<F16>;
+  constexpr int L = 1024;
+  constexpr int NS = people_slots<MAXP>();
+  extern __shared__ __align__(128) uint8_t lat_smem[];
+  __shared__ uint64_t wfull[NS], wfree[NS];
+  uint8_t* ring = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(lat_smem) + 127) & ~uintptr_t(127));
+  float* sP = reinterpret_cast<float*>(ring + NS * LPART_BYTES);   // [MAXP][L]
+  float* sQ = sP + MAXP * L;                                       // [MAXP][L]
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  const uint32_t rank = cl_rank();
+  const int P = a.rows;
+  const int nhid = a.nlayers - 2;
+  const int nparts = LOPW * nhid;
+  auto part_src = [&](int p) {
+    const int l = 1 + p / LOPW, o = p % LOPW;
+    return a.wt + (static_cast<size_t>(l) * L + rank * 64 + o * LNW) * a.kpad;
+  };
+  if (threadIdx.x == 0) {
+    for (int s = 0; s < NS; ++s) { lat_mbar_init(&wfull[s], 1); lat_mbar_init(&wfree[s], LNW); }
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    for (int p = 0; p < NS && p < nparts; ++p) bulk_load(ring + p * LPART_BYTES, part_src(p), LPART_BYTES, &wfull[p], 4);
+  }
+  // keypoints of all P people (one read per CTA from mapped host memory) -> person r's scratch in sQ[r] -> normalised
+  // input in sQ[r][0..31]; no other CTA writes sQ before the first cluster barrier
+  {
+    if (threadIdx.x < 36 * P) {
+      const int r = threadIdx.x / 36, j = threadIdx.x - r * 36;
+      reinterpret_cast<double*>(sQ + r * L + 64)[j] = *reinterpret_cast<const volatile double*>(a.rt.kp + threadIdx.x);
+    }
+    __syncthreads();
+    if (threadIdx.x < 32 * P) {
+      const int r = threadIdx.x >> 5, c = threadIdx.x & 31;
+      const rt::Tables* tb = a.rt.tab;
+      const double v = (openpose_h36m_coord(reinterpret_cast<const double*>(sQ + r * L + 64), tb->use2[c]) - tb->mu2[c]) / tb->sd2[c];
+      const float vf = static_cast<float>(v);
+      sQ[r * L + c] = vf;
+      if (rank == 0 && a.rt.enc) a.rt.enc[threadIdx.x] = vf;
+    }
+  }
+  uint2 w0[LOPW]; float b0[LOPW];
+#pragma unroll
+  for (int o = 0; o < LOPW; ++o) {
+    const int n = static_cast<int>(rank) * 64 + o * LNW + warp;
+    w0[o] = make_uint2(0, 0);
+    if (lane < 8) w0[o] = __ldg(reinterpret_cast<const uint2*>(a.wt + static_cast<size_t>(n) * a.kpad + lane * 4));
+    b0[o] = __ldg(a.bias + n);
+  }
+  float bias_next[LOPW];
+#pragma unroll
+  for (int o = 0; o < LOPW; ++o) bias_next[o] = (nhid > 0) ? __ldg(a.bias + L + rank * 64 + o * LNW + warp) : 0.f;
+  __syncthreads();
+
+  // ---- layer 0 (reads x in sQ[r], writes sP[r])
+#pragma unroll 1
+  for (int r = 0; r < P; ++r) {
+    float hv4[4] = {0.f, 0.f, 0.f, 0.f};
+    if (lane < 8) { const float4 h = *reinterpret_cast<const float4*>(sQ + r * L + lane * 4); hv4[0] = h.x; hv4[1] = h.y; hv4[2] = h.z; hv4[3] = h.w; }
+#pragma unroll
+    for (int o = 0; o < LOPW; ++o) {
+      const typename O::T2* w2 = reinterpret_cast<const typename O::T2*>(&w0[o]);
+      float acc = hv4[0] * O::lo(w2[0]) + hv4[1] * O::hi(w2[0]) + hv4[2] * O::lo(w2[1]) + hv4[3] * O::hi(w2[1]);
+      for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
+      const float v = fmaxf(acc + b0[o], 0.f);
+      if (lane < LC) st_cluster_f32(sP + r * L + rank * 64 + o * LNW + warp, static_cast<uint32_t>(lane), v);
+    }
+  }
+  cl_sync();
+  // ---- hidden layers: one weight row in registers, every person's activations from shared memory
+  int p = 0;
+  for (int l = 1; l <= nhid; ++l) {
+    const float* src = (l & 1) ? sP : sQ;
+    float* dst = (l & 1) ? sQ : sP;
+    const bool add_res = a.residual && l >= 2 && !(l & 1);
+    float bias[LOPW];
+#pragma unroll
+    for (int o = 0; o < LOPW; ++o) bias[o] = bias_next[o];
+    if (l < nhid) {
+#pragma unroll
+      for (int o = 0; o < LOPW; ++o) bias_next[o] = __ldg(a.bias + (l + 1) * L + rank * 64 + o * LNW + warp);
+    }
+#pragma unroll 1
+    for (int o = 0; o < LOPW; ++o, ++p) {
+      const int slot = p % NS;
+      const int n = static_cast<int>(rank) * 64 + o * LNW + warp;
+      lat_mbar_wait(&wfull[slot], (p / NS) & 1);
+      const uint2* wrow = reinterpret_cast<const uint2*>(ring + slot * LPART_BYTES + warp * 2048);
+      uint2 wv[8];
+#pragma unroll
+      for (int i = 0; i < 8; ++i) wv[i] = wrow[i * 32 + lane];          // k = i*128 + lane*4 .. +3 : conflict-free
+      const float bo = o == 0 ? bias[0] : o == 1 ? bias[1] : o == 2 ? bias[2] : bias[3];
+#pragma unroll 1
+      for (int r = 0; r < P; ++r) {
+        const float* h = src + r * L + lane * 4;
+        float acc0 = 0.f, acc1 = 0.f;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const float4 hv = *reinterpret_cast<const float4*>(h + i * 128);
+          const typename O::T2* w2 = reinterpret_cast<const typename O::T2*>(&wv[i]);
+          acc0 = fmaf(hv.x, O::lo(w2[0]), acc0); acc1 = fmaf(hv.y, O::hi(w2[0]), acc1);
+          acc0 = fmaf(hv.z, O::lo(w2[1]), acc0); acc1 = fmaf(hv.w, O::hi(w2[1]), acc1);
+        }
+        if (r == 0) {
+          // person 0's products have consumed the row's words: release the slot.  Not earlier: the ring reads are
+          // asynchronous loads, and one still in flight would see the refill.
+          __syncwarp();
+          if (lane == 0) lat_mbar_arrive(&wfree[slot]);
+          // refill the slot with part p+NS as soon as all warps have released it
+          if (threadIdx.x == 0 && p + NS < nparts) {
+            lat_mbar_wait(&wfree[slot], (p / NS) & 1);
+            bulk_load(ring + slot * LPART_BYTES, part_src(p + NS), LPART_BYTES, &wfull[slot], 4);
+          }
+          __syncwarp();
+        }
+        float acc = acc0 + acc1;
+        for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
+        float v = fmaxf(acc + bo, 0.f);
+        if (add_res) v += sP[r * L + n];
+        if (lane < LC) st_cluster_f32(dst + r * L + n, static_cast<uint32_t>(lane), v);
+      }
+    }
+    cl_sync();
+  }
+  // ---- output layer: feature g = rank*LNW + warp < out, weights straight from L2, one fmaf chain per person
+  {
+    const int l = a.nlayers - 1;
+    const int g = static_cast<int>(rank) * LNW + warp;
+    if (g < a.out) {
+      const float* src = (l & 1) ? sP : sQ;
+      const __nv_bfloat16* wrow = a.wt + (static_cast<size_t>(l) * L + g) * a.kpad;
+      uint2 wv[8];
+#pragma unroll
+      for (int i = 0; i < 8; ++i) wv[i] = __ldg(reinterpret_cast<const uint2*>(wrow + i * 128 + lane * 4));
+      const float bg = __ldg(a.bias + l * L + g);
+      const int j = a.rt.tab->use3[g];
+      const double sd = a.rt.tab->sd3[j], mu = a.rt.tab->mu3[j];
+#pragma unroll 1
+      for (int r = 0; r < P; ++r) {
+        float acc = 0.f;
+#pragma unroll
+        for (int i = 0; i < 8; ++i) {
+          const float4 hv = *reinterpret_cast<const float4*>(src + r * L + i * 128 + lane * 4);
+          const typename O::T2* w2 = reinterpret_cast<const typename O::T2*>(&wv[i]);
+          acc = fmaf(hv.x, O::lo(w2[0]), acc); acc = fmaf(hv.y, O::hi(w2[0]), acc);
+          acc = fmaf(hv.z, O::lo(w2[1]), acc); acc = fmaf(hv.w, O::hi(w2[1]), acc);
+        }
+        for (int s = 16; s > 0; s >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, s);
+        if (lane == 0) {
+          const float yv = acc + bg;
+          a.y[r * a.out + g] = yv;
+          a.rt.pose[r * 96 + j] = __dadd_rn(__dmul_rn(static_cast<double>(yv), sd), mu);
+        }
+      }
+    }
+  }
+  // all P people's outputs are ordered before the cluster barrier, the flag store after it (as in the one-person frame)
+  cl_sync();
+  if (rank == 0 && threadIdx.x == 0)
+    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(a.rt.flag), "l"(a.rt.seq) : "memory");
+}
+
+// 2 .. 8 people: <4> keeps the one-person kernel's 6-slot ring, <8> needs 64 KB of activations and keeps 5 slots.  Returns 1 when the kernel cannot serve this model / device.
+static int launch_latency_people(p3d_model* m, const rt::Fused& f, float* y, int people, cudaStream_t st) {
+  using K = void (*)(const LatArgs);
+  struct Inst { K fn; int smem; };
+  static const Inst inst[2][2] = {{{latency_people_kernel<4, false>, people_smem<4>()}, {latency_people_kernel<8, false>, people_smem<8>()}},
+                                   {{latency_people_kernel<4, true>, people_smem<4>()}, {latency_people_kernel<8, true>, people_smem<8>()}}};
+  static int ok_dev[64] = {0};                      // per device: 0 = not probed yet, 1 = usable, 2 = not usable
+  int& okd = ok_dev[m->cfg.device & 63];
+  if (okd == 0) {
+    P3D_TRY(refuse_in_capture(st, "realtime: probing the multi-person cluster kernel"));
+    bool ok = true;
+    for (const auto& row : inst)
+      for (const Inst& k : row) {
+        ok = ok && cudaFuncSetAttribute(k.fn, cudaFuncAttributeNonPortableClusterSizeAllowed, 1) == cudaSuccess &&
+             cudaFuncSetAttribute(k.fn, cudaFuncAttributeMaxDynamicSharedMemorySize, k.smem) == cudaSuccess;
+        if (!ok) break;
+        cudaLaunchConfig_t cfg{};
+        cfg.gridDim = dim3(LC); cfg.blockDim = dim3(LNT); cfg.dynamicSmemBytes = k.smem;
+        cudaLaunchAttribute attr[1];
+        attr[0].id = cudaLaunchAttributeClusterDimension; attr[0].val.clusterDim.x = LC; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+        cfg.attrs = attr; cfg.numAttrs = 1;
+        int nclusters = 0;
+        ok = cudaOccupancyMaxActiveClusters(&nclusters, k.fn, &cfg) == cudaSuccess && nclusters >= 1;
+      }
+    cudaGetLastError();
+    if (const char* e = getenv("P3D_LAT_CLUSTER")) ok = ok && atoi(e);
+    okd = ok ? 1 : 2;
+  }
+  if (okd != 1) return 1;
+  const Inst& k = inst[m->cfg.mode == P3D_MODE_FP16 ? 1 : 0][people <= 4 ? 0 : 1];
+  LatArgs a;
+  a.rt = f;
+  a.rows = people; a.x = nullptr; a.y = y; a.wt = m->wt_bf16; a.bias = m->bias_fold; a.hP = a.hQ = nullptr; a.counter = nullptr; a.base = 0;
+  a.stamps = nullptr;
+  a.L = m->L; a.nlayers = static_cast<int>(m->layers.size()); a.out = m->out_size; a.kpad = m->kpad; a.residual = m->cfg.residual;
+  cudaLaunchConfig_t cfg{};
+  cfg.gridDim = dim3(LC); cfg.blockDim = dim3(LNT); cfg.dynamicSmemBytes = k.smem; cfg.stream = st;
+  cudaLaunchAttribute attr[1];
+  attr[0].id = cudaLaunchAttributeClusterDimension; attr[0].val.clusterDim.x = LC; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
+  cfg.attrs = attr; cfg.numAttrs = 1;
+  P3D_CUDA(cudaLaunchKernelEx(&cfg, k.fn, a));
+  P3D_LAUNCH_CHECK();
+  return P3D_OK;
+}
+
 
 // ----------------------------------------------------------------------------- batch-1 whole-chip kernel
 // The 16-CTA cluster kernel above streams 512 KB of weights per SM; it is bound by what ONE SM can ingest (measured:
@@ -852,6 +1070,15 @@ int forward_latency_cluster(p3d_model* m, const float* x, float* y, cudaStream_t
 int forward_latency_cluster_rt(p3d_model* m, const rt::Fused& f, float* y, cudaStream_t st) {
   if (m->L != 1024 || (m->cfg.mode != P3D_MODE_BF16 && m->cfg.mode != P3D_MODE_FP16)) return 1;
   return launch_latency_cluster(m, nullptr, y, &f, st);
+}
+// 1 .. 8 people of one frame in one launch (f.kp [P,36], f.enc [P,32], f.pose [P,96], y [P,out]); one person is the
+// frame above, unchanged.  Returns 1 when the frame cannot run on the cluster kernel (the caller stages it).
+int forward_latency_cluster_rt_people(p3d_model* m, const rt::Fused& f, float* y, int people, cudaStream_t st) {
+  if (people == 1) return forward_latency_cluster_rt(m, f, y, st);
+  if (m->L != 1024 || (m->cfg.mode != P3D_MODE_BF16 && m->cfg.mode != P3D_MODE_FP16) || m->layers.size() < 3 ||
+      people < 2 || people > 8)
+    return 1;
+  return launch_latency_people(m, f, y, people, st);
 }
 
 int forward_small(p3d_model* m, const float* x, float* y, int64_t B, cudaStream_t st) {

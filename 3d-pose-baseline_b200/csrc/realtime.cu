@@ -17,13 +17,16 @@
 
 namespace p3d {
 namespace prep { int prepare(p3d_model* m, cudaStream_t st); }
+namespace simt { int forward_latency_cluster_rt_people(p3d_model* m, const rt::Fused& f, float* y, int people, cudaStream_t st); }
 namespace rt {
 
-struct HostIO {                      // one mapped pinned block shared with the kernel
-  double kp[36];
-  double pose[96];
-  float enc[32];
-  float y[48];
+constexpr int kMaxPeople = 8;        // people of one frame the cluster kernel serves in one launch
+
+struct HostIO {                      // one mapped pinned block shared with the kernel: up to kMaxPeople people
+  double kp[kMaxPeople][36];
+  double pose[kMaxPeople][96];
+  float enc[kMaxPeople][32];
+  float y[kMaxPeople * 48];          // [P][out]
   unsigned long long flag;
 };
 
@@ -37,8 +40,9 @@ struct p3d_realtime {
   p3d::rt::HostIO* io = nullptr;     // cudaHostAlloc'ed, mapped
   cudaStream_t stream = nullptr;
   unsigned long long seq = 0;
-  // staging of the generic batch-1 path (width != 1024 / fp32 mode / no 16-CTA cluster)
+  // staging of the generic path (width != 1024 / fp32 mode / no 16-CTA cluster / more than kMaxPeople people)
   double* d_kp = nullptr; float* d_enc = nullptr; float* d_y = nullptr; double* d_pose = nullptr;
+  int64_t d_cap = 0;                 // rows the staging buffers hold
 };
 
 namespace p3d {
@@ -68,6 +72,37 @@ __global__ void backend_kernel(const float* __restrict__ y, const Tables* __rest
     const double v = s >= 0 ? static_cast<double>(y[b * out + s]) : 0.0;
     pose[i] = __dadd_rn(__dmul_rn(v, tab->sd3[j]), tab->mu3[j]);
   }
+}
+
+// grow the staging buffers to B rows (the previous call synchronised its stream, nothing still reads them)
+static int ensure_staging(p3d_realtime* r, int64_t B) {
+  if (B <= r->d_cap) return P3D_OK;
+  cudaFree(r->d_kp); cudaFree(r->d_enc); cudaFree(r->d_y); cudaFree(r->d_pose);
+  r->d_kp = nullptr; r->d_enc = nullptr; r->d_y = nullptr; r->d_pose = nullptr; r->d_cap = 0;
+  P3D_CUDA(cudaMalloc(&r->d_kp, sizeof(double) * 36 * B));
+  P3D_CUDA(cudaMalloc(&r->d_enc, sizeof(float) * 32 * B));
+  P3D_CUDA(cudaMalloc(&r->d_y, sizeof(float) * 48 * B));
+  P3D_CUDA(cudaMalloc(&r->d_pose, sizeof(double) * 96 * B));
+  r->d_cap = B;
+  return P3D_OK;
+}
+
+// spin on the mapped flag until the kernel raised it to seq; look at the stream now and then so that a failed launch
+// cannot hang the caller
+static int wait_flag(p3d_realtime* r, unsigned long long seq, const char* who) {
+  volatile unsigned long long* flag = &r->io->flag;
+  const auto t0 = std::chrono::steady_clock::now();
+  unsigned spins = 0;
+  while (*flag != seq) {
+    if ((++spins & 0xFFFF) == 0) {
+      const cudaError_t q = cudaStreamQuery(r->stream);
+      if (q != cudaSuccess && q != cudaErrorNotReady) { set_error("%s: %s", who, cudaGetErrorString(q)); return P3D_ERR_CUDA; }
+      if (q == cudaSuccess && *flag != seq) { set_error("%s: the kernel finished without raising its flag", who); return P3D_ERR_CUDA; }
+      if (std::chrono::steady_clock::now() - t0 > std::chrono::seconds(10)) { set_error("%s: timed out", who); return P3D_ERR_CUDA; }
+    }
+  }
+  __sync_synchronize();
+  return P3D_OK;
 }
 
 static inline int grid_for(long long n) { long long g = (n + 255) / 256; if (g > 148 * 8) g = 148 * 8; return static_cast<int>(g < 1 ? 1 : g); }
@@ -120,11 +155,10 @@ int p3d_realtime_create(p3d_model* m, const double* mean2d, const double* std2d,
   if (cudaMemcpy(r->dev_tab, &t, sizeof(t), cudaMemcpyHostToDevice) != cudaSuccess) return fail("cudaMemcpy");
   if (cudaHostAlloc(reinterpret_cast<void**>(&r->io), sizeof(rt::HostIO), cudaHostAllocMapped) != cudaSuccess) return fail("cudaHostAlloc");
   memset(r->io, 0, sizeof(rt::HostIO));
-  for (int j = 0; j < 96; ++j) r->io->pose[j] = 0.0 * t.sd3[j] + t.mu3[j];     // ignored dims never change (data_utils.py:305-310)
+  for (int b = 0; b < rt::kMaxPeople; ++b)          // ignored dims never change (data_utils.py:305-310)
+    for (int j = 0; j < 96; ++j) r->io->pose[b][j] = 0.0 * t.sd3[j] + t.mu3[j];
   if (cudaStreamCreateWithFlags(&r->stream, cudaStreamNonBlocking) != cudaSuccess) return fail("cudaStreamCreate");
-  if (cudaMalloc(&r->d_kp, sizeof(double) * 36) != cudaSuccess || cudaMalloc(&r->d_enc, sizeof(float) * 32) != cudaSuccess ||
-      cudaMalloc(&r->d_y, sizeof(float) * 48) != cudaSuccess || cudaMalloc(&r->d_pose, sizeof(double) * 96) != cudaSuccess)
-    return fail("cudaMalloc");
+  if (rt::ensure_staging(r, 1) != P3D_OK) return fail("cudaMalloc");
   *out = r;
   return P3D_OK;
 }
@@ -154,41 +188,67 @@ int p3d_realtime_step_host(p3d_realtime* r, const double* xy36_host, float* enc_
   P3D_TRY(order_after_model_work(m, r->stream));     // a training step still running on the caller's stream owns the weights
   if (!m->pack_valid) { P3D_TRY(prep::prepare(m, r->stream)); }
   rt::HostIO* io = r->io;
-  memcpy(io->kp, xy36_host, sizeof(double) * 36);
+  memcpy(io->kp[0], xy36_host, sizeof(double) * 36);
   rt::Fused f;
-  f.tab = r->dev_tab; f.kp = io->kp; f.enc = io->enc; f.pose = io->pose; f.flag = &io->flag; f.seq = ++r->seq;
+  f.tab = r->dev_tab; f.kp = io->kp[0]; f.enc = io->enc[0]; f.pose = io->pose[0]; f.flag = &io->flag; f.seq = ++r->seq;
   int rc = simt::forward_latency_cluster_rt(m, f, io->y, r->stream);
   if (rc < 0) return rc;
   if (rc == 0) {
-    // spin on the mapped flag; look at the stream now and then so that a failed launch cannot hang the caller
-    volatile unsigned long long* flag = &io->flag;
-    const auto t0 = std::chrono::steady_clock::now();
-    unsigned spins = 0;
-    while (*flag != f.seq) {
-      if ((++spins & 0xFFFF) == 0) {
-        const cudaError_t q = cudaStreamQuery(r->stream);
-        if (q != cudaSuccess && q != cudaErrorNotReady) { set_error("realtime_step_host: %s", cudaGetErrorString(q)); return P3D_ERR_CUDA; }
-        if (q == cudaSuccess && *flag != f.seq) { set_error("realtime_step_host: the kernel finished without raising its flag"); return P3D_ERR_CUDA; }
-        if (std::chrono::steady_clock::now() - t0 > std::chrono::seconds(10)) { set_error("realtime_step_host: timed out"); return P3D_ERR_CUDA; }
-      }
-    }
-    __sync_synchronize();
-    memcpy(pose3d_host, io->pose, sizeof(double) * 96);
+    P3D_TRY(rt::wait_flag(r, f.seq, "realtime_step_host"));
+    memcpy(pose3d_host, io->pose[0], sizeof(double) * 96);
     if (enc_in_host_or_null) memcpy(enc_in_host_or_null, io->enc, sizeof(float) * 32);
     if (y_host_or_null) memcpy(y_host_or_null, io->y, sizeof(float) * out);
     return P3D_OK;
   }
   // generic route (width != 1024, fp32 mode, or a 16-CTA cluster cannot be scheduled): staged copies around the kernels
   P3D_TRY(order_after_model_work(r->model, r->stream));
-  P3D_CUDA(cudaMemcpyAsync(r->d_kp, io->kp, sizeof(double) * 36, cudaMemcpyHostToDevice, r->stream));
+  P3D_CUDA(cudaMemcpyAsync(r->d_kp, io->kp[0], sizeof(double) * 36, cudaMemcpyHostToDevice, r->stream));
   P3D_TRY(rt::step_device(r, r->d_kp, r->d_enc, r->d_y, r->d_pose, 1, r->stream));
-  P3D_CUDA(cudaMemcpyAsync(io->pose, r->d_pose, sizeof(double) * 96, cudaMemcpyDeviceToHost, r->stream));
-  P3D_CUDA(cudaMemcpyAsync(io->enc, r->d_enc, sizeof(float) * 32, cudaMemcpyDeviceToHost, r->stream));
+  P3D_CUDA(cudaMemcpyAsync(io->pose[0], r->d_pose, sizeof(double) * 96, cudaMemcpyDeviceToHost, r->stream));
+  P3D_CUDA(cudaMemcpyAsync(io->enc[0], r->d_enc, sizeof(float) * 32, cudaMemcpyDeviceToHost, r->stream));
   P3D_CUDA(cudaMemcpyAsync(io->y, r->d_y, sizeof(float) * out, cudaMemcpyDeviceToHost, r->stream));
   P3D_CUDA(cudaStreamSynchronize(r->stream));
-  memcpy(pose3d_host, io->pose, sizeof(double) * 96);
+  memcpy(pose3d_host, io->pose[0], sizeof(double) * 96);
   if (enc_in_host_or_null) memcpy(enc_in_host_or_null, io->enc, sizeof(float) * 32);
   if (y_host_or_null) memcpy(y_host_or_null, io->y, sizeof(float) * out);
+  return P3D_OK;
+}
+
+int p3d_realtime_step_people_host(p3d_realtime* r, const double* xy36_host, int P, float* enc_in_host_or_null,
+                                  float* y_host_or_null, double* pose3d_host) {
+  P3D_REQUIRE(r && xy36_host && pose3d_host, "realtime_step_people_host: null argument");
+  P3D_REQUIRE(P >= 0, "realtime_step_people_host: negative number of people");
+  if (P == 0) return P3D_OK;
+  p3d_model* m = r->model;
+  P3D_CUDA(cudaSetDevice(m->cfg.device));
+  const int out = m->out_size;
+  P3D_TRY(order_after_model_work(m, r->stream));     // a training step still running on the caller's stream owns the weights
+  if (!m->pack_valid) { P3D_TRY(prep::prepare(m, r->stream)); }
+  rt::HostIO* io = r->io;
+  if (P <= rt::kMaxPeople) {
+    memcpy(io->kp, xy36_host, sizeof(double) * 36 * P);
+    rt::Fused f;
+    f.tab = r->dev_tab; f.kp = io->kp[0]; f.enc = io->enc[0]; f.pose = io->pose[0]; f.flag = &io->flag; f.seq = ++r->seq;
+    const int rc = simt::forward_latency_cluster_rt_people(m, f, io->y, P, r->stream);
+    if (rc < 0) return rc;
+    if (rc == 0) {
+      P3D_TRY(rt::wait_flag(r, f.seq, "realtime_step_people_host"));
+      memcpy(pose3d_host, io->pose, sizeof(double) * 96 * P);
+      if (enc_in_host_or_null) memcpy(enc_in_host_or_null, io->enc, sizeof(float) * 32 * P);
+      if (y_host_or_null) memcpy(y_host_or_null, io->y, sizeof(float) * out * P);
+      return P3D_OK;
+    }
+  }
+  // staged route: one upload of all P people, the batched device step, the downloads, one synchronise
+  P3D_TRY(rt::ensure_staging(r, P));
+  P3D_CUDA(cudaMemcpyAsync(r->d_kp, xy36_host, sizeof(double) * 36 * P, cudaMemcpyHostToDevice, r->stream));
+  P3D_TRY(rt::step_device(r, r->d_kp, r->d_enc, r->d_y, r->d_pose, P, r->stream));
+  P3D_CUDA(cudaMemcpyAsync(pose3d_host, r->d_pose, sizeof(double) * 96 * P, cudaMemcpyDeviceToHost, r->stream));
+  if (enc_in_host_or_null)
+    P3D_CUDA(cudaMemcpyAsync(enc_in_host_or_null, r->d_enc, sizeof(float) * 32 * P, cudaMemcpyDeviceToHost, r->stream));
+  if (y_host_or_null)
+    P3D_CUDA(cudaMemcpyAsync(y_host_or_null, r->d_y, sizeof(float) * out * P, cudaMemcpyDeviceToHost, r->stream));
+  P3D_CUDA(cudaStreamSynchronize(r->stream));
   return P3D_OK;
 }
 

@@ -94,6 +94,7 @@ PROTOTYPES = {
     "p3d_realtime_create": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, C.POINTER(c_void_p)]),
     "p3d_realtime_destroy": (None, [c_void_p]),
     "p3d_realtime_step_host": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "p3d_realtime_step_people_host": (c_int, [c_void_p, c_void_p, c_int, c_void_p, c_void_p, c_void_p]),
     "p3d_realtime_step": (c_int, [c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_int64, c_void_p]),
     "p3d_model_p2p_handle": (c_int, [c_void_p, c_void_p]),
     "p3d_model_p2p_attach": (c_int, [c_void_p, c_void_p, c_int, c_int]),

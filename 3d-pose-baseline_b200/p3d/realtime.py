@@ -6,9 +6,14 @@
     xy = keypoints_to_xy(json.load(f)["people"][0]["pose_keypoints_2d"])      # :69-135 (list handling)
     enc_in, poses3d_norm, poses3d = lifter.step(xy)                            # :137-171 (one CUDA launch)
 
+    xys, frame = read_openpose_json(path, all_people=True)                     # every person of the frame
+    enc_in, poses3d_norm, poses3d = lifter.step_people(xys)                    # [P,32], [P,out], [P,96]
+
 `step` runs keypoint re-ordering, hip/neck/thorax synthesis, normalisation, the six-layer lifter and
 unNormalizeData in a single 16-CTA cluster kernel that reads from and writes to mapped pinned memory
-(p3d_realtime_step_host).  `step_batch` does the same for many frames on device buffers.
+(p3d_realtime_step_host).  `step_people` lifts up to 8 people of one frame in that same single launch, each person
+bit-identical to its own `step` (p3d_realtime_step_people_host; more people, or a model the cluster kernel does not
+serve, take one staged batched step).  `step_batch` does the same for many frames on device buffers.
 JSON parsing / list surgery stays on the host exactly as in the reference; plotting is out of scope -
 `display_transform` is the coordinate shuffle the reference applies right before viz.show3Dpose (:178-195).
 """
@@ -46,13 +51,16 @@ def keypoints_to_xy(pose_keypoints_2d):
     return xy
 
 
-def read_openpose_json(path):
-    """First person of an OpenPose JSON file (:67-69) -> (xy list, frame number from the file name :81-82)."""
+def read_openpose_json(path, all_people=False):
+    """First person of an OpenPose JSON file (:67-69) -> (xy list, frame number from the file name :81-82).
+    all_people=True: ([xy list of every person], frame number); [] for a frame with nobody in it."""
     with open(path) as f:
         data = json.load(f)
-    xy = keypoints_to_xy(data["people"][0]["pose_keypoints_2d"])
     idx = re.findall(r"(\d+)", path)
-    return xy, (int(idx[-1]) if idx else 0)
+    frame = int(idx[-1]) if idx else 0
+    if all_people:
+        return [keypoints_to_xy(p["pose_keypoints_2d"]) for p in data["people"]], frame
+    return keypoints_to_xy(data["people"][0]["pose_keypoints_2d"]), frame
 
 
 def display_transform(poses3d, spine_x, spine_y):
@@ -70,6 +78,8 @@ def display_transform(poses3d, spine_x, spine_y):
 
 class RealtimeLifter(object):
     """Owns the device tables and the mapped host block of one realtime session (p3d_realtime_*)."""
+
+    MAX_PEOPLE = 8          # people of one frame step_people lifts in one launch (p3d_realtime_step_people_host)
 
     def __init__(self, model, data_mean_2d, data_std_2d, dim_to_use_2d, data_mean_3d, data_std_3d, dim_to_use_3d):
         self.model = model
@@ -96,6 +106,12 @@ class RealtimeLifter(object):
         self._pose = np.empty((1, 96), dtype=np.float64)
         self._args = (self._handle, C.c_void_p(self._kp.ctypes.data), C.c_void_p(self._enc.ctypes.data),
                       C.c_void_p(self._y.ctypes.data), C.c_void_p(self._pose.ctypes.data))
+        # the same for the up to MAX_PEOPLE people of one frame that step_people serves in one launch
+        self._kps = np.zeros((self.MAX_PEOPLE, 36), dtype=np.float64)
+        self._encs = np.empty((self.MAX_PEOPLE, 32), dtype=np.float32)
+        self._ys = np.empty((self.MAX_PEOPLE, self.output_size), dtype=np.float32)
+        self._poses = np.empty((self.MAX_PEOPLE, 96), dtype=np.float64)
+        self._people_ptrs = tuple(C.c_void_p(a.ctypes.data) for a in (self._kps, self._encs, self._ys, self._poses))
 
     def step(self, xy):
         """One frame: xy = at least 36 coordinates (x0,y0,x1,y1,...; :137-142 use the first 36).
@@ -108,6 +124,34 @@ class RealtimeLifter(object):
         self._kp[:] = xy[:36]
         check(lib.p3d_realtime_step_host(*self._args))
         return self._enc.copy(), self._y.copy(), self._pose.copy()      # fresh arrays, like the reference returns
+
+    def step_people(self, xys):
+        """Every person of one frame: xys = P coordinate lists (or a [P, >=36] array), the first 36 values of each used
+        as in `step`.  Returns fresh (enc_in [P,32] fp32, poses3d_normalised [P,out] fp32, poses3d [P,96] fp64); row p
+        equals `step(xys[p])` bit for bit when P <= 8 and the model runs `step` as one launch (width 1024, bf16 or fp16).
+        Otherwise the people run as one staged batch and equal `step_batch` of the same keypoints."""
+        P = len(xys)
+        for xy in xys:
+            if len(xy) < 36:
+                raise IndexError("need at least 36 keypoint coordinates, got %d" % len(xy))
+        if self._handle is None:
+            raise RuntimeError("RealtimeLifter is closed")
+        if P == 0:
+            return (np.empty((0, 32), np.float32), np.empty((0, self.output_size), np.float32),
+                    np.empty((0, 96), np.float64))
+        if P <= self.MAX_PEOPLE:
+            kp, enc, y, pose = self._kps, self._encs, self._ys, self._poses
+            ptrs = self._people_ptrs
+        else:
+            kp = np.empty((P, 36), np.float64)
+            enc = np.empty((P, 32), np.float32)
+            y = np.empty((P, self.output_size), np.float32)
+            pose = np.empty((P, 96), np.float64)
+            ptrs = tuple(C.c_void_p(a.ctypes.data) for a in (kp, enc, y, pose))
+        for i, xy in enumerate(xys):
+            kp[i] = xy[:36]
+        check(lib.p3d_realtime_step_people_host(self._handle, ptrs[0], P, ptrs[1], ptrs[2], ptrs[3]))
+        return enc[:P].copy(), y[:P].copy(), pose[:P].copy()
 
     def step_batch(self, xy):
         """Many frames at once: xy [B,36] (NumPy or torch CUDA fp64) -> (enc_in [B,32], y [B,out], poses3d [B,96])."""

@@ -234,6 +234,17 @@ void p3d_realtime_destroy(p3d_realtime* r);
  * enc_in_host[32] and y_host[out] (the normalised input / prediction) are optional. */
 int p3d_realtime_step_host(p3d_realtime* r, const double* xy36_host, float* enc_in_host_or_null, float* y_host_or_null,
                            double* pose3d_host /*[96]*/);
+/* P people of one frame, HOST buffers, synchronous: xy36_host[P,36] -> enc_in[P,32], y[P,out] (both optional), pose3d[P,96].
+ * Routes:
+ *   - P = 1 .. 8, linear_size 1024, bf16 or fp16 mode, at least 3 layers, a schedulable 16-CTA cluster: ONE kernel launch
+ *     over mapped pinned memory, as p3d_realtime_step_host (P = 1 launches exactly its kernel).  Every person's enc_in, y
+ *     and pose3d are bit-identical to that person's p3d_realtime_step_host frame.
+ *   - otherwise (P > 8, other widths, fp32 / bf16x3 models, no cluster): one upload, the batched device step of
+ *     p3d_realtime_step with B = P, the downloads and a synchronise.  The results equal p3d_realtime_step on the same
+ *     keypoints bit for bit.
+ * P = 0 returns P3D_OK and launches nothing; P < 0 or a null xy36_host / pose3d_host is P3D_ERR_ARG. */
+int p3d_realtime_step_people_host(p3d_realtime* r, const double* xy36_host, int P, float* enc_in_host_or_null,
+                                  float* y_host_or_null, double* pose3d_host);
 /* B frames, DEVICE buffers, asynchronous on `stream`: xy36[B,36] fp64 -> enc_in[B,32], y[B,out], pose3d[B,96] (optional). */
 int p3d_realtime_step(p3d_realtime* r, const double* xy36, float* enc_in, float* y, double* pose3d_or_null, int64_t B,
                       void* stream);
